@@ -3,7 +3,7 @@
 achieved HBM GB/s vs peak).
 
     python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload cfg2|cfg1|cfg1_16|cfg3|cfg3_rot90|cfg5|cfg5_32]
-                    [--cameras C]
+                    [--cameras C] [--dump-outputs DIR]
 
 A step = one pass of the hot path over one batch of synthetic packed12 frames already resident in HBM: the fused
 packed12 -> demosaic -> tone map -> quantise sweep of batch k (``Camera32/16.process_packed12``) while the joint
@@ -15,7 +15,9 @@ records over NVLink mailboxes so that all cameras share one exposure (``--shared
 ``--cameras C`` instead shards C camera streams over the ranks (BASELINE configs[2]: 12 cameras; strong scaling).
 
 Prints ONE JSON line (keys at the bottom of main()).  The default N = 1 run also times the other BASELINE
-configurations (>= 0.5 s each) into ``configs``.  ``--impl reference`` times the CPU restatement of the reference path
+configurations (>= 0.5 s each) into ``configs``.  ``--dump-outputs DIR`` writes the outputs of the last of the K timed
+steps (rank 0) as float32 ``DIR/out<i>.npy`` (see ``dump_outputs``): the inputs are seeded, so two builds run with the
+same arguments can be compared output for output.  ``--impl reference`` times the CPU restatement of the reference path
 (oracle/c/isp_oracle.c, OpenMP on all host cores): Taichi, and therefore the reference's own CPU backend, is not
 installable in this image.
 """
@@ -295,10 +297,33 @@ def launches_per_step(tonemap, isp_dt, resize, shared, lookahead, map16=False):
     return sweep + (2 if (shared or lookahead) else 1)
 
 
+DUMP_BYTES = 48 << 20      # what --dump-outputs writes at most, sample index included
+
+
+def dump_outputs(outs, directory):
+    """The outputs of one step as float32 ``out<i>.npy`` (exact for u8 / u16 / f16): whole when all of them fit
+    DUMP_BYTES, otherwise the same sample of flat element indices from each -- drawn without replacement by
+    ``np.random.default_rng(0)`` and sorted, so it depends on the output shape only -- stored as float64
+    ``sample_index.npy``."""
+    import torch
+    os.makedirs(directory, exist_ok=True)
+    numel = outs[0].numel()
+    k = DUMP_BYTES // (4 * len(outs) + 8)
+    idx = None
+    if 4 * numel * len(outs) > DUMP_BYTES:
+        idx = np.sort(np.random.default_rng(0).choice(numel, k, replace=False))
+        np.save(os.path.join(directory, "sample_index.npy"), idx.astype(np.float64))
+        idx = torch.from_numpy(idx).to(outs[0].device)
+    for i, o in enumerate(outs):
+        v = o.float()                                   # before the gather: CUDA has none for uint16
+        np.save(os.path.join(directory, f"out{i}.npy"), (v if idx is None else v.reshape(-1)[idx]).cpu().numpy())
+
+
 def run_workload(ctx: Ctx, name: str, steps: int, warmup: int, min_seconds: float = 0.0, shared=None, cameras: int = 0,
-                 isolate: bool = True):
+                 isolate: bool = True, dump_dir=None):
     """Times `steps` steps of workload `name` (max over ranks, CUDA events), then -- when min_seconds > 0 -- keeps the same
     steps running for at least that long (timed the same way: the sustained figure with the clocks sampled under it).
+    dump_dir: where rank 0 writes the outputs of the last of the `steps` timed steps (dump_outputs).
     Returns a dict of results plus the live objects the caller may reuse (isp, frames)."""
     torch = ctx.torch
     import taichi_image_b200 as tib
@@ -402,6 +427,8 @@ def run_workload(ctx: Ctx, name: str, steps: int, warmup: int, min_seconds: floa
     kern_ms_cool = kernel_alone() if (isolate and n > 0) else None
     total_px = world * px_per_step if not cameras else cameras * h * w
     ms, t0, t1 = timed(steps)
+    if dump_dir and rank == 0 and n > 0:
+        dump_outputs(outs, dump_dir)
     res = {"workload": desc, "value": total_px * steps / (ms * 1e-3) / 1e9, "ms_per_step": ms / steps, "steps": steps,
            "frames_per_gpu": n, "height": h, "width": w, "tonemap": tonemap, "out_dtype": out_dt, "isp_dtype": isp_dt}
     clocks = ctx.sampler.window(t0, t1) if ctx.sampler else None
@@ -545,7 +572,8 @@ def main():
     os.dup2(2, 1)                      # fd 1 -> stderr for native libraries and stray prints
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=200)
+    ap.add_argument("--steps", type=int, default=200, help="timed steps of the workload: `value` and --dump-outputs come "
+                    "from exactly these (the sustained window and the other configurations are timed separately)")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--workload", default="cfg2", choices=sorted(WORKLOADS))
@@ -564,15 +592,23 @@ def main():
     ap.add_argument("--min-seconds", type=float, default=0.5, help="length of the sustained window after the K timed steps")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step of the workload to DIR/out<i>.npy (float32; a fixed "
+                         "sample of at most 48 MiB in all, see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs writes the outputs of the CUDA path (--impl b200)")
         return run_reference(args)
 
     ctx = Ctx(args)
     world, rank = ctx.world, ctx.rank
     shared = (world > 1) if args.shared_exposure < 0 else bool(args.shared_exposure)
     name = args.workload
-    top = run_workload(ctx, name, args.steps, args.warmup, min_seconds=args.min_seconds, shared=shared, cameras=args.cameras)
+    top = run_workload(ctx, name, args.steps, args.warmup, min_seconds=args.min_seconds, shared=shared, cameras=args.cameras,
+                       dump_dir=args.dump_outputs)
     live = top.pop("_live")
     n, h, w, isp_dt, tonemap, out_dt, tm, desc = WORKLOADS[name]
 

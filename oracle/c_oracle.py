@@ -4,6 +4,7 @@ from __future__ import annotations
 import ctypes as C
 import os
 import subprocess
+import tempfile
 
 import numpy as np
 
@@ -14,14 +15,21 @@ PATTERN_CODE = {"RGGB": 0, "GRBG": 1, "GBRG": 2, "BGGR": 3}
 
 
 def build(force=False) -> str:
-    if force or not os.path.exists(LIB) or os.path.getmtime(LIB) < os.path.getmtime(SRC):
-        os.makedirs(os.path.dirname(LIB), exist_ok=True)
-        subprocess.run(["gcc", "-O2", "-fopenmp", "-ffp-contract=off", "-fno-fast-math", "-shared", "-fPIC",
-                        "-o", LIB, SRC, "-lm"], check=True)
-    return LIB
+    """The library build.py left in the tree when it is current; otherwise a fresh build in a temporary directory
+    that lives as long as this process, so that running the oracle (tests, bench.py's CPU baseline) never writes
+    into a tree that may be read-only."""
+    global _tmp
+    if not force and os.path.exists(LIB) and os.path.getmtime(LIB) >= os.path.getmtime(SRC):
+        return LIB
+    _tmp = tempfile.TemporaryDirectory(prefix="isp_oracle_")
+    out = os.path.join(_tmp.name, os.path.basename(LIB))
+    subprocess.run(["gcc", "-O2", "-fopenmp", "-ffp-contract=off", "-fno-fast-math", "-shared", "-fPIC",
+                    "-o", out, SRC, "-lm"], check=True)
+    return out
 
 
 _lib = None
+_tmp = None
 
 
 def lib():
