@@ -32,7 +32,7 @@
 extern "C" {
 #endif
 
-#define B200ISP_VERSION 100            /* 0.1.0 */
+#define B200ISP_VERSION 101            /* 0.1.1 */
 #define B200ISP_MAX_FRAMES 64          /* frames per batched call */
 #define B200ISP_METRICS 9              /* camera_isp.py:102-115 */
 
@@ -187,8 +187,6 @@ typedef struct {
   int demosaic;                 /* b200isp_demosaic_t: 0 = Malvar-He-Cutler (bayer.py:30-55), 1 = bilinear (extension) */
   int out_yuv420;               /* 1: every output is a planar YUV 4:2:0 image, (3H/2, W) u8 (color/yuv_420.py:95-118), instead
                                    of RGB -- Camera16 + Reinhard + u8 with reinhard_scratch only; other combinations fail */
-  int reinhard_group;           /* Camera32 Reinhard (max sweep + write sweep per group of frames): frames per group;
-                                   0 = default (all frames of the call in one pair of launches) */
   int out_height, out_width;    /* > 0: bilinear resize of the demosaiced image BEFORE metering / tone map (camera_isp.py:302-315,
                                    :371-373; interpolate.py:59-66) fused into the pass: outputs are (out_height, out_width, 3) */
   float scale_r, scale_c;       /* source position of output (ro, co) = (ro / scale_r, co / scale_c) in f32, interpolate.py:60 */
@@ -201,8 +199,8 @@ typedef struct {
                                    flip_horiz 1, flip_vert 2, rotate_180 3, transpose 4, rotate_270 5, rotate_90 6, transverse 7 */
   int reinhard_mode;            /* Camera32 Reinhard -> u8 with reinhard_scratch: 0 = one sweep that also stores the map as u16 fixed point
                                    + a normalise pass (u8 within 1 LSB of the two-sweep result; color_adapt == 0, 0.3 <= gamma <= 1;
-                                   frames whose map leaves [0, 1) are redone exactly), 1 = always the exact max sweep + write sweep,
-                                   2 = experiment: exact integer-RGB scratch (csrc/reinhard_u16.cuh) */
+                                   frames whose map leaves [0, 1) are redone exactly), 1 = always the exact max sweep + write sweep;
+                                   any other value also takes the exact form */
   int ids_layout;               /* packed layout of the input frames: 0 = standard (packed.py:23-31), 1 = IDS (packed.py:36-44),
                                    decoded inside the row loader (4 instead of 2 instructions per sample, no re-pack pass) */
   void* profile_start;          /* optional cudaEvent_t pair recorded on `stream` immediately before / after */
@@ -211,7 +209,8 @@ typedef struct {
   size_t meter_cache_bytes;     /*   metering phase then re-reads the phase-1 samples instead of recomputing them */
   void* reinhard_scratch;       /* optional device scratch, >= n_frames*H*W*3*2 bytes: Camera16 Reinhard then runs ONE sweep that */
   size_t reinhard_scratch_bytes;/*   stores the f16 map (camera_isp.py:211) + an element-wise normalise / quantise pass; Camera32 -> u8
-                                     likewise with a u16 fixed-point map (see reinhard_mode) */
+                                     likewise with a u16 fixed-point map (see reinhard_mode).  Camera16 -> u8 with gamma != 1 and a
+                                     further n_frames*65536 bytes behind the maps runs that pass through a per-frame table */
 } b200isp_fused_params;
 
 /* camera_isp.py:333-340 load_packed12 + :376-385 update_metering + :394-413 tonemap_* over a

@@ -1,10 +1,9 @@
 #!/bin/bash
-# final tree of round 2 (turned pass at 8 CTAs per SM, gated sweeps with the early exit): full GPU suite, smoke, turned A/B,
+# final tree of round 2 (turned pass at 8 CTAs per SM, gated sweeps with the early exit): full GPU suite, smoke,
 # the default bench line
 mkdir -p gpurun_out
 python -m pytest tests -m gpu -q > gpurun_out/pytest_gpu.log 2>&1; echo "pytest rc=$?"; tail -3 gpurun_out/pytest_gpu.log
 python __graft_entry__.py smoke > gpurun_out/smoke.log 2>&1; echo "smoke rc=$?"; tail -1 gpurun_out/smoke.log
-python scripts/gpu_turned_ab.py > gpurun_out/turned_ab3.txt 2>&1; cat gpurun_out/turned_ab3.txt
 python bench.py > gpurun_out/r2t_bench_n1.json 2> gpurun_out/r2t_bench_n1.err; echo "bench rc=$?"
 python - <<PY
 import json

@@ -12,4 +12,4 @@ from .dtypes import (u8, u16, i16, f16, f32, uint8, uint16, int16, float16, floa
 from . import types, util, packed, bayer, tonemap, interpolate, color, camera_isp, distributed  # noqa: F401
 from .camera_isp import Camera16, Camera32  # noqa: F401
 
-__version__ = "0.1.0"
+__version__ = "0.1.1"

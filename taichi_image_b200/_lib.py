@@ -33,7 +33,7 @@ class FusedParams(C.Structure):
                 ("gamma", C.c_float), ("intensity", C.c_float), ("light_adapt", C.c_float),
                 ("color_adapt", C.c_float), ("metering_stride", C.c_int), ("alpha", C.c_float),
                 ("update_metering", C.c_int), ("rows_per_task", C.c_int), ("demosaic", C.c_int), ("out_yuv420", C.c_int),
-                ("reinhard_group", C.c_int), ("out_height", C.c_int), ("out_width", C.c_int),
+                ("out_height", C.c_int), ("out_width", C.c_int),
                 ("scale_r", C.c_float), ("scale_c", C.c_float), ("resize_gather", C.c_int), ("out_pitch", C.c_int), ("flip", C.c_int), ("reinhard_mode", C.c_int), ("ids_layout", C.c_int),
                 ("profile_start", C.c_void_p), ("profile_stop", C.c_void_p),
                 ("meter_cache", C.c_void_p), ("meter_cache_bytes", C.c_size_t),

@@ -457,7 +457,6 @@ def camera_isp(name: str, dtype=f32):
             p.out_yuv420 = int(bool(yuv420))
             p.ids_layout = int(bool(self._ids_layout if ids_format is None else ids_format))
             p.flip = int(flip)
-            p.reinhard_group = int(os.environ.get("B200ISP_REINHARD_GROUP", "0"))      # tuning knob (0 = library default)
             plan = self._resize_plan(h, w)
             ho, wo = h, w
             if plan is not None:                 # resize fused into the pass (demosaic + bilinear gather)
@@ -474,7 +473,7 @@ def camera_isp(name: str, dtype=f32):
                     cache = self._meter_cache = torch.empty(need, dtype=torch.uint8, device=self.device)
                 p.meter_cache, p.meter_cache_bytes = cache.data_ptr(), cache.numel()
                 self._meter_n = need // 12
-            if tonemap == "reinhard" and (plan is not None or (isp_dtype == f16 and os.environ.get("B200ISP_CAM16_RECOMPUTE", "0") != "1")):
+            if tonemap == "reinhard" and (plan is not None or isp_dtype == f16):
                 # scratch for the un-normalised Reinhard map in the ISP dtype: Camera16 (one sweep + a light normalise
                 # pass, csrc/fused_isp.cuh) and every resizing ISP (output resolution, csrc/fused_resize.cu)
                 # (+ 64 KB per frame: the table of the normalise pass, csrc/fused_isp.cuh run_lut_pass; unused by resizing ISPs)
@@ -483,18 +482,6 @@ def camera_isp(name: str, dtype=f32):
                 if sc is None or sc.numel() < need or sc.device != torch.device(self.device):
                     sc = self._reinhard_scratch = torch.empty(need, dtype=torch.uint8, device=self.device)
                 p.reinhard_scratch, p.reinhard_scratch_bytes = sc.data_ptr(), sc.numel()
-            elif (tonemap == "reinhard" and isp_dtype == f32 and ccm is None and float(tm.get("color_adapt", 0.0)) == 0.0
-                  and not yuv420 and os.environ.get("B200ISP_CAM32_ONE_SWEEP", "0") == "1"):
-                # EXPERIMENT, off by default (profiles/r02_reinhard_u16.txt: exact, but 8 % slower than the two sweeps):
-                # Camera32 without colour correction: scratch for the exact integer RGB (3 x u16 per pixel) + the f32 side
-                # table of the image-frame pixels -- one sweep + an element-wise pass (csrc/reinhard_u16.cuh)
-                a16 = lambda x: (x + 15) & ~15
-                need = len(frames) * (a16(h * w * 6) + a16((4 * w + 4 * (h - 4)) * 12))
-                sc = getattr(self, "_reinhard_scratch", None)
-                if sc is None or sc.numel() < need or sc.device != torch.device(self.device):
-                    sc = self._reinhard_scratch = torch.empty(need, dtype=torch.uint8, device=self.device)
-                p.reinhard_scratch, p.reinhard_scratch_bytes = sc.data_ptr(), sc.numel()
-                p.reinhard_mode = 2
             elif (tonemap == "reinhard" and isp_dtype == f32 and out_dtype.name == "u8" and not self.reinhard_exact
                   and float(tm.get("color_adapt", 0.0)) == 0.0 and 0.3 <= float(tm.get("gamma", 1.0)) <= 1.0
                   and not yuv420 and (not flip or flip & 4) and not p.ids_layout):
@@ -502,7 +489,7 @@ def camera_isp(name: str, dtype=f32):
                 # normalise / gamma / quantise pass instead of the max sweep + write sweep (csrc/fused_isp.cuh, run_fused);
                 # the u8 result is within 1 LSB of the exact form, ISP(reinhard_exact=True) / B200ISP_REINHARD_EXACT=1 keep
                 # the two sweeps.  The library falls back to them on its own when the scratch does not apply (pitched outputs).
-                need = len(frames) * h * w * 6 + len(frames) * 65536          # maps + the 64 KB tables of the normalise pass
+                need = len(frames) * h * w * 6
                 sc = getattr(self, "_reinhard_scratch", None)
                 if sc is None or sc.numel() < need or sc.device != torch.device(self.device):
                     sc = self._reinhard_scratch = torch.empty(need, dtype=torch.uint8, device=self.device)
@@ -518,7 +505,7 @@ def camera_isp(name: str, dtype=f32):
             (the tiled transform kernel then runs on the results)"""
             shape = (height,)
             flip = 0
-            if not self._resizes and not yuv420 and self.demosaic == "malvar" and os.environ.get("B200ISP_NO_FUSED_TRANSFORM", "0") != "1":
+            if not self._resizes and not yuv420 and self.demosaic == "malvar":
                 T = interpolate.ImageTransform
                 flip = {T.flip_horiz: 1, T.flip_vert: 2, T.rotate_180: 3, T.transpose: 4, T.rotate_270: 5, T.rotate_90: 6,
                         T.transverse: 7}.get(self.transform, 0)
@@ -530,10 +517,9 @@ def camera_isp(name: str, dtype=f32):
                 if flip & 4:
                     turn_ok = shape[0] % 8 == 0 and shape[0] >= 16
                     in_pass = (turn_ok and tonemap == "reinhard" and out_dtype == u8 and not ids_format
-                               and os.environ.get("B200ISP_TURN_IN_PASS", "1") != "0"
-                               and ((isp_dtype == f16 and os.environ.get("B200ISP_CAM16_RECOMPUTE", "0") != "1")
+                               and (isp_dtype == f16
                                     or (isp_dtype == f32 and not self.reinhard_exact and float(color_adapt) == 0.0
-                                        and 0.3 <= float(gamma) <= 1.0 and os.environ.get("B200ISP_CAM32_ONE_SWEEP", "0") != "1")))
+                                        and 0.3 <= float(gamma) <= 1.0)))
                     if not (in_pass or (turn_ok and os.environ.get("B200ISP_FUSED_TRANSPOSE", "0") == "1")):
                         flip = 0
             return flip

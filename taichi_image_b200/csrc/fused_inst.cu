@@ -5,8 +5,8 @@
 
 namespace isp {
 #ifdef ISP_INST_RMAX
-template int run_rmax<ISP_INST_CAM16 != 0>(const FramePtrs&, IspConsts, int, int, int, cudaStream_t);
-template int run_rstore<ISP_INST_CAM16 != 0>(const FramePtrs&, IspConsts, int, int, cudaStream_t, void*, void*, int);
+template int run_rmax<ISP_INST_CAM16 != 0>(const FramePtrs&, IspConsts, int, int, cudaStream_t);
+template int run_rstore<ISP_INST_CAM16 != 0>(const FramePtrs&, IspConsts, int, int, cudaStream_t, void*, void*);
 #else
 template int run_fused<ISP_INST_CAM16 != 0, ISP_INST_OUT>(const FramePtrs&, int, const b200isp_fused_params&, IspConsts, cudaStream_t);
 #endif

@@ -74,10 +74,6 @@ struct Packed12Loader2 {
   int frame0;
   int ids;               // 0: standard layout (packed.py:23-31), 1: IDS layout (packed.py:36-44), kernel-uniform
   static constexpr uint32_t kRowMask = 0x007FF800u;
-#ifndef ISP_S2_RING
-#define ISP_S2_RING 0      // measured on cfg2 (see stream2.cuh): register fetch 172 us; ring + 3x unroll 229 us; ring + 1 step 185 us
-#endif
-  static constexpr bool kRing = ISP_S2_RING != 0;     // K_CORE stages its rows through the cp.async ring (stream2.cuh)
   struct Raw { uint32_t w[5]; };
   struct Cursor { const uint32_t* p; uint32_t mL, mR; bool left, right, pf; };
 
@@ -791,10 +787,9 @@ struct EpiLinear2 {
   __device__ __forceinline__ void finish(State&, int, int, bool) const {}
 
   static constexpr bool kSplitEdge = FAST;
-#ifndef ISP_LINEAR_COMPACT
-#define ISP_LINEAR_COMPACT 1      // measured on cfg2: kernel alone 169 vs 171 us, step (sweep || metering) 197 vs 204 us
-#endif
-  static constexpr bool kCompactLoop = ISP_LINEAR_COMPACT != 0;
+  // single-step loop (stream2_rows), measured on cfg2 against the 3x unrolled one: kernel alone 169 vs 171 us, step
+  // (sweep || metering) 197 vs 204 us
+  static constexpr bool kCompactLoop = true;
   template <bool GAMMA>
   __device__ __forceinline__ void emit_t(const State& st, int row, const Vals24& x) const {
     uint32_t v[24];
@@ -1109,23 +1104,6 @@ struct Packed12Sampler {
 // apart, so a warp's loads are contiguous) and evaluates exactly the partial-sum formulas of the sweep,
 // i.e. the very value the sweep will produce for that pixel -- including the samples on the 2-pixel image
 // frame (row 0 / column 0), which use the same zero-sample + renormalisation scheme (border_fix.cuh).
-// The metering pass touches 5 of every 8 packed rows right before the sweep reads all of them: load them with
-// the L2 evict-last policy so the sweep finds them in the 126 MB L2 (its own output goes out evict-first).
-#ifndef ISP_METER_KEEP_L2
-#define ISP_METER_KEEP_L2 0      // measured on cfg2: no gain (533.9 vs 532.0 Gpx/s), kept as a build option
-#endif
-__device__ __forceinline__ uint32_t ldg_keep(const uint32_t* p) {
-#if ISP_METER_KEEP_L2
-  uint64_t pol;
-  uint32_t v;
-  asm("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(pol));
-  asm volatile("ld.global.nc.L2::cache_hint.b32 %0, [%1], %2;" : "=r"(v) : "l"(p), "l"(pol));
-  return v;
-#else
-  return __ldg(p);
-#endif
-}
-
 template <bool CAM16>
 struct Packed12FastSampler {
   Packed12Src<CAM16> src;
@@ -1202,11 +1180,11 @@ struct Packed12FastSampler {
 
   // interior sample: p = word of pixel (row, col) (col % 8 == 0)
   __device__ __forceinline__ void sample_fast(const uint32_t* p, int row, float (&rgb)[3]) const {
-    const uint32_t a0 = ldg_keep(p - 2 * pitch_words);                                   // row-2: col
-    const uint32_t bm = ldg_keep(p - pitch_words - 1), b0 = ldg_keep(p - pitch_words);      // row-1: col-1..col+1
-    const uint32_t cm = ldg_keep(p - 1), c0 = ldg_keep(p), c1 = ldg_keep(p + 1);               // row  : col-2..col+2
-    const uint32_t dm = ldg_keep(p + pitch_words - 1), d0 = ldg_keep(p + pitch_words);      // row+1
-    const uint32_t e0 = ldg_keep(p + 2 * pitch_words);                                   // row+2
+    const uint32_t a0 = __ldg(p - 2 * pitch_words);                                   // row-2: col
+    const uint32_t bm = __ldg(p - pitch_words - 1), b0 = __ldg(p - pitch_words);      // row-1: col-1..col+1
+    const uint32_t cm = __ldg(p - 1), c0 = __ldg(p), c1 = __ldg(p + 1);               // row  : col-2..col+2
+    const uint32_t dm = __ldg(p + pitch_words - 1), d0 = __ldg(p + pitch_words);      // row+1
+    const uint32_t e0 = __ldg(p + 2 * pitch_words);                                   // row+2
     float S[3], sc[3];
     bool brow, gsite;
     sums_from_words(a0, bm, b0, cm, c0, c1, dm, d0, e0, row, S, sc, brow, gsite);
@@ -1326,14 +1304,13 @@ static int launch_reinhard(const Packed12Loader2<CAM16, EXT>& ld, const FramePtr
 // EXT: the extended kernels (IDS layout in the row loader, flips in the store); Malvar only -- the host mirror routes
 // bilinear + IDS / flip through the re-pack pass / the transform kernel.
 template <bool CAM16, int MODE, typename OutT, bool EXT>
-static int run_pass_ext(const FramePtrs& fp, IspConsts k, int frame0, int nframes, int rows_per_task, cudaStream_t s,
-                        void* ev_start, void* ev_stop) {
-  k.frame0 = frame0;
+static int run_pass_ext(const FramePtrs& fp, IspConsts k, int nframes, int rows_per_task, cudaStream_t s, void* ev_start, void* ev_stop) {
+  k.frame0 = 0;
   const Stream2Geom g = make_geom2(k.H, k.W, nframes, rows_per_task, (EXT && MODE != MODE_RMAX && (k.flip & 4)) ? 8 : 2);
   const bool bl = !EXT && k.kbase != 0;
   if (EXT && k.kbase != 0) { set_error("process_packed12: the IDS layout / flips are fused for the Malvar demosaic only"); return B200ISP_E_ARG; }
   Packed12Loader2<CAM16, EXT> ld;
-  ld.fp = fp; ld.pitch_words = k.W * 3 / 8; ld.frame0 = frame0; ld.ids = k.ids;
+  ld.fp = fp; ld.pitch_words = k.W * 3 / 8; ld.frame0 = 0; ld.ids = k.ids;
   int st = B200ISP_OK;
   auto record = [&](void* ev) { record_profile_event(ev, s); };
   if (ev_start) record(ev_start);
@@ -1357,12 +1334,12 @@ static int run_pass_ext(const FramePtrs& fp, IspConsts k, int frame0, int nframe
 }
 
 template <bool CAM16, int MODE, typename OutT>
-static int run_pass(const FramePtrs& fp, IspConsts k, int frame0, int nframes, int rows_per_task, cudaStream_t s,
+static int run_pass(const FramePtrs& fp, IspConsts k, int nframes, int rows_per_task, cudaStream_t s,
                     void* ev_start = nullptr, void* ev_stop = nullptr) {
   // the max sweep stores nothing: it only needs the extended loader for IDS frames
   const bool ext = k.ids != 0 || (MODE != MODE_RMAX && k.flip != 0);
-  if (ext) return run_pass_ext<CAM16, MODE, OutT, true>(fp, k, frame0, nframes, rows_per_task, s, ev_start, ev_stop);
-  return run_pass_ext<CAM16, MODE, OutT, false>(fp, k, frame0, nframes, rows_per_task, s, ev_start, ev_stop);
+  if (ext) return run_pass_ext<CAM16, MODE, OutT, true>(fp, k, nframes, rows_per_task, s, ev_start, ev_stop);
+  return run_pass_ext<CAM16, MODE, OutT, false>(fp, k, nframes, rows_per_task, s, ev_start, ev_stop);
 }
 
 // ---------------------------------------------------------------- Camera16 Reinhard in ONE sweep + a light second pass
@@ -1446,7 +1423,7 @@ __global__ void __launch_bounds__(256) reinhard_map16_out_kernel(const FramePtrs
   if constexpr (!PITCHED) {
     // two 16-value chunks per iteration, the four 16-byte loads issued before the first use.  Measured on cfg3 (gamma 0.9):
     // 8 CTAs per SM 131 us, 4: 155 us, 2: slower still -- unlike a plain copy this pass wants every thread slot
-    // (profiles/r02_reinhard_map16.txt); B200ISP_MAP16_CTAS overrides
+    // (profiles/r02_reinhard_map16.txt)
     uint4* dst = reinterpret_cast<uint4*>(fp.out[frame]);
     const long long n16 = (long long)H * W * 3 / 16;                   // H even, W % 8 == 0
     for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n16; i += 2 * stride) {
@@ -1492,7 +1469,9 @@ __global__ void __launch_bounds__(256) reinhard_map16_out_kernel(const FramePtrs
 // maximum.  reinhard_lut_build_kernel evaluates that function once per pattern and frame with exactly the arithmetic of
 // reinhard_scratch_out_kernel / map16_pair (so the result is bit-identical to them); reinhard_lut_out_kernel keeps the frame's
 // 64 KB table in shared memory and turns every value into one LDS.U8: no MUFU (the arithmetic pass needs 6 per pixel and sits
-// at 74 % of the MUFU pipe), 10 instead of 21 instructions per pixel -- the pass becomes a plain HBM stream.
+// at 74 % of the MUFU pipe), 10 instead of 21 instructions per pixel -- the pass becomes a plain HBM stream.  run_fused
+// uses it for Camera16 only: the Camera32 pass (reinhard_map16_out_kernel) is bound by its 2 : 1 read / write DRAM stream
+// (4.75 TB/s), not by the MUFU pipe, and the table form measured 134.9 vs 131.5 us on cfg3.
 constexpr int kLutBytes = 65536;
 template <bool CAM16>
 __global__ void __launch_bounds__(256) reinhard_lut_build_kernel(uint8_t* lut /* n_frames x 65536 */, float gamma, const Workspace* ws) {
@@ -1713,13 +1692,13 @@ static int run_out_transposed(const FramePtrs& sc, const FramePtrs& fp, int n_fr
 // pass A for frames [0, nframes): instantiated once per ISP dtype (fused_inst.cu with ISP_INST_RMAX); Camera16 stores the f16
 // map (any color_adapt), Camera32 the u16 fixed-point map (color_adapt == 0 only: the caller checks)
 template <bool CAM16>
-int run_rstore(const FramePtrs& fp_scratch, IspConsts k, int nframes, int rows_per_task, cudaStream_t s, void* ev_start, void* ev_stop, int frame0) {
-  k.frame0 = frame0;
+int run_rstore(const FramePtrs& fp_scratch, IspConsts k, int nframes, int rows_per_task, cudaStream_t s, void* ev_start, void* ev_stop) {
+  k.frame0 = 0;
   const Stream2Geom g = make_geom2(k.H, k.W, nframes, rows_per_task);
   int st = B200ISP_OK;
   if (ev_start) record_profile_event(ev_start, s);
   auto launch = [&](auto ld, bool bl) -> int {
-    ld.fp = fp_scratch; ld.pitch_words = k.W * 3 / 8; ld.frame0 = frame0; ld.ids = k.ids;
+    ld.fp = fp_scratch; ld.pitch_words = k.W * 3 / 8; ld.frame0 = 0; ld.ids = k.ids;
     ISP_DISPATCH_PATTERN(k.pattern, P, {
       if (k.ca == 0.f) { EpiReinhardMax2<CAM16, true, true> e{fp_scratch, k}; st = launch_stream2<P>(ld, e, g, s, "isp_stream<reinhard_store>", bl); }
       else if constexpr (CAM16) { EpiReinhardMax2<true, false, true> e{fp_scratch, k}; st = launch_stream2<P>(ld, e, g, s, "isp_stream<reinhard_store>", bl); }
@@ -1742,39 +1721,13 @@ int run_rstore(const FramePtrs& fp_scratch, IspConsts k, int nframes, int rows_p
 // launches of CTAs that exit immediately.
 int run_rmax_gated(const FramePtrs& fp, IspConsts k, int nframes, int rows_per_task, cudaStream_t s);
 
-// frame-global Reinhard max for frames [frame0, frame0 + nframes): independent of the output dtype,
-// instantiated once per ISP dtype (fused_inst.cu with ISP_INST_RMAX)
+// frame-global Reinhard max: independent of the output dtype, instantiated once per ISP dtype (fused_inst.cu with ISP_INST_RMAX)
 template <bool CAM16>
-int run_rmax(const FramePtrs& fp, IspConsts k, int frame0, int nframes, int rows_per_task, cudaStream_t s) {
-  return run_pass<CAM16, MODE_RMAX, uint8_t>(fp, k, frame0, nframes, rows_per_task, s);
+int run_rmax(const FramePtrs& fp, IspConsts k, int nframes, int rows_per_task, cudaStream_t s) {
+  return run_pass<CAM16, MODE_RMAX, uint8_t>(fp, k, nframes, rows_per_task, s);
 }
 
 int run_write_gated(const FramePtrs& fp, IspConsts k, int nframes, int rows_per_task, cudaStream_t s);
-// library-owned high-priority side stream + fork / join events, one set per device (created on first use, never destroyed)
-struct SideStream { cudaStream_t stream; cudaEvent_t ev[2 * B200ISP_MAX_FRAMES]; };
-SideStream* side_stream();
-// B200ISP_MAP16_OVERLAP: frame groups of the overlapped one-sweep Reinhard form (0 / 1 = off); B200ISP_MAP16_OVERLAP_CTAS: CTAs
-// per SM of the normalise pass while it runs under a sweep
-static inline int map16_overlap_groups(int n_frames) {
-  static const int want = [] { const char* e = getenv("B200ISP_MAP16_OVERLAP"); return e ? atoi(e) : 1; }();      // measured: does not pay
-  if (want <= 1 || n_frames < 4) return 1;
-  return std::min(want, n_frames / 2);
-}
-static inline int map16_overlap_ctas() {
-  static const int v = [] { const char* e = getenv("B200ISP_MAP16_OVERLAP_CTAS"); const int x = e ? atoi(e) : 0; return x > 0 ? x : 2; }();
-  return v;
-}
-// B200ISP_REINHARD_LUT: 0 = arithmetic normalise pass everywhere, 1 (default) = table pass for Camera16, 2 = also for Camera32
-// (A/B measurements; the results are bit-identical)
-static inline int lut_pass_mode() {
-  static const int mode = [] { const char* e = getenv("B200ISP_REINHARD_LUT"); return e ? atoi(e) : 1; }();
-  return mode;
-}
-
-// one-sweep Camera32 Reinhard, exact-integer experiment (reinhard_u16.cuh / reinhard_u16.cu)
-size_t reinhard_u16_frame_bytes(int H, int W);
-template <typename OutT>
-int run_reinhard_u16(const FramePtrs& fp, int n_frames, const b200isp_fused_params& p, IspConsts k, cudaStream_t s);
 
 template <bool CAM16, typename OutT>
 int run_fused(const FramePtrs& fp, int n_frames, const b200isp_fused_params& p, IspConsts k, cudaStream_t s) {
@@ -1789,16 +1742,14 @@ int run_fused(const FramePtrs& fp, int n_frames, const b200isp_fused_params& p, 
   }
   constexpr bool kIspOut = (CAM16 && std::is_same<OutT, __half>::value) || (!CAM16 && std::is_same<OutT, float>::value);
   if (p.tonemap == B200ISP_TM_NONE) {
-    if constexpr (kIspOut) return run_pass<CAM16, MODE_RGB, OutT>(fp, k, 0, n_frames, rpt, s, p.profile_start, p.profile_stop);
+    if constexpr (kIspOut) return run_pass<CAM16, MODE_RGB, OutT>(fp, k, n_frames, rpt, s, p.profile_start, p.profile_stop);
     else { set_error("process_packed12: TM_NONE writes the ISP dtype"); return B200ISP_E_DTYPE; }
   }
   if constexpr (std::is_same<OutT, float>::value) {
     set_error("process_packed12: tone-mapped output must be u8, u16 or f16");
     return B200ISP_E_DTYPE;
   } else {
-    if (p.tonemap == B200ISP_TM_LINEAR) return run_pass<CAM16, MODE_LINEAR, OutT>(fp, k, 0, n_frames, rpt, s, p.profile_start, p.profile_stop);
-    // Reinhard: the second sweep should find the packed frames in L2 -> interleave max / write passes
-    // per group of frames whose packed bytes stay well inside the 126 MB L2.
+    if (p.tonemap == B200ISP_TM_LINEAR) return run_pass<CAM16, MODE_LINEAR, OutT>(fp, k, n_frames, rpt, s, p.profile_start, p.profile_stop);
     // frame_max and frame_max2 are adjacent in the workspace: one memset node
     static_assert(offsetof(Workspace, frame_max2) == offsetof(Workspace, frame_max) + sizeof(float) * B200ISP_MAX_FRAMES, "adjacent");
     int st = cuda_status(cudaMemsetAsync(k.ws->frame_max, 0, sizeof(float) * 2 * B200ISP_MAX_FRAMES, s), "memset frame_max");
@@ -1815,7 +1766,7 @@ int run_fused(const FramePtrs& fp, int n_frames, const b200isp_fused_params& p, 
         IspConsts kp = k;            // the map is a plain dense (H, W, 3) image whatever the output looks like
         kp.flip = 0;
         kp.orow = 3 * k.W;
-        st = run_rstore<true>(sc, kp, n_frames, rpt, s, p.profile_start, p.profile_stop, 0);
+        st = run_rstore<true>(sc, kp, n_frames, rpt, s, p.profile_start, p.profile_stop);
         if (st) return st;
         if (turned) return run_out_transposed<true>(sc, fp, n_frames, k, s);     // the normalise pass turns the image
         if (p.out_yuv420) {
@@ -1825,7 +1776,7 @@ int run_fused(const FramePtrs& fp, int n_frames, const b200isp_fused_params& p, 
         }
         const long long n_elems = (long long)k.H * k.W * 3;
         if constexpr (std::is_same<OutT, uint8_t>::value) {
-          if (k.gamma != 1.0f && p.reinhard_scratch_bytes >= need + (size_t)n_frames * kLutBytes && lut_pass_mode() >= 1)
+          if (k.gamma != 1.0f && p.reinhard_scratch_bytes >= need + (size_t)n_frames * kLutBytes)
             return run_lut_pass<true>(sc, fp, n_frames, n_elems, (uint8_t*)p.reinhard_scratch + need, k.gamma, k.ws, s);
         }
         const dim3 grid((unsigned)std::min<long long>((n_elems / 8 + 255) / 256, 4 * kNumSMs), (unsigned)n_frames);
@@ -1838,11 +1789,11 @@ int run_fused(const FramePtrs& fp, int n_frames, const b200isp_fused_params& p, 
       // (6 B/px scratch) + an element-wise normalise / gamma / quantise pass.  The second demosaic of the two-sweep form
       // (66 of its 106 instructions per pixel) disappears; the u8 result is within 1 LSB of the two-sweep result
       // (measured: profiles/r02_reinhard_map16.txt).  Frames whose map does not fit [0, 1) (reinhard_map16_declined) are
-      // redone exactly by the gated sweeps.  reinhard_mode 1 forces the exact two-sweep form.
+      // redone exactly by the gated sweeps.  Any reinhard_mode other than 0 forces the exact two-sweep form.
       const size_t need = (size_t)n_frames * k.H * k.W * 3 * sizeof(uint16_t);
       const bool turned = (k.flip & 4) && k.orow % 8 == 0;
       if (p.reinhard_mode == 0 && k.ca == 0.f && k.gamma <= 1.0f && k.gamma >= 0.3f && !p.out_yuv420 && (k.flip == 0 || turned) && k.ids == 0 &&
-          p.reinhard_scratch && p.reinhard_scratch_bytes >= need && p.reinhard_group <= 0) {
+          p.reinhard_scratch && p.reinhard_scratch_bytes >= need) {
         FramePtrs sc = fp;
         for (int f = 0; f < n_frames; ++f) sc.out[f] = (char*)p.reinhard_scratch + (size_t)f * k.H * k.W * 3 * sizeof(uint16_t);
         if (turned) {
@@ -1851,7 +1802,7 @@ int run_fused(const FramePtrs& fp, int n_frames, const b200isp_fused_params& p, 
           IspConsts kp = k;
           kp.flip = 0;
           kp.orow = 3 * k.W;
-          st = run_rstore<false>(sc, kp, n_frames, rpt, s, p.profile_start, p.profile_stop, 0);
+          st = run_rstore<false>(sc, kp, n_frames, rpt, s, p.profile_start, p.profile_stop);
           if (st) return st;
           kp.gate = 1;
           st = run_rmax_gated(sc, kp, n_frames, rpt, s);
@@ -1860,57 +1811,18 @@ int run_fused(const FramePtrs& fp, int n_frames, const b200isp_fused_params& p, 
           if (st) return st;
           return run_out_transposed<false>(sc, fp, n_frames, k, s);
         }
+        // the normalise pass runs after the sweep with 8 CTAs per SM; running it under the sweep on a side stream measured
+        // 212-186 vs 215 Gpixel/s on cfg3 (profiles/r02_reinhard_map16.txt)
+        st = run_rstore<false>(sc, k, n_frames, rpt, s, p.profile_start, p.profile_stop);
+        if (st) return st;
         const long long n_elems = (long long)k.H * k.W * 3;
-        static const int ctas_per_sm = [] { const char* e = getenv("B200ISP_MAP16_CTAS"); const int v = e ? atoi(e) : 0; return v > 0 ? v : 8; }();
         const bool gam = k.gamma != 1.0f, pitched = k.orow != 3 * k.W;
-        auto pass_b = [&](int f0, int nf, int per_sm, cudaStream_t ps) -> int {
-          const dim3 grid((unsigned)std::min<long long>((n_elems / 16 + 255) / 256, (per_sm * kNumSMs + nf - 1) / nf), (unsigned)nf);
-          if (gam && pitched) reinhard_map16_out_kernel<true, true><<<grid, 256, 0, ps>>>(sc, fp, k.H, k.W, k.orow, k.gamma, k.ws, f0);
-          else if (gam) reinhard_map16_out_kernel<true, false><<<grid, 256, 0, ps>>>(sc, fp, k.H, k.W, k.orow, k.gamma, k.ws, f0);
-          else if (pitched) reinhard_map16_out_kernel<false, true><<<grid, 256, 0, ps>>>(sc, fp, k.H, k.W, k.orow, k.gamma, k.ws, f0);
-          else reinhard_map16_out_kernel<false, false><<<grid, 256, 0, ps>>>(sc, fp, k.H, k.W, k.orow, k.gamma, k.ws, f0);
-          return cuda_status(cudaPeekAtLastError(), "reinhard_map16_out_kernel");
-        };
-        // Overlapped form -- EXPERIMENT, off by default (B200ISP_MAP16_OVERLAP=<groups>; profiles/r02_reinhard_map16.txt: cfg3
-        // 215 Gpixel/s serial, 212 / 208 / 203 / 186 with 2 or 3 groups and 1-3 CTAs of the pass per SM -- the pass takes the
-        // residency and the issue slots it uses away from the sweep, and the look-ahead metering already fills the idle ones).
-        // >= 4 frames, no profiling events: the frames are cut into groups; the normalise pass of group g runs
-        // on a high-priority side stream UNDER the map sweep of group g + 1 with a small grid (the sweep is bound by issue
-        // slots and fills the register file, the pass by MUFU / memory: a few of its CTAs per SM take one sweep CTA's place and
-        // use what the sweep leaves idle); the last group's pass runs alone with the full grid.  Fork / join through events,
-        // so the call stays one stream-ordered unit and is CUDA-graph capturable.
-        const int groups = (p.profile_start || p.profile_stop) ? 1 : map16_overlap_groups(n_frames);
-        if (groups > 1) {
-          SideStream* side = side_stream();
-          if (!side) return B200ISP_E_CUDA;
-          const int per = (n_frames + groups - 1) / groups;
-          int g = 0;
-          for (int f0 = 0; f0 < n_frames; f0 += per, ++g) {
-            const int nf = std::min(per, n_frames - f0);
-            st = run_rstore<false>(sc, k, nf, rpt, s, nullptr, nullptr, f0);
-            if (st) return st;
-            if (f0 + nf < n_frames) {
-              if ((st = cuda_status(cudaEventRecord(side->ev[2 * g], s), "event record"))) return st;
-              if ((st = cuda_status(cudaStreamWaitEvent(side->stream, side->ev[2 * g], 0), "stream wait"))) return st;
-              if ((st = pass_b(f0, nf, map16_overlap_ctas(), side->stream))) return st;
-              if ((st = cuda_status(cudaEventRecord(side->ev[2 * g + 1], side->stream), "event record"))) return st;
-            } else {
-              if ((st = pass_b(f0, nf, ctas_per_sm, s))) return st;
-            }
-          }
-          for (int j = 0; j + 1 < g; ++j)
-            if ((st = cuda_status(cudaStreamWaitEvent(s, side->ev[2 * j + 1], 0), "stream wait"))) return st;
-        } else {
-          st = run_rstore<false>(sc, k, n_frames, rpt, s, p.profile_start, p.profile_stop, 0);
-          if (st) return st;
-          // the table form of the pass (run_lut_pass) is opt-in here: measured 134.9 vs 131.5 us on cfg3 -- this pass is bound by
-          // its 2 : 1 read / write DRAM stream (4.75 TB/s), not by the MUFU pipe; Camera16 (scalar f16 arithmetic) gains 2 %
-          if (gam && !pitched && p.reinhard_scratch_bytes >= need + (size_t)n_frames * kLutBytes && lut_pass_mode() == 2)
-            st = run_lut_pass<false>(sc, fp, n_frames, n_elems, (uint8_t*)p.reinhard_scratch + need, k.gamma, k.ws, s);
-          else
-            st = pass_b(0, n_frames, ctas_per_sm, s);
-          if (st) return st;
-        }
+        const dim3 grid((unsigned)std::min<long long>((n_elems / 16 + 255) / 256, (8 * kNumSMs + n_frames - 1) / n_frames), (unsigned)n_frames);
+        if (gam && pitched) reinhard_map16_out_kernel<true, true><<<grid, 256, 0, s>>>(sc, fp, k.H, k.W, k.orow, k.gamma, k.ws, 0);
+        else if (gam) reinhard_map16_out_kernel<true, false><<<grid, 256, 0, s>>>(sc, fp, k.H, k.W, k.orow, k.gamma, k.ws, 0);
+        else if (pitched) reinhard_map16_out_kernel<false, true><<<grid, 256, 0, s>>>(sc, fp, k.H, k.W, k.orow, k.gamma, k.ws, 0);
+        else reinhard_map16_out_kernel<false, false><<<grid, 256, 0, s>>>(sc, fp, k.H, k.W, k.orow, k.gamma, k.ws, 0);
+        if ((st = cuda_status(cudaPeekAtLastError(), "reinhard_map16_out_kernel"))) return st;
         IspConsts kg = k;
         kg.gate = 1;
         st = run_rmax_gated(fp, kg, n_frames, rpt, s);
@@ -1918,31 +1830,18 @@ int run_fused(const FramePtrs& fp, int n_frames, const b200isp_fused_params& p, 
         return run_write_gated(fp, kg, n_frames, rpt, s);
       }
     }
-    if constexpr (!CAM16) {
-      // EXPERIMENT (reinhard_mode 2): Camera32 without colour correction, color_adapt == 0: ONE sweep that also stores the exact
-      // integer RGB (3 x u16 per pixel) + an element-wise map / normalise / quantise pass (reinhard_u16.cuh)
-      if (p.reinhard_mode == 2 && !k.ccm && k.ca == 0.f && !p.out_yuv420 && k.flip == 0 && k.ids == 0 && k.H >= 4 && k.W >= 8 && p.reinhard_scratch &&
-          p.reinhard_scratch_bytes >= (size_t)n_frames * reinhard_u16_frame_bytes(k.H, k.W))
-        return run_reinhard_u16<OutT>(fp, n_frames, p, k, s);
-    }
     // Camera32 (or no scratch): max sweep, then the write sweep recomputes the map.  Both sweeps are bound by
     // instruction issue, not by DRAM, so the second read of the packed frames (1.5 B/px) is cheaper than cutting the
     // call into L2-sized groups whose short launches end in idle tails (measured, profiles/r02_reinhard_diet.txt).
-    int group = p.reinhard_group > 0 ? p.reinhard_group : n_frames;
-    for (int f = 0; f < n_frames; f += group) {
-      const int n = (n_frames - f < group) ? n_frames - f : group;
-      st = run_rmax<CAM16>(fp, k, f, n, rpt, s);
-      if (st) return st;
-      st = run_pass<CAM16, MODE_REINHARD, OutT>(fp, k, f, n, rpt, s, f == 0 ? p.profile_start : nullptr, f == 0 ? p.profile_stop : nullptr);
-      if (st) return st;
-    }
-    return B200ISP_OK;
+    st = run_rmax<CAM16>(fp, k, n_frames, rpt, s);
+    if (st) return st;
+    return run_pass<CAM16, MODE_REINHARD, OutT>(fp, k, n_frames, rpt, s, p.profile_start, p.profile_stop);
   }
 }
 
-extern template int run_rstore<true>(const FramePtrs&, IspConsts, int, int, cudaStream_t, void*, void*, int);
-extern template int run_rstore<false>(const FramePtrs&, IspConsts, int, int, cudaStream_t, void*, void*, int);
-extern template int run_rmax<true>(const FramePtrs&, IspConsts, int, int, int, cudaStream_t);
-extern template int run_rmax<false>(const FramePtrs&, IspConsts, int, int, int, cudaStream_t);
+extern template int run_rstore<true>(const FramePtrs&, IspConsts, int, int, cudaStream_t, void*, void*);
+extern template int run_rstore<false>(const FramePtrs&, IspConsts, int, int, cudaStream_t, void*, void*);
+extern template int run_rmax<true>(const FramePtrs&, IspConsts, int, int, cudaStream_t);
+extern template int run_rmax<false>(const FramePtrs&, IspConsts, int, int, cudaStream_t);
 
 }  // namespace isp

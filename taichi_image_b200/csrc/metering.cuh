@@ -420,13 +420,12 @@ inline int meter_grid(long long n) {
 
 // Grid of the two-launch (look-ahead / shared) form, which runs on a high-priority side stream UNDER the previous batch's
 // sweep: its CTAs take SM slots away from the sweep for as long as they live, so a latency-bound sampler should not
-// flood the GPU.  Samplers may define kSideGridCap (CTAs); B200ISP_METER_GRID_CAP overrides it (tuning knob).
+// flood the GPU.  Samplers may define kSideGridCap (CTAs).
 template <class Sampler, class = void> struct side_grid_cap { static constexpr int value = 4 * kNumSMs; };
 template <class Sampler> struct side_grid_cap<Sampler, std::enable_if_t<(Sampler::kSideGridCap > 0)>> { static constexpr int value = Sampler::kSideGridCap; };
 template <class Sampler>
 inline int meter_side_grid(long long n) {
-  int cap = side_grid_cap<Sampler>::value;
-  if (const char* e = getenv("B200ISP_METER_GRID_CAP")) { const int v = atoi(e); if (v > 0) cap = v; }
+  const int cap = side_grid_cap<Sampler>::value;
   const int g = meter_grid(n);
   return g < cap ? g : cap;
 }

@@ -356,9 +356,8 @@ int run_demosaic_sweep_impl(const void* bayer, void* rgb, int H, int W, int patt
   epi.out = (T*)rgb; epi.H = H; epi.W = W; epi.ccm = ccm != nullptr; epi.kbase = bilinear ? kBilinearBase : 0;
   for (int i = 0; i < 9; ++i) epi.m[i] = ccm ? ccm[i] : 0.f;
   // one frame per call: 16-row chunks (measured at 8K, profiles/r02_plane_sweep.txt: 12-16 rows best for u8 / u16 / f32,
-  // 24+ rows lose 5-10 % to the tail of the last wave).  B200ISP_PLANE_RPT: tuning knob of scripts/plane_rpt_sweep.py
-  const char* env = getenv("B200ISP_PLANE_RPT");
-  const Stream2Geom g = make_geom2(H, W, 1, env ? atoi(env) : 16);
+  // 24+ rows lose 5-10 % to the tail of the last wave)
+  const Stream2Geom g = make_geom2(H, W, 1, 16);
   int st = B200ISP_OK;
   ISP_DISPATCH_PATTERN(pattern, P, { st = launch_stream2<P>(ld, epi, g, s, "bayer_to_rgb", bilinear); });
   return st;

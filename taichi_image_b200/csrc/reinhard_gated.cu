@@ -32,22 +32,4 @@ int run_write_gated(const FramePtrs& fp, IspConsts k, int nframes, int rows_per_
   return st;
 }
 
-
-// side stream of the overlapped one-sweep form (fused_isp.cuh, run_fused)
-SideStream* side_stream() {
-  static SideStream res[64];
-  static bool ready[64] = {};
-  int dev = 0;
-  if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) { set_error("side_stream: no current device"); return nullptr; }
-  if (!ready[dev]) {
-    int lo = 0, hi = 0;
-    cudaDeviceGetStreamPriorityRange(&lo, &hi);          // hi = numerically lowest = greatest priority
-    if (cudaStreamCreateWithPriority(&res[dev].stream, cudaStreamNonBlocking, hi) != cudaSuccess) { set_error("side_stream: stream creation failed"); return nullptr; }
-    for (auto& e : res[dev].ev)
-      if (cudaEventCreateWithFlags(&e, cudaEventDisableTiming) != cudaSuccess) { set_error("side_stream: event creation failed"); return nullptr; }
-    ready[dev] = true;
-  }
-  return &res[dev];
-}
-
 }  // namespace isp

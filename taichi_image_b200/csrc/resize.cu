@@ -359,16 +359,13 @@ extern "C" int b200isp_transform(const void* src, void* dst, int dtype, int src_
   // 3- / 6-byte pixels, both extents multiples of 8, vector-aligned bases: whole-word pixel tiles (transform_turn_kernel)
   if (swaps && (pb == 3 || pb == 6) && src_h % 8 == 0 && src_w % 8 == 0 &&
       ((reinterpret_cast<uintptr_t>(src) | reinterpret_cast<uintptr_t>(dst)) & (pb == 3 ? 7u : 15u)) == 0) {
-    static const bool off = [] { const char* e = getenv("B200ISP_TRANSFORM_TURN"); return e && atoi(e) == 0; }();   // A/B measurements
-    if (!off) {
-      const int mr = (transform == B200ISP_T_ROT90 || transform == B200ISP_T_TRANSVERSE) ? 1 : 0;
-      const int mc = (transform == B200ISP_T_ROT270 || transform == B200ISP_T_TRANSVERSE) ? 1 : 0;
-      const dim3 grid((src_h + kTurnRows - 1) / kTurnRows, (src_w + kTurnCols - 1) / kTurnCols);
-      if (pb == 3) transform_turn_kernel<3><<<grid, 256, 0, s>>>((const uint8_t*)src, (uint8_t*)dst, src_h, src_w, mr, mc);
-      else transform_turn_kernel<6><<<grid, 256, 0, s>>>((const uint8_t*)src, (uint8_t*)dst, src_h, src_w, mr, mc);
-      ISP_LAUNCH_CHECK("transform_turn_kernel");
-      return B200ISP_OK;
-    }
+    const int mr = (transform == B200ISP_T_ROT90 || transform == B200ISP_T_TRANSVERSE) ? 1 : 0;
+    const int mc = (transform == B200ISP_T_ROT270 || transform == B200ISP_T_TRANSVERSE) ? 1 : 0;
+    const dim3 grid((src_h + kTurnRows - 1) / kTurnRows, (src_w + kTurnCols - 1) / kTurnCols);
+    if (pb == 3) transform_turn_kernel<3><<<grid, 256, 0, s>>>((const uint8_t*)src, (uint8_t*)dst, src_h, src_w, mr, mc);
+    else transform_turn_kernel<6><<<grid, 256, 0, s>>>((const uint8_t*)src, (uint8_t*)dst, src_h, src_w, mr, mc);
+    ISP_LAUNCH_CHECK("transform_turn_kernel");
+    return B200ISP_OK;
   }
   if (words) {
     const uint32_t* sw = (const uint32_t*)src;

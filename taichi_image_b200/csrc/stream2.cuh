@@ -26,8 +26,8 @@
 // masks the halo columns of the first / last thread column.  Six full pair rows form the window.  The shipped
 // loop is ONE copy of the two-row step that slides the window with register moves (+4 MOV per pixel): rotating the
 // rows by unrolling the step three times needs no moves but triples the hot code, and the sweep is instruction-cache
-// bound before it is move bound (DESIGN 6c: 3x unrolled 171 us vs single step 162 us on cfg2).  The unrolled forms
-// remain behind Epi::kCompactLoop == false / ISP_S2_COMPACT_UNROLL (experiments, see experiments.cuh).
+// bound before it is move bound (DESIGN 6c: 3x unrolled 171 us vs single step 162 us on cfg2).  Epilogues with
+// Epi::kCompactLoop == false (the small RGB epilogue of TM_NONE) keep the three-copy form outside K_GENERAL.
 #pragma once
 #include "stream_engine.cuh"
 
@@ -263,41 +263,20 @@ __device__ __forceinline__ void stream2_rows(const Loader& ld, const Epi& epi, t
     epi.template emit<!BROW0, !GFIRST0, KIND>(st, row_ + 1, R_, G_, B_);                                        \
   }
 
-#ifndef ISP_S2_SLIDE_FADD2
-#define ISP_S2_SLIDE_FADD2 1
-#endif
-#ifndef ISP_S2_COMPACT_UNROLL
-#define ISP_S2_COMPACT_UNROLL 1     // measured: 1 step 607 / 147 Gpx/s (cfg2 / cfg3), 2 steps 585 / 120 -- code size beats moves
-#endif
-  if constexpr (KIND == K_GENERAL || BL || (Epi::kCompactLoop && ISP_S2_COMPACT_UNROLL == 1)) {
+  if constexpr (KIND == K_GENERAL || BL || Epi::kCompactLoop) {
     // cold kind, or an epilogue so large that three copies of the step overflow the instruction cache (Reinhard:
     // 51 KB hot, no_instruction 3.1 cycles per issue): one copy of the step, the window slides by register moves
+    // (measured: 1 step 607 / 147 Gpx/s (cfg2 / cfg3), 2 steps 585 / 120 -- code size beats moves).
     // The slide as packed additions of -0.0 (exact identity for every float): one FADD2 moves a register PAIR, and because
     // the result is a fresh value ptxas gives it the loop-carried register directly -- a plain copy costs two MOVs per pair
-    // (64 per step = 4 per pixel; ISP_S2_SLIDE_FADD2=0 restores them).  ptxas does not fold the addition away.
+    // (64 per step = 4 per pixel).  ptxas does not fold the addition away.
 #pragma unroll 1
     for (int row = r0; row < rend; row += 2) {
       ISP_STEP(0, row);
 #pragma unroll
       for (int k = 0; k < 4; ++k)
 #pragma unroll
-        for (int i = 0; i < 8; ++i) {
-#if ISP_S2_SLIDE_FADD2
-          W[k][i] = add2(W[k + 2][i], bc(-0.0f));
-#else
-          W[k][i] = W[k + 2][i];
-#endif
-        }
-    }
-  } else if constexpr (Epi::kCompactLoop) {
-    // two copies of the step: half the register moves of the single-step form, two thirds of the unrolled code
-#pragma unroll 1
-    for (int row = r0; row < rend; row += 4) {
-      ISP_STEP(0, row);
-      if (row + 2 >= rend) break;
-      ISP_STEP(1, row + 2);
-#pragma unroll
-      for (int i = 0; i < 8; ++i) { W[2][i] = W[0][i]; W[3][i] = W[1][i]; W[0][i] = W[4][i]; W[1][i] = W[5][i]; }
+        for (int i = 0; i < 8; ++i) W[k][i] = add2(W[k + 2][i], bc(-0.0f));
     }
   } else {
 #pragma unroll 1
@@ -312,27 +291,10 @@ __device__ __forceinline__ void stream2_rows(const Loader& ld, const Epi& epi, t
 #undef ISP_STEP
 }
 
-// Experiments that did not ship (shared-memory row rings filled by cp.async / by TMA bulk copies) live in experiments.cuh,
-// compiled in only with -DISP_S2_RING=1|2.
-#ifndef ISP_S2_RING
-#define ISP_S2_RING 0
-#endif
-#if ISP_S2_RING
-}  // namespace isp
-#include "experiments.cuh"
-namespace isp {
-#else
-constexpr int kRingStages = 1;
-constexpr int kRowSlotWords = 1;
-#endif
-
 // Epi::kGated: the epilogue can decline whole frames at run time (enabled(frame), warp-uniform) -- the gated fallback sweeps
 // of the one-sweep Reinhard path (fused_isp.cuh); every other epilogue has no such member and no such code.
 template <class Epi, class = void> struct has_gate { static constexpr bool value = false; };
 template <class Epi> struct has_gate<Epi, std::enable_if_t<Epi::kGated>> { static constexpr bool value = true; };
-
-template <class Loader, class = void> struct has_ring { static constexpr bool value = false; };
-template <class Loader> struct has_ring<Loader, std::enable_if_t<Loader::kRing>> { static constexpr bool value = true; };
 
 // BL: bilinear demosaic instead of Malvar-He-Cutler.  The bilinear kernels have no K_CORE copy of the loop and use
 // the single-step body (their binary stays small; the arithmetic saved is hidden behind the same DRAM traffic).
@@ -373,10 +335,6 @@ __device__ __forceinline__ void stream2_task(const Loader& ld, const Epi& epi, c
   wc.stage = stage_warp;
 
   constexpr bool kSplit = Epi::kSplitEdge && !BL;
-  constexpr bool kUseRing = has_ring<Loader>::value && kSplit;
-#if ISP_S2_RING
-  __shared__ __align__(16) uint32_t ring[kUseRing ? kS2Warps * kRingWarpWords : 4];
-#endif
 
   typename Epi::State st;
   epi.init(st, frame, tcol, wc);
@@ -385,15 +343,7 @@ __device__ __forceinline__ void stream2_task(const Loader& ld, const Epi& epi, c
     const int kind = (border || !epi.fast_kinds_ok(st)) ? K_GENERAL
                      : ((!kSplit || strip == 0 || strip == g.warps_per_row - 1) ? K_EDGE : K_CORE);
     if constexpr (kSplit) {
-      if (kind == K_CORE) {
-#if ISP_S2_RING
-        if constexpr (kUseRing)
-          stream2_rows_ring<BROW0, GFIRST0>(ld, epi, st, g, frame, tcol, r0, rend,
-                                            ring + (threadIdx.x >> 5) * kRingWarpWords);
-        else
-#endif
-          stream2_rows<BROW0, GFIRST0, K_CORE, BL>(ld, epi, st, g, frame, tcol, r0, rend);
-      }
+      if (kind == K_CORE) stream2_rows<BROW0, GFIRST0, K_CORE, BL>(ld, epi, st, g, frame, tcol, r0, rend);
     }
     if (kind == K_EDGE) stream2_rows<BROW0, GFIRST0, K_EDGE, BL>(ld, epi, st, g, frame, tcol, r0, rend);
     else if (kind == K_GENERAL) stream2_rows<BROW0, GFIRST0, K_GENERAL, BL>(ld, epi, st, g, frame, tcol, r0, rend);

@@ -81,37 +81,17 @@ struct WarpCtx {
 // Output rows are written once and never re-read by the ISP: store them with the evict-first policy so that
 // they do not push the packed input rows (which the metering pass has just pulled into the 126 MB L2 and the
 // sweep is about to read) out of L2.
-#ifndef ISP_STREAMING_STORES
-#define ISP_STREAMING_STORES 1
-#endif
-__device__ __forceinline__ void st_out(uint4* p, const uint4& v) {
-#if ISP_STREAMING_STORES
-  __stcs(p, v);
-#else
-  *p = v;
-#endif
-}
-__device__ __forceinline__ void st_out(uint2* p, const uint2& v) {
-#if ISP_STREAMING_STORES
-  __stcs(p, v);
-#else
-  *p = v;
-#endif
-}
+__device__ __forceinline__ void st_out(uint4* p, const uint4& v) { __stcs(p, v); }
+__device__ __forceinline__ void st_out(uint2* p, const uint2& v) { __stcs(p, v); }
 // the same store executed only where idx < n, as ONE predicated instruction: written in C (`if (idx < n) st_out(...)`) the
 // compiler sinks the shared-memory load and the address arithmetic into the condition and branches over them -- BSSY + BRA +
 // BSYNC per store, 9 instructions per row in every sweep without a K_CORE copy (ncu source view of the Reinhard map sweep)
-#if ISP_STREAMING_STORES
-#define ISP_ST_OUT_OP "st.global.cs"
-#else
-#define ISP_ST_OUT_OP "st.global"
-#endif
 __device__ __forceinline__ void st_out_lt(uint4* p, const uint4& v, int idx, int n) {
-  asm volatile("{\n\t.reg .pred q;\n\tsetp.lt.s32 q, %5, %6;\n\t@q " ISP_ST_OUT_OP ".v4.u32 [%0], {%1, %2, %3, %4};\n\t}"
+  asm volatile("{\n\t.reg .pred q;\n\tsetp.lt.s32 q, %5, %6;\n\t@q st.global.cs.v4.u32 [%0], {%1, %2, %3, %4};\n\t}"
                :: "l"(p), "r"(v.x), "r"(v.y), "r"(v.z), "r"(v.w), "r"(idx), "r"(n) : "memory");
 }
 __device__ __forceinline__ void st_out_lt(uint2* p, const uint2& v, int idx, int n) {
-  asm volatile("{\n\t.reg .pred q;\n\tsetp.lt.s32 q, %3, %4;\n\t@q " ISP_ST_OUT_OP ".v2.u32 [%0], {%1, %2};\n\t}"
+  asm volatile("{\n\t.reg .pred q;\n\tsetp.lt.s32 q, %3, %4;\n\t@q st.global.cs.v2.u32 [%0], {%1, %2};\n\t}"
                :: "l"(p), "r"(v.x), "r"(v.y), "r"(idx), "r"(n) : "memory");
 }
 

@@ -148,28 +148,6 @@ def test_map16_overlapped_groups(cuda, n):
             assert_close_int(to_np(g), e, 1, f"oracle, step {step} frame {i}")
 
 
-def test_map16_overlapped_form_in_a_subprocess(cuda):
-    """the experiment switch B200ISP_MAP16_OVERLAP is read once per process: run the overlapped form (2 groups, normalise pass of
-    group 0 on the library's side stream under the sweep of group 1) in a child process against the exact form"""
-    import os, subprocess, sys
-    code = (
-        "import numpy as np, torch\n"
-        "from tests.util import rng, packed_frame, to_cuda, to_np, assert_close_int\n"
-        "from tests.test_gpu_reinhard_map16 import make\n"
-        "r = rng(77); fast, exact = make(False), make(True)\n"
-        "for step in range(3):\n"
-        "    dev = [to_cuda(packed_frame(r, 44, 1032)) for _ in range(6)]\n"
-        "    a = fast.process_packed12(dev, tonemap='reinhard', gamma=0.9, intensity=3.0)\n"
-        "    b = exact.process_packed12(dev, tonemap='reinhard', gamma=0.9, intensity=3.0)\n"
-        "    fr = [assert_close_int(to_np(x), to_np(y), 1, 'overlapped') for x, y in zip(a, b)]\n"
-        "    assert max(fr) < 0.02\n"
-        "print('overlap ok')\n")
-    env = dict(os.environ, B200ISP_MAP16_OVERLAP="2", B200ISP_MAP16_OVERLAP_CTAS="2")
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    res = subprocess.run([sys.executable, "-c", code], env=env, cwd=root, capture_output=True, text=True, timeout=600)
-    assert res.returncode == 0 and "overlap ok" in res.stdout, res.stdout + res.stderr
-
-
 @pytest.mark.parametrize("cam,gamma", [("Camera32", 0.9), ("Camera32", 1.0), ("Camera16", 0.6)])
 def test_scratch_and_outputs_stay_inside_their_buffers(cuda, cam, gamma):
     """guard bands (compute-sanitizer is not available on the GPU pool): the map scratch -- exactly the size the host mirror asks

@@ -11,7 +11,7 @@ from oracle import isp_oracle as O
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
-def test_library_loads_and_exports_every_declared_symbol():
+def test_library_loads_exports_every_declared_symbol_and_reports_abi_101():
     from taichi_image_b200 import _lib
     header = open(os.path.join(ROOT, "include", "b200isp.h")).read()
     declared = set(re.findall(r"\b(b200isp_[a-z0-9_]+)\s*\(", header))
@@ -21,14 +21,15 @@ def test_library_loads_and_exports_every_declared_symbol():
     for name in sorted(declared):
         assert hasattr(lib, name), f"{name} declared in include/b200isp.h but not exported"
     assert declared == set(_lib.EXPORTS), declared ^ set(_lib.EXPORTS)
-    assert _lib.lib.b200isp_version() == 100
+    assert _lib.lib.b200isp_version() == 101
     assert _lib.WORKSPACE_BYTES >= 4096
 
 
 def test_fused_params_struct_matches_header():
     from taichi_image_b200 import _lib
-    # 7 ints, 9 floats, 4 floats, int, float, 7 ints, 2 floats, 5 ints (36 x 4 bytes, no padding) + 4 pointers + 2 size_t
-    assert ctypes.sizeof(_lib.FusedParams) == 4 * (7 + 9 + 4 + 1 + 1 + 7 + 2 + 5) + 6 * ctypes.sizeof(ctypes.c_void_p)
+    # 7 ints, 9 floats, 4 floats, int, float, 6 ints, 2 floats, 5 ints (35 x 4 bytes) + 4 bytes of padding before the first
+    # pointer + 4 pointers + 2 size_t
+    assert ctypes.sizeof(_lib.FusedParams) == 4 * (7 + 9 + 4 + 1 + 1 + 6 + 2 + 5) + 4 + 6 * ctypes.sizeof(ctypes.c_void_p)
     header = open(os.path.join(ROOT, "include", "b200isp.h")).read()
     body = header[header.index("typedef struct {"):header.index("} b200isp_fused_params;")]
     names = re.findall(r"\b(?:int|float|void\*|size_t)\s+([a-z_0-9, \[\]]+);", body)
@@ -182,7 +183,7 @@ def test_c_abi_rejects_bad_arguments_without_touching_the_gpu():
 
 
 
-def test_transform_routing_of_the_fused_call(monkeypatch):
+def test_fused_call_routes_transforms_without_routing_switches(monkeypatch):
     """host logic of ISP._fused_flip (no GPU): which ISP transforms the fused call applies itself -- flips in the sweep's
     store on every path, transposing transforms (interpolate.py:36-56) in the normalise pass of the one-sweep Reinhard -> u8
     forms only; everything else returns 0 = the transform kernel runs behind the call"""
@@ -190,8 +191,7 @@ def test_transform_routing_of_the_fused_call(monkeypatch):
     from taichi_image_b200 import camera_isp, bayer
     from taichi_image_b200.dtypes import u8, u16, f16
     from taichi_image_b200.interpolate import ImageTransform as T
-    for var in ("B200ISP_FUSED_TRANSPOSE", "B200ISP_TURN_IN_PASS", "B200ISP_NO_FUSED_TRANSFORM", "B200ISP_CAM16_RECOMPUTE",
-                "B200ISP_CAM32_ONE_SWEEP", "B200ISP_REINHARD_EXACT"):
+    for var in ("B200ISP_FUSED_TRANSPOSE", "B200ISP_REINHARD_EXACT"):
         monkeypatch.delenv(var, raising=False)
     cpu = torch.device("cpu")
     codes = {T.flip_horiz: 1, T.flip_vert: 2, T.rotate_180: 3, T.transpose: 4, T.rotate_270: 5, T.rotate_90: 6, T.transverse: 7}
@@ -212,7 +212,5 @@ def test_transform_routing_of_the_fused_call(monkeypatch):
     assert isp._fused_flip(3000, "reinhard", u8, 1.2, 0.0) == 0 and isp._fused_flip(3000, "reinhard", u8, 0.9, 0.5) == 0
     assert camera_isp.Camera32(bayer.BayerPattern.RGGB, transform=T.rotate_90, reinhard_exact=True, device=cpu)._fused_flip(3000, "reinhard", u8, 0.9, 0.0) == 0
     assert camera_isp.Camera16(bayer.BayerPattern.RGGB, transform=T.rotate_90, device=cpu)._fused_flip(3000, "reinhard", u8, 1.2, 0.5) == 6
-    monkeypatch.setenv("B200ISP_TURN_IN_PASS", "0")
-    assert isp._fused_flip(3000, "reinhard", u8, 0.9, 0.0) == 0
     monkeypatch.setenv("B200ISP_FUSED_TRANSPOSE", "1")                                               # the sweep's own transposing store (opt-in)
     assert isp._fused_flip(3000, "linear", u16, 1.0, 0.0) == 6
