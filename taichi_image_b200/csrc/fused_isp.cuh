@@ -1210,8 +1210,7 @@ struct Packed12FastSampler {
     float x[3];
 #pragma unroll
     for (int ch = 0; ch < 3; ++ch) x[ch] = frame_exact(CAM16 ? S[ch] * (sc[ch] * 0.0625f) : fmaf(S[ch], sc[ch] * kn, -16.f * kn), t[ch]);
-    if (k.ccm) ccm_apply(k.m, x[0], x[1], x[2]);
-    rgb[0] = round_isp<CAM16>(clamp01(x[0])); rgb[1] = round_isp<CAM16>(clamp01(x[1])); rgb[2] = round_isp<CAM16>(clamp01(x[2]));
+    raw_to_rgb<CAM16>(k, x, rgb);       // the sweep's own CCM (FMA chain; identity without CCM), clamp and rounding
   }
 
   __device__ __forceinline__ bool on_frame(int row, int col) const { return row < 2 || row >= k.H - 2 || col < 2 || col >= k.W - 2; }
