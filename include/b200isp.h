@@ -32,7 +32,7 @@
 extern "C" {
 #endif
 
-#define B200ISP_VERSION 101            /* 0.1.1 */
+#define B200ISP_VERSION 102            /* 0.1.2 */
 #define B200ISP_MAX_FRAMES 64          /* frames per batched call */
 #define B200ISP_METRICS 9              /* camera_isp.py:102-115 */
 
@@ -198,19 +198,18 @@ typedef struct {
                                    rows, bit 2 = transpose (output (W, H), out_pitch counts elements of ITS rows; needs height % 8 == 0):
                                    flip_horiz 1, flip_vert 2, rotate_180 3, transpose 4, rotate_270 5, rotate_90 6, transverse 7 */
   int reinhard_mode;            /* Camera32 Reinhard -> u8 with reinhard_scratch: 0 = one sweep that also stores the map as u16 fixed point
-                                   + a normalise pass (u8 within 1 LSB of the two-sweep result; color_adapt == 0, 0.3 <= gamma <= 1;
-                                   frames whose map leaves [0, 1) are redone exactly), 1 = always the exact max sweep + write sweep;
-                                   any other value also takes the exact form */
+                                   + a normalise pass where it applies (b200isp_reinhard_scratch_bytes; u8 within 1 LSB of the
+                                   two-sweep result, frames whose map leaves [0, 1) are redone exactly), 1 = always the exact max
+                                   sweep + write sweep; any other value also takes the exact form */
   int ids_layout;               /* packed layout of the input frames: 0 = standard (packed.py:23-31), 1 = IDS (packed.py:36-44),
                                    decoded inside the row loader (4 instead of 2 instructions per sample, no re-pack pass) */
   void* profile_start;          /* optional cudaEvent_t pair recorded on `stream` immediately before / after */
   void* profile_stop;           /*   the dominant streaming kernel (bench.py's live roofline timing); NULL = off */
   void* meter_cache;            /* optional device scratch: >= n_frames*ceil(H/stride)*ceil(W/stride)*12 bytes; the second */
   size_t meter_cache_bytes;     /*   metering phase then re-reads the phase-1 samples instead of recomputing them */
-  void* reinhard_scratch;       /* optional device scratch, >= n_frames*H*W*3*2 bytes: Camera16 Reinhard then runs ONE sweep that */
-  size_t reinhard_scratch_bytes;/*   stores the f16 map (camera_isp.py:211) + an element-wise normalise / quantise pass; Camera32 -> u8
-                                     likewise with a u16 fixed-point map (see reinhard_mode).  Camera16 -> u8 with gamma != 1 and a
-                                     further n_frames*65536 bytes behind the maps runs that pass through a per-frame table */
+  void* reinhard_scratch;       /* optional device scratch of b200isp_reinhard_scratch_bytes(params, n_frames) bytes: Reinhard then */
+  size_t reinhard_scratch_bytes;/*   runs ONE sweep that stores the map (camera_isp.py:211) + an element-wise normalise / quantise
+                                     pass.  YUV 4:2:0 output and Reinhard with resize require it */
 } b200isp_fused_params;
 
 /* camera_isp.py:333-340 load_packed12 + :376-385 update_metering + :394-413 tonemap_* over a
@@ -220,6 +219,10 @@ typedef struct {
 int b200isp_process_packed12(const uint8_t* const* packed_host, void* const* out_host, int n_frames,
                              const b200isp_fused_params* params, float* metrics,
                              void* workspace, b200isp_stream stream);
+/* The bytes of reinhard_scratch with which b200isp_process_packed12(params, n_frames frames) runs its one-sweep Reinhard
+ * form; 0 when that call uses no scratch (no Reinhard tone map, or the exact two-sweep form) or refuses the parameter
+ * block whatever scratch it gets.  Reads only the scalar fields of params and makes no CUDA call. */
+size_t b200isp_reinhard_scratch_bytes(const b200isp_fused_params* params, int n_frames);
 
 /* EXTENSION (north_star "percentile histogram"; no reference counterpart): luminance histogram of the metering
  * samples (n_samples RGB float triples as written to fused_params.meter_cache), bin = min(bins-1, trunc(gray*bins)),

@@ -84,7 +84,8 @@ SIGNATURES = {
     "b200isp_meter_packed12_phase2": [C.POINTER(_vp), _i, C.POINTER(FusedParams), _vp, _i, _vp, _vp, _vp, _vp],
 }
 _SPECIAL = {"b200isp_version": ([], C.c_int), "b200isp_last_error": ([], C.c_char_p),
-            "b200isp_workspace_bytes": ([], C.c_size_t), "b200isp_mailbox_bytes": ([_i], C.c_size_t)}
+            "b200isp_workspace_bytes": ([], C.c_size_t), "b200isp_mailbox_bytes": ([_i], C.c_size_t),
+            "b200isp_reinhard_scratch_bytes": ([C.POINTER(FusedParams), _i], C.c_size_t)}
 EXPORTS = tuple(SIGNATURES) + tuple(_SPECIAL)
 
 

@@ -435,11 +435,9 @@ def camera_isp(name: str, dtype=f32):
             return [interpolate.transform(output, self.transform) for output in outputs]
 
         # ------------------------------------------------------------ fused path
-        def _fused_params(self, frames, tonemap, out_dtype, tm, update_metering=False, alpha=0.0, rows_per_task=0,
-                          profile_events=None, yuv420=False, ids_format=None, flip=0):
-            """b200isp_fused_params for a list of same-shape packed12 frames (include/b200isp.h)"""
-            h, w3 = frames[0].shape
-            w = w3 * 2 // 3
+        def _param_block(self, h, w, tonemap, out_dtype, tm, yuv420=False, ids_format=None, flip=0, out_pitch=0):
+            """b200isp_fused_params (include/b200isp.h) describing the images and the tone map of a call on (h, w) frames;
+            no buffer attached"""
             p = _lib.FusedParams()
             p.height, p.width, p.pattern = h, w, self.bayer_pattern.value
             p.isp_dtype, p.out_dtype, p.tonemap = isp_dtype.code, out_dtype.code, _TONEMAP_CODE[tonemap]
@@ -451,19 +449,29 @@ def camera_isp(name: str, dtype=f32):
             p.intensity = float(tm.get("intensity", 1.0))
             p.light_adapt = float(tm.get("light_adapt", 1.0))
             p.color_adapt = float(tm.get("color_adapt", 0.0))
-            p.metering_stride, p.alpha = int(self.metering_stride), float(alpha)
-            p.update_metering, p.rows_per_task = int(update_metering), int(rows_per_task)
+            p.metering_stride = int(self.metering_stride)
             p.demosaic = 1 if self.demosaic == "bilinear" else 0
             p.out_yuv420 = int(bool(yuv420))
             p.ids_layout = int(bool(self._ids_layout if ids_format is None else ids_format))
-            p.flip = int(flip)
+            p.flip, p.out_pitch = int(flip), int(out_pitch)
+            if tonemap == "reinhard" and self.reinhard_exact:
+                p.reinhard_mode = 1
             plan = self._resize_plan(h, w)
-            ho, wo = h, w
             if plan is not None:                 # resize fused into the pass (demosaic + bilinear gather)
                 (wo, ho), (sr, sc) = plan
                 p.out_height, p.out_width, p.scale_r, p.scale_c = int(ho), int(wo), float(sr), float(sc)
                 p.resize_gather = int(os.environ.get("B200ISP_RESIZE_GATHER", "0"))        # testing / profiling knob
+            return p
+
+        def _fused_params(self, frames, tonemap, out_dtype, tm, update_metering=False, alpha=0.0, rows_per_task=0,
+                          profile_events=None, yuv420=False, ids_format=None, flip=0, out_pitch=0):
+            """b200isp_fused_params for a list of same-shape packed12 frames (include/b200isp.h), with the buffers the call uses"""
+            h, w3 = frames[0].shape
+            p = self._param_block(h, w3 * 2 // 3, tonemap, out_dtype, tm, yuv420, ids_format, flip, out_pitch)
+            p.alpha = float(alpha)
+            p.update_metering, p.rows_per_task = int(update_metering), int(rows_per_task)
             if update_metering:                  # scratch for the phase-1 samples (re-read by phase 2)
+                ho, wo = (p.out_height, p.out_width) if p.out_height > 0 else (p.height, p.width)
                 stride = max(int(self.metering_stride), 1)
                 need = len(frames) * (-(-ho // stride)) * (-(-wo // stride)) * 12
                 cache = getattr(self, "_meter_cache", None)
@@ -473,29 +481,14 @@ def camera_isp(name: str, dtype=f32):
                     cache = self._meter_cache = torch.empty(need, dtype=torch.uint8, device=self.device)
                 p.meter_cache, p.meter_cache_bytes = cache.data_ptr(), cache.numel()
                 self._meter_n = need // 12
-            if tonemap == "reinhard" and (plan is not None or isp_dtype == f16):
-                # scratch for the un-normalised Reinhard map in the ISP dtype: Camera16 (one sweep + a light normalise
-                # pass, csrc/fused_isp.cuh) and every resizing ISP (output resolution, csrc/fused_resize.cu)
-                # (+ 64 KB per frame: the table of the normalise pass, csrc/fused_isp.cuh run_lut_pass; unused by resizing ISPs)
-                need = len(frames) * ho * wo * 3 * isp_dtype.itemsize + len(frames) * 65536
+            # scratch of the one-sweep Reinhard forms, sized by the library that chooses the form (csrc/fused_isp.cuh
+            # reinhard_plan); none where the call runs the exact max sweep + write sweep
+            need = _lib.lib.b200isp_reinhard_scratch_bytes(p, len(frames))
+            if need:
                 sc = getattr(self, "_reinhard_scratch", None)
                 if sc is None or sc.numel() < need or sc.device != torch.device(self.device):
                     sc = self._reinhard_scratch = torch.empty(need, dtype=torch.uint8, device=self.device)
                 p.reinhard_scratch, p.reinhard_scratch_bytes = sc.data_ptr(), sc.numel()
-            elif (tonemap == "reinhard" and isp_dtype == f32 and out_dtype.name == "u8" and not self.reinhard_exact
-                  and float(tm.get("color_adapt", 0.0)) == 0.0 and 0.3 <= float(tm.get("gamma", 1.0)) <= 1.0
-                  and not yuv420 and (not flip or flip & 4) and not p.ids_layout):
-                # Camera32 -> u8: ONE sweep that also stores the Reinhard map as u16 fixed point (6 B/px scratch) + a light
-                # normalise / gamma / quantise pass instead of the max sweep + write sweep (csrc/fused_isp.cuh, run_fused);
-                # the u8 result is within 1 LSB of the exact form, ISP(reinhard_exact=True) / B200ISP_REINHARD_EXACT=1 keep
-                # the two sweeps.  The library falls back to them on its own when the scratch does not apply (pitched outputs).
-                need = len(frames) * h * w * 6
-                sc = getattr(self, "_reinhard_scratch", None)
-                if sc is None or sc.numel() < need or sc.device != torch.device(self.device):
-                    sc = self._reinhard_scratch = torch.empty(need, dtype=torch.uint8, device=self.device)
-                p.reinhard_scratch, p.reinhard_scratch_bytes = sc.data_ptr(), sc.numel()
-            if tonemap == "reinhard" and self.reinhard_exact:
-                p.reinhard_mode = 1
             if profile_events is not None:      # (start, stop) torch.cuda.Event pair, see bench.py
                 p.profile_start, p.profile_stop = profile_events[0].cuda_event, profile_events[1].cuda_event
             return p
@@ -503,7 +496,6 @@ def camera_isp(name: str, dtype=f32):
         def _fused_flip(self, height, tonemap, out_dtype, gamma, color_adapt, ids_format=False, yuv420=False):
             """b200isp_fused_params.flip code of ``self.transform`` when the fused call applies the transform itself, else 0
             (the tiled transform kernel then runs on the results)"""
-            shape = (height,)
             flip = 0
             if not self._resizes and not yuv420 and self.demosaic == "malvar":
                 T = interpolate.ImageTransform
@@ -511,16 +503,16 @@ def camera_isp(name: str, dtype=f32):
                         T.transverse: 7}.get(self.transform, 0)
                 # Transposing transforms (rotate_90 is the rig script's default): the one-sweep Reinhard -> u8 forms turn the
                 # image in their element-wise normalise pass (csrc/fused_isp.cuh reinhard_out_transposed_kernel: shared-memory
-                # tile, 384-byte output pieces) -- no transform kernel, no extra 3 + 3 B/px.  Elsewhere the sweep's own
-                # transposing store stays OPT-IN (B200ISP_FUSED_TRANSPOSE=1): its 24-byte column pieces are partial-sector
-                # writes, L2 fills every one of them from DRAM (profiles/r02_transpose_store.txt: RGB16 linear 2.2x SLOWER)
+                # tile, 384-byte output pieces) -- no transform kernel, no extra 3 + 3 B/px.  The call takes such a form exactly
+                # when the library asks for a scratch for it; no rule of that query reads the width, so any valid width does.
+                # Elsewhere the sweep's own transposing store stays OPT-IN (B200ISP_FUSED_TRANSPOSE=1): its 24-byte column
+                # pieces are partial-sector writes, L2 fills every one of them from DRAM (profiles/r02_transpose_store.txt:
+                # RGB16 linear 2.2x SLOWER)
                 if flip & 4:
-                    turn_ok = shape[0] % 8 == 0 and shape[0] >= 16
-                    in_pass = (turn_ok and tonemap == "reinhard" and out_dtype == u8 and not ids_format
-                               and (isp_dtype == f16
-                                    or (isp_dtype == f32 and not self.reinhard_exact and float(color_adapt) == 0.0
-                                        and 0.3 <= float(gamma) <= 1.0)))
-                    if not (in_pass or (turn_ok and os.environ.get("B200ISP_FUSED_TRANSPOSE", "0") == "1")):
+                    p = self._param_block(height, 8, tonemap, out_dtype, dict(gamma=gamma, color_adapt=color_adapt),
+                                          yuv420, bool(ids_format), flip)
+                    if not (_lib.lib.b200isp_reinhard_scratch_bytes(p, 1) or
+                            (height % 8 == 0 and height >= 16 and os.environ.get("B200ISP_FUSED_TRANSPOSE", "0") == "1")):
                         flip = 0
             return flip
 
@@ -534,14 +526,13 @@ def camera_isp(name: str, dtype=f32):
                 # host only ever sees 1.5 bytes per pixel
                 return self._run_fused_yuv_two_step(frames, tonemap, out_dtype, out, tm, update_metering, alpha, rows_per_task,
                                                     profile_events)
-            p = self._fused_params(frames, tonemap, out_dtype, tm, update_metering, alpha, rows_per_task, profile_events, yuv420,
-                                   ids_format, flip)
             plan = self._resize_plan(h, w)
             if plan is not None:
                 w, h = plan[0]
             oshape = (h * 3 // 2, w) if yuv420 else (h, w, 3)       # planar YUV 4:2:0: color/yuv_420.py:95-118
             if flip & 4:
                 oshape = (w, h, 3)                                  # transposing transform applied by the store
+            out_pitch = 0
             if out is None:
                 out = [torch.empty(oshape, dtype=out_dtype.torch, device=self.device) for _ in frames]
             else:
@@ -555,7 +546,9 @@ def camera_isp(name: str, dtype=f32):
                         "outputs must be contiguous or row-pitched (H, W, 3) views"
                 if not out[0].is_contiguous():
                     assert plan is None and not yuv420, "pitched outputs need the plain RGB sweep (no resize, no YUV)"
-                    p.out_pitch = int(pitch)
+                    out_pitch = pitch
+            p = self._fused_params(frames, tonemap, out_dtype, tm, update_metering, alpha, rows_per_task, profile_events, yuv420,
+                                   ids_format, flip, out_pitch=out_pitch)
             metrics_ptr = 0 if self.metrics is None else self.metrics.data_ptr()
             with torch.cuda.device(self.device):
                 _lib.check(_lib.lib.b200isp_process_packed12(

@@ -14,31 +14,22 @@ extern template int run_fused<false, float>(const FramePtrs&, int, const b200isp
 
 using namespace isp;
 
-// Common argument checks + frame table + constants of the fused entry points.
-static int fused_setup(const char* what, const uint8_t* const* packed_host, void* const* out_host, int n_frames,
-                       const b200isp_fused_params* params, float* metrics, void* workspace, FramePtrs& fp, IspConsts& k) {
-  ISP_REQUIRE(packed_host && params && workspace, B200ISP_E_ARG, "%s: null pointer", what);
-  const b200isp_fused_params& p = *params;
+// Checks of the parameter block common to the fused entry points, and the constants derived from it, except the two
+// pointers k.metrics / k.ws.  Reads no pointer, so b200isp_reinhard_scratch_bytes runs it on a machine without a GPU.
+static int fused_consts(const char* what, int n_frames, const b200isp_fused_params& p, IspConsts& k) {
   ISP_REQUIRE(n_frames >= 1 && n_frames <= B200ISP_MAX_FRAMES, B200ISP_E_FRAMES,
               "%s: %d frames (1..%d supported per call)", what, n_frames, B200ISP_MAX_FRAMES);
   ISP_REQUIRE(p.height >= 4 && p.width >= 8 && p.height % 2 == 0 && p.width % 8 == 0, B200ISP_E_SHAPE,
               "%s: fused path needs even height >= 4 and width %% 8 == 0, got %dx%d", what, p.height, p.width);
   ISP_REQUIRE(p.pattern >= 0 && p.pattern <= 3, B200ISP_E_ARG, "%s: unknown pattern %d", what, p.pattern);
   ISP_REQUIRE(p.isp_dtype == B200ISP_F16 || p.isp_dtype == B200ISP_F32, B200ISP_E_DTYPE, "%s: isp_dtype must be f16/f32", what);
-  for (int i = 0; i < n_frames; ++i) {
-    fp.in[i] = packed_host[i];
-    fp.out[i] = out_host ? out_host[i] : nullptr;
-    ISP_REQUIRE(fp.in[i] && (fp.out[i] || !out_host), B200ISP_E_ARG, "%s: null frame pointer %d", what, i);
-    ISP_REQUIRE(((reinterpret_cast<uintptr_t>(fp.in[i]) & 3u) == 0) && ((reinterpret_cast<uintptr_t>(fp.out[i]) & 15u) == 0),
-                B200ISP_E_ALIGN, "%s: frame %d needs 4-byte aligned input and 16-byte aligned output", what, i);
-  }
   k.H = p.height; k.W = p.width; k.pattern = p.pattern;
   k.ccm = p.has_ccm ? 1 : 0;
   for (int i = 0; i < 9; ++i) k.m[i] = p.has_ccm ? p.ccm[i] : (i % 4 == 0 ? 1.f : 0.f);   // identity: see raw_to_rgb
   k.gamma = p.gamma; k.intensity = p.intensity; k.la = p.light_adapt; k.ca = p.color_adapt;
   ISP_REQUIRE(p.demosaic == B200ISP_DEMOSAIC_MALVAR || p.demosaic == B200ISP_DEMOSAIC_BILINEAR, B200ISP_E_ARG,
               "%s: unknown demosaic %d", what, p.demosaic);
-  k.metrics = metrics; k.ws = (Workspace*)workspace; k.frame0 = 0;
+  k.frame0 = 0;
   k.kbase = p.demosaic == B200ISP_DEMOSAIC_BILINEAR ? kBilinearBase : 0;
   k.flip = p.flip & 7;
   k.gate = 0;
@@ -53,6 +44,73 @@ static int fused_setup(const char* what, const uint8_t* const* packed_host, void
               "%s: out_pitch must be >= 3 * (output width) elements and a multiple of 16 bytes", what);
   ISP_REQUIRE(p.out_pitch <= 0 || (!resizes(p) && !p.out_yuv420), B200ISP_E_ARG, "%s: out_pitch needs the plain RGB sweep (no resize, no YUV)", what);
   return B200ISP_OK;
+}
+
+// fused_consts + the frame table of the fused entry points.
+static int fused_setup(const char* what, const uint8_t* const* packed_host, void* const* out_host, int n_frames,
+                       const b200isp_fused_params* params, float* metrics, void* workspace, FramePtrs& fp, IspConsts& k) {
+  ISP_REQUIRE(packed_host && params && workspace, B200ISP_E_ARG, "%s: null pointer", what);
+  const int st = fused_consts(what, n_frames, *params, k);
+  if (st) return st;
+  for (int i = 0; i < n_frames; ++i) {
+    fp.in[i] = packed_host[i];
+    fp.out[i] = out_host ? out_host[i] : nullptr;
+    ISP_REQUIRE(fp.in[i] && (fp.out[i] || !out_host), B200ISP_E_ARG, "%s: null frame pointer %d", what, i);
+    ISP_REQUIRE(((reinterpret_cast<uintptr_t>(fp.in[i]) & 3u) == 0) && ((reinterpret_cast<uintptr_t>(fp.out[i]) & 15u) == 0),
+                B200ISP_E_ALIGN, "%s: frame %d needs 4-byte aligned input and 16-byte aligned output", what, i);
+  }
+  k.metrics = metrics; k.ws = (Workspace*)workspace;
+  return B200ISP_OK;
+}
+
+// The further checks of b200isp_process_packed12 that read only the parameter block.
+static int process_checks(const b200isp_fused_params& p) {
+  ISP_REQUIRE(p.tonemap >= B200ISP_TM_LINEAR && p.tonemap <= B200ISP_TM_NONE, B200ISP_E_ARG, "process_packed12: unknown tonemap %d", p.tonemap);
+  ISP_REQUIRE(p.tonemap == B200ISP_TM_NONE || p.gamma > 0.f, B200ISP_E_ARG, "process_packed12: gamma must be positive");
+  if (p.tonemap == B200ISP_TM_NONE)
+    ISP_REQUIRE(p.out_dtype == p.isp_dtype, B200ISP_E_DTYPE, "process_packed12: TM_NONE writes the ISP dtype");
+  else
+    ISP_REQUIRE(p.out_dtype == B200ISP_U8 || p.out_dtype == B200ISP_U16 || p.out_dtype == B200ISP_F16, B200ISP_E_DTYPE,
+                "process_packed12: tone-mapped output must be u8, u16 or f16");
+  if (resizes(p)) {
+    ISP_REQUIRE(p.scale_r > 0.f && p.scale_c > 0.f, B200ISP_E_ARG, "process_packed12: resize scales must be positive");
+    ISP_REQUIRE(!p.out_yuv420, B200ISP_E_ARG, "process_packed12: YUV 4:2:0 output is not available with resize");
+  }
+  ISP_REQUIRE(!p.out_yuv420 || (p.isp_dtype == B200ISP_F16 && p.out_dtype == B200ISP_U8 && p.tonemap == B200ISP_TM_REINHARD),
+              B200ISP_E_ARG, "process_packed12: YUV 4:2:0 output needs Camera16 (f16), Reinhard, u8 and the reinhard_scratch buffer");
+  return B200ISP_OK;
+}
+
+namespace isp {
+ReinhardPlan reinhard_plan(const b200isp_fused_params& p, const IspConsts& k, int n_frames) {
+  if (p.tonemap != B200ISP_TM_REINHARD) return {ReinhardForm::kNone, 0, 0};
+  const bool cam16 = p.isp_dtype == B200ISP_F16;
+  if (resizes(p)) {
+    const size_t map = (size_t)n_frames * p.out_height * p.out_width * 3 * (cam16 ? sizeof(__half) : sizeof(float));
+    return {ReinhardForm::kResizeMap, map, map};
+  }
+  const size_t map = (size_t)n_frames * k.H * k.W * 3 * (cam16 ? sizeof(__half) : sizeof(uint16_t));
+  const bool u8 = p.out_dtype == B200ISP_U8;
+  // the normalise pass turns the image (reinhard_out_transposed_kernel); the map itself is a plain (H, W, 3) image
+  const bool turned = (k.flip & 4) && u8 && k.orow % 8 == 0 && k.ids == 0;
+  if (cam16) {
+    if (turned) return {ReinhardForm::kF16Turned, map, map};
+    // the other normalise passes index the output flat: dense, unflipped outputs only
+    if (k.flip != 0 || k.orow != 3 * k.W) return {ReinhardForm::kExact, 0, 0};
+    if (p.out_yuv420) return {ReinhardForm::kF16Yuv, map, map};
+    if (u8 && k.gamma != 1.0f) return {ReinhardForm::kF16Table, map, map + (size_t)n_frames * kLutBytes};
+    return {ReinhardForm::kF16Arith, map, map};
+  }
+  if (u8 && p.reinhard_mode == 0 && k.ca == 0.f && k.gamma <= 1.0f && k.gamma >= 0.3f && (k.flip == 0 || turned) && k.ids == 0)
+    return {turned ? ReinhardForm::kU16Turned : ReinhardForm::kU16Map, map, map};
+  return {ReinhardForm::kExact, 0, 0};
+}
+}  // namespace isp
+
+extern "C" size_t b200isp_reinhard_scratch_bytes(const b200isp_fused_params* params, int n_frames) {
+  IspConsts k;
+  if (!params || fused_consts("reinhard_scratch_bytes", n_frames, *params, k) || process_checks(*params)) return 0;
+  return reinhard_plan(*params, k, n_frames).bytes;
 }
 
 // Builds the metering sampler for the packed frames (stride % 8 == 0: word-aligned fast sampler) and
@@ -156,18 +214,12 @@ extern "C" int b200isp_process_packed12(const uint8_t* const* packed_host, void*
   FramePtrs fp; IspConsts k;
   ISP_REQUIRE(out_host, B200ISP_E_ARG, "process_packed12: null output list");
   {
-    const int st = fused_setup("process_packed12", packed_host, out_host, n_frames, params, metrics, workspace, fp, k);
+    int st = fused_setup("process_packed12", packed_host, out_host, n_frames, params, metrics, workspace, fp, k);
+    if (!st) st = process_checks(*params);
     if (st) return st;
   }
   const b200isp_fused_params& p = *params;
-  ISP_REQUIRE(p.tonemap >= B200ISP_TM_LINEAR && p.tonemap <= B200ISP_TM_NONE, B200ISP_E_ARG, "process_packed12: unknown tonemap %d", p.tonemap);
   ISP_REQUIRE(p.tonemap == B200ISP_TM_NONE || metrics, B200ISP_E_ARG, "process_packed12: metrics required for tone mapping");
-  ISP_REQUIRE(p.tonemap == B200ISP_TM_NONE || p.gamma > 0.f, B200ISP_E_ARG, "process_packed12: gamma must be positive");
-  if (p.tonemap == B200ISP_TM_NONE)
-    ISP_REQUIRE(p.out_dtype == p.isp_dtype, B200ISP_E_DTYPE, "process_packed12: TM_NONE writes the ISP dtype");
-  else
-    ISP_REQUIRE(p.out_dtype == B200ISP_U8 || p.out_dtype == B200ISP_U16 || p.out_dtype == B200ISP_F16, B200ISP_E_DTYPE,
-                "process_packed12: tone-mapped output must be u8, u16 or f16");
   cudaStream_t s = (cudaStream_t)stream;
   const bool cam16 = p.isp_dtype == B200ISP_F16;
 
@@ -178,11 +230,7 @@ extern "C" int b200isp_process_packed12(const uint8_t* const* packed_host, void*
     if (st) return st;
   }
 
-  if (resizes(p)) {
-    ISP_REQUIRE(p.scale_r > 0.f && p.scale_c > 0.f, B200ISP_E_ARG, "process_packed12: resize scales must be positive");
-    ISP_REQUIRE(!p.out_yuv420, B200ISP_E_ARG, "process_packed12: YUV 4:2:0 output is not available with resize");
-    return run_resize(fp, n_frames, p, k, s);
-  }
+  if (resizes(p)) return run_resize(fp, n_frames, p, k, s);
 #define RUN(CAM, T) return run_fused<CAM, T>(fp, n_frames, p, k, s)
   if (cam16) {
     switch (p.out_dtype) {

@@ -1728,16 +1728,37 @@ int run_rmax(const FramePtrs& fp, IspConsts k, int nframes, int rows_per_task, c
 
 int run_write_gated(const FramePtrs& fp, IspConsts k, int nframes, int rows_per_task, cudaStream_t s);
 
+// How b200isp_process_packed12 runs the Reinhard tone map of a parameter block that passed its checks, and the bytes of
+// reinhard_scratch that form uses: the maps of all frames, plus the per-frame tables of kF16Table.  reinhard_plan
+// (fused_api.cu) is the only place that decides this; run_fused, run_resize_t and b200isp_reinhard_scratch_bytes ask it.
+// A scratch smaller than map_bytes means the exact form (YUV 4:2:0 and resizing ISPs: refused); one that holds the maps
+// but not the tables means kF16Arith, whose result is bit-identical to kF16Table's.
+enum class ReinhardForm {
+  kNone,          // no Reinhard tone map (linear, TM_NONE): one sweep
+  kExact,         // max sweep + write sweep (run_rmax, MODE_REINHARD)
+  kResizeMap,     // resizing ISP: the map at output resolution in the ISP dtype + a normalise pass (fused_resize.cu)
+  kF16Turned,     // Camera16 f16 map + reinhard_out_transposed_kernel (transposing transforms)
+  kF16Yuv,        // Camera16 f16 map + reinhard_scratch_yuv_kernel
+  kF16Table,      // Camera16 f16 map + run_lut_pass (u8, gamma != 1: a 64 KB table per frame behind the maps)
+  kF16Arith,      // Camera16 f16 map + reinhard_scratch_out_kernel
+  kU16Map,        // Camera32 u16 fixed-point map + reinhard_map16_out_kernel + the gated exact sweeps
+  kU16Turned,     // Camera32 u16 fixed-point map + the gated exact sweeps + reinhard_out_transposed_kernel
+};
+struct ReinhardPlan {
+  ReinhardForm form;
+  size_t map_bytes, bytes;    // 0 for kNone and kExact
+};
+ReinhardPlan reinhard_plan(const b200isp_fused_params& p, const IspConsts& k, int n_frames);
+
 template <bool CAM16, typename OutT>
 int run_fused(const FramePtrs& fp, int n_frames, const b200isp_fused_params& p, IspConsts k, cudaStream_t s) {
   const int rpt = p.rows_per_task;
-  if (p.out_yuv420) {
-    const bool ok = CAM16 && std::is_same<OutT, uint8_t>::value && p.tonemap == B200ISP_TM_REINHARD && p.reinhard_scratch &&
-                    p.reinhard_scratch_bytes >= (size_t)n_frames * k.H * k.W * 3 * sizeof(__half);
-    if (!ok) {
-      set_error("process_packed12: YUV 4:2:0 output needs Camera16 (f16), Reinhard, u8 and the reinhard_scratch buffer");
-      return B200ISP_E_ARG;
-    }
+  ReinhardPlan plan = reinhard_plan(p, k, n_frames);
+  if (plan.map_bytes && (!p.reinhard_scratch || p.reinhard_scratch_bytes < plan.map_bytes)) plan.form = ReinhardForm::kExact;
+  else if (plan.form == ReinhardForm::kF16Table && p.reinhard_scratch_bytes < plan.bytes) plan.form = ReinhardForm::kF16Arith;
+  if (p.out_yuv420 && plan.form == ReinhardForm::kExact) {
+    set_error("process_packed12: YUV 4:2:0 output needs Camera16 (f16), Reinhard, u8 and the reinhard_scratch buffer");
+    return B200ISP_E_ARG;
   }
   constexpr bool kIspOut = (CAM16 && std::is_same<OutT, __half>::value) || (!CAM16 && std::is_same<OutT, float>::value);
   if (p.tonemap == B200ISP_TM_NONE) {
@@ -1755,11 +1776,8 @@ int run_fused(const FramePtrs& fp, int n_frames, const b200isp_fused_params& p, 
     if (st) return st;
     if constexpr (CAM16) {
       // Camera16: the reference stores the map as f16 anyway -> one sweep writes it to the caller's scratch, a light
-      // element-wise pass normalises it (no second sweep, no L2 grouping); dense outputs only (the normalise pass
-      // indexes the output flat), pitched outputs take the two-sweep form below
-      const size_t need = (size_t)n_frames * k.H * k.W * 3 * sizeof(__half);
-      const bool turned = (k.flip & 4) && std::is_same<OutT, uint8_t>::value && !p.out_yuv420 && k.orow % 8 == 0 && k.ids == 0;
-      if (p.reinhard_scratch && p.reinhard_scratch_bytes >= need && ((k.orow == 3 * k.W && k.flip == 0) || turned)) {
+      // element-wise pass normalises it (no second sweep, no L2 grouping)
+      if (plan.form != ReinhardForm::kExact) {
         FramePtrs sc = fp;
         for (int f = 0; f < n_frames; ++f) sc.out[f] = (char*)p.reinhard_scratch + (size_t)f * k.H * k.W * 3 * sizeof(__half);
         IspConsts kp = k;            // the map is a plain dense (H, W, 3) image whatever the output looks like
@@ -1767,16 +1785,16 @@ int run_fused(const FramePtrs& fp, int n_frames, const b200isp_fused_params& p, 
         kp.orow = 3 * k.W;
         st = run_rstore<true>(sc, kp, n_frames, rpt, s, p.profile_start, p.profile_stop);
         if (st) return st;
-        if (turned) return run_out_transposed<true>(sc, fp, n_frames, k, s);     // the normalise pass turns the image
-        if (p.out_yuv420) {
+        if (plan.form == ReinhardForm::kF16Turned) return run_out_transposed<true>(sc, fp, n_frames, k, s);     // the normalise pass turns the image
+        if (plan.form == ReinhardForm::kF16Yuv) {
           const dim3 grid((unsigned)((k.W / 8 + 127) / 128), (unsigned)(k.H / 2), (unsigned)n_frames);
           reinhard_scratch_yuv_kernel<<<grid, 128, 0, s>>>(sc, fp, k.H, k.W, k.gamma, k.ws);
           return cuda_status(cudaPeekAtLastError(), "reinhard_scratch_yuv_kernel");
         }
         const long long n_elems = (long long)k.H * k.W * 3;
         if constexpr (std::is_same<OutT, uint8_t>::value) {
-          if (k.gamma != 1.0f && p.reinhard_scratch_bytes >= need + (size_t)n_frames * kLutBytes)
-            return run_lut_pass<true>(sc, fp, n_frames, n_elems, (uint8_t*)p.reinhard_scratch + need, k.gamma, k.ws, s);
+          if (plan.form == ReinhardForm::kF16Table)
+            return run_lut_pass<true>(sc, fp, n_frames, n_elems, (uint8_t*)p.reinhard_scratch + plan.map_bytes, k.gamma, k.ws, s);
         }
         const dim3 grid((unsigned)std::min<long long>((n_elems / 8 + 255) / 256, 4 * kNumSMs), (unsigned)n_frames);
         reinhard_scratch_out_kernel<OutT><<<grid, 256, 0, s>>>(sc, fp, n_elems, k.gamma, k.ws);
@@ -1788,14 +1806,11 @@ int run_fused(const FramePtrs& fp, int n_frames, const b200isp_fused_params& p, 
       // (6 B/px scratch) + an element-wise normalise / gamma / quantise pass.  The second demosaic of the two-sweep form
       // (66 of its 106 instructions per pixel) disappears; the u8 result is within 1 LSB of the two-sweep result
       // (measured: profiles/r02_reinhard_map16.txt).  Frames whose map does not fit [0, 1) (reinhard_map16_declined) are
-      // redone exactly by the gated sweeps.  Any reinhard_mode other than 0 forces the exact two-sweep form.
-      const size_t need = (size_t)n_frames * k.H * k.W * 3 * sizeof(uint16_t);
-      const bool turned = (k.flip & 4) && k.orow % 8 == 0;
-      if (p.reinhard_mode == 0 && k.ca == 0.f && k.gamma <= 1.0f && k.gamma >= 0.3f && !p.out_yuv420 && (k.flip == 0 || turned) && k.ids == 0 &&
-          p.reinhard_scratch && p.reinhard_scratch_bytes >= need) {
+      // redone exactly by the gated sweeps.
+      if (plan.form != ReinhardForm::kExact) {
         FramePtrs sc = fp;
         for (int f = 0; f < n_frames; ++f) sc.out[f] = (char*)p.reinhard_scratch + (size_t)f * k.H * k.W * 3 * sizeof(uint16_t);
-        if (turned) {
+        if (plan.form == ReinhardForm::kU16Turned) {
           // transposing transform: map sweep (plain row stores), then the gated exact sweeps leave the frames the map declined
           // as plain (H, W, 3) u8 images in their scratch, then ONE pass normalises / turns every frame into the output
           IspConsts kp = k;

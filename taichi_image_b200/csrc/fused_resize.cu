@@ -101,7 +101,7 @@ static int run_resize_t(const FramePtrs& fp, int n_frames, const b200isp_fused_p
     }
   } else {
     const size_t frame_bytes = (size_t)p.out_height * p.out_width * 3 * sizeof(IspT);
-    ISP_REQUIRE(p.reinhard_scratch && p.reinhard_scratch_bytes >= frame_bytes * n_frames, B200ISP_E_ARG,
+    ISP_REQUIRE(p.reinhard_scratch && p.reinhard_scratch_bytes >= reinhard_plan(p, k, n_frames).bytes, B200ISP_E_ARG,
                 "process_packed12: Reinhard with resize needs reinhard_scratch of n_frames * out_height * out_width * 3 ISP-dtype values");
     st = cuda_status(cudaMemsetAsync(k.ws->frame_max, 0, sizeof(float) * B200ISP_MAX_FRAMES, s), "memset frame_max");
     if (st) return st;

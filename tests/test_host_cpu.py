@@ -11,7 +11,7 @@ from oracle import isp_oracle as O
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
-def test_library_loads_exports_every_declared_symbol_and_reports_abi_101():
+def test_library_loads_exports_every_declared_symbol_and_reports_abi_102():
     from taichi_image_b200 import _lib
     header = open(os.path.join(ROOT, "include", "b200isp.h")).read()
     declared = set(re.findall(r"\b(b200isp_[a-z0-9_]+)\s*\(", header))
@@ -21,7 +21,7 @@ def test_library_loads_exports_every_declared_symbol_and_reports_abi_101():
     for name in sorted(declared):
         assert hasattr(lib, name), f"{name} declared in include/b200isp.h but not exported"
     assert declared == set(_lib.EXPORTS), declared ^ set(_lib.EXPORTS)
-    assert _lib.lib.b200isp_version() == 101
+    assert _lib.lib.b200isp_version() == 102
     assert _lib.WORKSPACE_BYTES >= 4096
 
 
@@ -214,3 +214,77 @@ def test_fused_call_routes_transforms_without_routing_switches(monkeypatch):
     assert camera_isp.Camera16(bayer.BayerPattern.RGGB, transform=T.rotate_90, device=cpu)._fused_flip(3000, "reinhard", u8, 1.2, 0.5) == 6
     monkeypatch.setenv("B200ISP_FUSED_TRANSPOSE", "1")                                               # the sweep's own transposing store (opt-in)
     assert isp._fused_flip(3000, "linear", u16, 1.0, 0.0) == 6
+
+
+def _expected_reinhard_scratch(isp, out, tonemap, gamma, ca, mode, flip, yuv, ids, pitched, resize, n, h, w, ho, wo):
+    """the bytes of reinhard_scratch with which b200isp_process_packed12 takes its one-sweep Reinhard form (the plan of
+    csrc/fused_isp.cuh reinhard_plan, restated); 0 where it uses no scratch or refuses the parameter block"""
+    f16, u8 = "f16", "u8"
+    if tonemap != "reinhard" or out == "f32":
+        return 0
+    refused = ((yuv and (isp != f16 or out != u8 or resize or flip or pitched)) or (flip and resize)
+               or (flip & 4 and h % 8) or (ids and resize) or (pitched and resize))
+    if refused:
+        return 0
+    g = np.float32(gamma)                 # the library sees the float32 of the parameter block
+    if resize:
+        return n * ho * wo * 3 * (2 if isp == f16 else 4)
+    if isp == f16:
+        if out == u8 and flip & 4 and not ids and not yuv:
+            return n * h * w * 6                                      # f16 map + turned pass
+        if yuv:
+            return n * h * w * 6                                      # f16 map + YUV pass
+        if not pitched and flip == 0:
+            return n * h * w * 6 + (n * 65536 if out == u8 and g != np.float32(1) else 0)   # table / arithmetic pass
+        return 0                                                      # exact two sweeps
+    if (out == u8 and mode == 0 and ca == 0 and np.float32(0.3) <= g <= np.float32(1) and not yuv and not ids
+            and (flip == 0 or flip & 4)):
+        return n * h * w * 6                                          # u16 map + map16 / turned pass + gated sweeps
+    return 0
+
+
+def test_reinhard_scratch_query_matches_the_plan_and_sizes_the_isp_scratch():
+    """b200isp_reinhard_scratch_bytes (no GPU) over every parameter that selects a Reinhard form, against the plan restated
+    above; ISP._fused_params asks it for exactly that scratch, and allocates none where the call runs the exact form"""
+    import itertools
+    import torch
+    from taichi_image_b200 import _lib, camera_isp, bayer, dtypes
+    query = _lib.lib.b200isp_reinhard_scratch_bytes
+    n, w, ho, wo = 3, 4096, 1080, 1920
+    pitch = 3 * w + 48                    # >= 3 * (output row) for both orientations, a multiple of 16 elements
+    tms = {"linear": 0, "reinhard": 1, "none": 2}
+    grid = itertools.product(("f16", "f32"), ("u8", "u16", "f16", "f32"), tms, (0.29, 0.3, 0.9, 1.0, 1.2), (0.0, 0.5),
+                             (0, 1, 2), range(8), (0, 1), (0, 1), (0, 1), (0, 1), (3000, 3004))
+    checked = 0
+    for isp, out, tm, gamma, ca, mode, flip, yuv, ids, pitched, resize, h in grid:
+        p = _lib.FusedParams()
+        p.height, p.width, p.isp_dtype, p.out_dtype = h, w, dtypes.as_dtype(isp).code, dtypes.as_dtype(out).code
+        p.tonemap, p.gamma, p.color_adapt, p.reinhard_mode = tms[tm], gamma, ca, mode
+        p.flip, p.out_yuv420, p.ids_layout, p.out_pitch = flip, yuv, ids, pitch if pitched else 0
+        if resize:
+            p.out_height, p.out_width, p.scale_r, p.scale_c = ho, wo, ho / h, wo / w
+        exp = _expected_reinhard_scratch(isp, out, tm, gamma, ca, mode, flip, yuv, ids, pitched, resize, n, h, w, ho, wo)
+        assert query(p, n) == exp, (isp, out, tm, gamma, ca, mode, flip, yuv, ids, pitched, resize, h)
+        checked += exp > 0
+    assert checked > 0
+    p = _lib.FusedParams()
+    p.height, p.width, p.isp_dtype, p.out_dtype, p.tonemap, p.gamma = 3000, w, dtypes.f16.code, dtypes.u8.code, 1, 0.9
+    assert query(p, n) == n * 3000 * w * 6 + n * 65536
+    assert query(p, 0) == 0 and query(p, 65) == 0 and query(None, n) == 0     # frame counts the call refuses, no block
+
+    # the ISP's parameter blocks (CPU tensors: _fused_params only reads their shape and allocates the scratch it is told)
+    cpu = torch.device("cpu")
+    T = camera_isp.interpolate.ImageTransform
+    for cam, exact, resize in itertools.product((camera_isp.Camera16, camera_isp.Camera32), (False, True), (False, True)):
+        isp = cam(bayer.BayerPattern.RGGB, device=cpu, reinhard_exact=exact, resize_size=(wo, ho) if resize else None)
+        for h in (3000, 3004):
+            frames = [torch.empty((h, w * 3 // 2), dtype=torch.uint8)] * n
+            for out, tm, gamma, ca, flip, yuv, ids, pitched in itertools.product(
+                    ("u8", "u16", "f16"), ("linear", "reinhard"), (0.29, 0.9, 1.0), (0.0, 0.5), (0, 3, 6), (0, 1), (0, 1), (0, 1)):
+                isp._reinhard_scratch = None
+                p = isp._fused_params(frames, tm, dtypes.as_dtype(out), dict(gamma=gamma, color_adapt=ca), yuv420=yuv,
+                                      ids_format=ids, flip=flip, out_pitch=pitch if pitched else 0)
+                exp = _expected_reinhard_scratch(isp.dtype.name, out, tm, gamma, ca, int(exact), flip, yuv, ids, pitched, resize,
+                                                 n, h, w, ho, wo)
+                assert p.reinhard_scratch_bytes == exp == query(p, n), (cam.__name__, exact, resize, h, out, tm, gamma, ca, flip, yuv, ids, pitched)
+                assert (isp._reinhard_scratch is None) == (exp == 0)
