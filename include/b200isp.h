@@ -32,7 +32,7 @@
 extern "C" {
 #endif
 
-#define B200ISP_VERSION 102            /* 0.1.2 */
+#define B200ISP_VERSION 103            /* 0.1.3 */
 #define B200ISP_MAX_FRAMES 64          /* frames per batched call */
 #define B200ISP_METRICS 9              /* camera_isp.py:102-115 */
 
@@ -193,10 +193,13 @@ typedef struct {
   int resize_gather;            /* 1: force the per-output-pixel gather instead of the resizing sweep (testing / profiling) */
   int out_pitch;                /* elements per OUTPUT row; 0 = dense (3 * width).  Larger: every output frame is a tile of a bigger
                                    image (the rig's camera grid, scripts/tonemap_scan.py:91-100) -- the sweep writes the tile in place */
-  int flip;                     /* ISP transform applied inside the call (interpolate.py:36-56; by the sweep's store, or -- transposing
-                                   transforms on the one-sweep Reinhard -> u8 forms -- by the normalise pass): bit 0 = mirror columns, bit 1 = mirror
-                                   rows, bit 2 = transpose (output (W, H), out_pitch counts elements of ITS rows; needs height % 8 == 0):
-                                   flip_horiz 1, flip_vert 2, rotate_180 3, transpose 4, rotate_270 5, rotate_90 6, transverse 7 */
+  int flip;                     /* ISP transform applied inside the call (interpolate.py:36-56): bit 0 = mirror columns, bit 1 = mirror
+                                   rows, bit 2 = transpose (output (W, H), out_pitch counts elements of ITS rows):
+                                   flip_horiz 1, flip_vert 2, rotate_180 3, transpose 4, rotate_270 5, rotate_90 6, transverse 7.
+                                   1..3 are applied by the sweep's store (no resize, no YUV).  4..7 are applied by the normalise pass
+                                   of a one-sweep Reinhard -> u8 form only: they need height % 8 == 0, height >= 16, a call for which
+                                   b200isp_reinhard_scratch_bytes is not 0 and that scratch; any other call with bit 2 fails with
+                                   B200ISP_E_ARG (run b200isp_transform on its result instead) */
   int reinhard_mode;            /* Camera32 Reinhard -> u8 with reinhard_scratch: 0 = one sweep that also stores the map as u16 fixed point
                                    + a normalise pass where it applies (b200isp_reinhard_scratch_bytes; u8 within 1 LSB of the
                                    two-sweep result, frames whose map leaves [0, 1) are redone exactly), 1 = always the exact max

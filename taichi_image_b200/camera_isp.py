@@ -503,16 +503,13 @@ def camera_isp(name: str, dtype=f32):
                         T.transverse: 7}.get(self.transform, 0)
                 # Transposing transforms (rotate_90 is the rig script's default): the one-sweep Reinhard -> u8 forms turn the
                 # image in their element-wise normalise pass (csrc/fused_isp.cuh reinhard_out_transposed_kernel: shared-memory
-                # tile, 384-byte output pieces) -- no transform kernel, no extra 3 + 3 B/px.  The call takes such a form exactly
-                # when the library asks for a scratch for it; no rule of that query reads the width, so any valid width does.
-                # Elsewhere the sweep's own transposing store stays OPT-IN (B200ISP_FUSED_TRANSPOSE=1): its 24-byte column
-                # pieces are partial-sector writes, L2 fills every one of them from DRAM (profiles/r02_transpose_store.txt:
-                # RGB16 linear 2.2x SLOWER)
+                # tile, 384-byte output pieces) -- no transform kernel, no extra 3 + 3 B/px.  The library accepts bit 2 exactly
+                # when it asks for a scratch for such a form; no rule of that query reads the width, so any valid width does.
+                # Every other call runs the transform kernel on its results.
                 if flip & 4:
                     p = self._param_block(height, 8, tonemap, out_dtype, dict(gamma=gamma, color_adapt=color_adapt),
                                           yuv420, bool(ids_format), flip)
-                    if not (_lib.lib.b200isp_reinhard_scratch_bytes(p, 1) or
-                            (height % 8 == 0 and height >= 16 and os.environ.get("B200ISP_FUSED_TRANSPOSE", "0") == "1")):
+                    if not _lib.lib.b200isp_reinhard_scratch_bytes(p, 1):
                         flip = 0
             return flip
 
@@ -531,7 +528,7 @@ def camera_isp(name: str, dtype=f32):
                 w, h = plan[0]
             oshape = (h * 3 // 2, w) if yuv420 else (h, w, 3)       # planar YUV 4:2:0: color/yuv_420.py:95-118
             if flip & 4:
-                oshape = (w, h, 3)                                  # transposing transform applied by the store
+                oshape = (w, h, 3)                                  # transposing transform applied by the normalise pass
             out_pitch = 0
             if out is None:
                 out = [torch.empty(oshape, dtype=out_dtype.torch, device=self.device) for _ in frames]
@@ -635,9 +632,9 @@ def camera_isp(name: str, dtype=f32):
                     return list(out)
                 return res
             tm = dict(gamma=gamma, intensity=intensity, light_adapt=light_adapt, color_adapt=color_adapt)
-            # every transform of interpolate.py:36-56 is applied by the sweep's store (no extra pass; csrc/fused_isp.cuh
-            # store_out): bit 0 mirrors the columns, bit 1 the rows, bit 2 transposes (needs height % 8 == 0, otherwise the
-            # tiled transform kernel runs on the results)
+            # the transforms of interpolate.py:36-56 inside the call (no extra pass): the flips by the sweep's store
+            # (csrc/fused_isp.cuh store_out), the transposing ones by the normalise pass of the one-sweep Reinhard -> u8 forms;
+            # otherwise (flip == 0) the tiled transform kernel runs on the results
             flip = self._fused_flip(shape[0], tonemap, out_dtype, gamma, color_adapt, ids_format, yuv420)
             if yuv420 or flip or self.transform == interpolate.ImageTransform.none:
                 finish = lambda outs: outs

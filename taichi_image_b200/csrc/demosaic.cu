@@ -19,13 +19,10 @@ template <typename T> struct PlaneSrc {
 
 template <typename InT, typename OutT>
 __global__ void __launch_bounds__(256) demosaic_pixel_kernel(const InT* __restrict__ bayer, OutT* __restrict__ out,
-                                                             int H, int W, int pattern, int ccm, const float9 m,
-                                                             int border_only, long long count) {
+                                                             int H, int W, int pattern, int ccm, const float9 m, long long count) {
   const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (idx >= count) return;
-  int row, col;
-  if (border_only) border_coord(idx, H, W, row, col);
-  else { row = (int)(idx / W); col = (int)(idx % W); }
+  const int row = (int)(idx / W), col = (int)(idx % W);
   const PlaneSrc<InT> src{bayer, W};
   float c[3], t[3];
   malvar_pixel(src, 0, pattern, row, col, H, W, c, t);
@@ -39,13 +36,12 @@ __global__ void __launch_bounds__(256) demosaic_pixel_kernel(const InT* __restri
 }
 
 template <typename InT, typename OutT>
-static int run_demosaic_pixel(const void* bayer, void* rgb, int H, int W, int pattern, const float* ccm,
-                              bool border_only, cudaStream_t s) {
+static int run_demosaic_pixel(const void* bayer, void* rgb, int H, int W, int pattern, const float* ccm, cudaStream_t s) {
   float9 m;
   for (int i = 0; i < 9; ++i) m.v[i] = ccm ? ccm[i] : 0.f;
-  const long long count = border_only ? border_count(H, W) : (long long)H * W;
+  const long long count = (long long)H * W;
   demosaic_pixel_kernel<InT, OutT><<<(unsigned)((count + 255) / 256), 256, 0, s>>>(
-      (const InT*)bayer, (OutT*)rgb, H, W, pattern, ccm != nullptr, m, border_only ? 1 : 0, count);
+      (const InT*)bayer, (OutT*)rgb, H, W, pattern, ccm != nullptr, m, count);
   return cuda_status(cudaPeekAtLastError(), "demosaic_pixel_kernel");
 }
 
@@ -172,7 +168,7 @@ extern "C" int b200isp_bayer_to_rgb(const void* bayer, int in_dtype, void* rgb, 
     ISP_DISPATCH_DTYPE(in_dtype, T, return (run_demosaic_sweep<T>(bayer, rgb, height, width, pattern, ccm9_host, false, s)));
   }
   ISP_DISPATCH_DTYPE(in_dtype, InT, {
-    ISP_DISPATCH_DTYPE(out_dtype, OutT, return (run_demosaic_pixel<InT, OutT>(bayer, rgb, height, width, pattern, ccm9_host, false, s)));
+    ISP_DISPATCH_DTYPE(out_dtype, OutT, return (run_demosaic_pixel<InT, OutT>(bayer, rgb, height, width, pattern, ccm9_host, s)));
   });
   return B200ISP_OK;
 }

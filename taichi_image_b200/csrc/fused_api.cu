@@ -1,4 +1,5 @@
-// C entry point of the fused packed12 sweep + the sparse metering launch (see fused_isp.cuh).
+// C entry point of the fused packed12 sweep + the sparse metering launch (see fused_isp.cuh), and the table form of the
+// Camera16 Reinhard normalise pass.
 #include "fused_isp.cuh"
 #include "resize_isp.cuh"
 
@@ -29,13 +30,12 @@ static int fused_consts(const char* what, int n_frames, const b200isp_fused_para
   k.gamma = p.gamma; k.intensity = p.intensity; k.la = p.light_adapt; k.ca = p.color_adapt;
   ISP_REQUIRE(p.demosaic == B200ISP_DEMOSAIC_MALVAR || p.demosaic == B200ISP_DEMOSAIC_BILINEAR, B200ISP_E_ARG,
               "%s: unknown demosaic %d", what, p.demosaic);
-  k.frame0 = 0;
   k.kbase = p.demosaic == B200ISP_DEMOSAIC_BILINEAR ? kBilinearBase : 0;
   k.flip = p.flip & 7;
   k.gate = 0;
   ISP_REQUIRE(!(k.flip && (resizes(p) || p.out_yuv420)), B200ISP_E_ARG, "%s: flips in the store need the plain RGB sweep (no resize, no YUV)", what);
   ISP_REQUIRE(!(k.flip & 4) || (p.height % 8 == 0 && p.height >= 16), B200ISP_E_SHAPE,
-              "%s: the transposing transforms in the store need height %% 8 == 0 and height >= 16, got %dx%d", what, p.height, p.width);
+              "%s: the transposing transforms need height %% 8 == 0 and height >= 16, got %dx%d", what, p.height, p.width);
   k.ids = p.ids_layout ? 1 : 0;
   ISP_REQUIRE(!(k.ids && resizes(p)), B200ISP_E_ARG, "%s: the IDS layout is not available with the fused resize (re-pack first)", what);
   const int out_cols = (k.flip & 4) ? p.height : p.width;        // the transposing transforms write (W, H) images
@@ -63,8 +63,8 @@ static int fused_setup(const char* what, const uint8_t* const* packed_host, void
   return B200ISP_OK;
 }
 
-// The further checks of b200isp_process_packed12 that read only the parameter block.
-static int process_checks(const b200isp_fused_params& p) {
+// The further checks of b200isp_process_packed12 that read only the parameter block (k: its fused_consts).
+static int process_checks(const b200isp_fused_params& p, const IspConsts& k) {
   ISP_REQUIRE(p.tonemap >= B200ISP_TM_LINEAR && p.tonemap <= B200ISP_TM_NONE, B200ISP_E_ARG, "process_packed12: unknown tonemap %d", p.tonemap);
   ISP_REQUIRE(p.tonemap == B200ISP_TM_NONE || p.gamma > 0.f, B200ISP_E_ARG, "process_packed12: gamma must be positive");
   if (p.tonemap == B200ISP_TM_NONE)
@@ -78,6 +78,11 @@ static int process_checks(const b200isp_fused_params& p) {
   }
   ISP_REQUIRE(!p.out_yuv420 || (p.isp_dtype == B200ISP_F16 && p.out_dtype == B200ISP_U8 && p.tonemap == B200ISP_TM_REINHARD),
               B200ISP_E_ARG, "process_packed12: YUV 4:2:0 output needs Camera16 (f16), Reinhard, u8 and the reinhard_scratch buffer");
+  if (k.flip & 4) {        // only the normalise pass of the one-sweep Reinhard -> u8 forms turns the image
+    const ReinhardForm f = reinhard_plan(p, k, 1).form;
+    ISP_REQUIRE(f == ReinhardForm::kF16Turned || f == ReinhardForm::kU16Turned, B200ISP_E_ARG,
+                "process_packed12: the transposing transforms need a one-sweep Reinhard -> u8 form (b200isp_reinhard_scratch_bytes > 0)");
+  }
   return B200ISP_OK;
 }
 
@@ -105,11 +110,62 @@ ReinhardPlan reinhard_plan(const b200isp_fused_params& p, const IspConsts& k, in
     return {turned ? ReinhardForm::kU16Turned : ReinhardForm::kU16Map, map, map};
   return {ReinhardForm::kExact, 0, 0};
 }
+
+// ReinhardForm::kF16Table: the table form of the Camera16 normalise pass (see kLutBytes in fused_isp.cuh)
+__global__ void __launch_bounds__(256) reinhard_lut_build_kernel(uint8_t* lut /* n_frames x 65536 */, float gamma, const Workspace* ws) {
+  const int frame = blockIdx.y;
+  const uint32_t v = blockIdx.x * 256 + threadIdx.x;
+  const float inv_max = __fdiv_rn(1.0f, fmaxf(1e-6f, __ldcg(&ws->frame_max[frame])));
+  float q = __saturatef(__half2float(__ushort_as_half((unsigned short)v)) * inv_max);
+  if (gamma != 1.0f) q = fast_pow(q, (float)(1.0 / (double)gamma));
+  lut[(size_t)frame * kLutBytes + v] = (uint8_t)Quant<uint8_t>::q(q);
+}
+
+__global__ void __launch_bounds__(512) reinhard_lut_out_kernel(const FramePtrs scratch, const FramePtrs fp, long long n16 /* 16-value chunks per frame */,
+                                                               const uint8_t* __restrict__ lut) {
+  extern __shared__ __align__(16) uint8_t s_lut[];
+  const int frame = gridDim.y - 1 - blockIdx.y;       // last frame first: the sweep wrote it last, part of its map is still in L2
+  {
+    const uint4* g = reinterpret_cast<const uint4*>(lut + (size_t)frame * kLutBytes);
+    uint4* s4 = reinterpret_cast<uint4*>(s_lut);
+    for (int i = threadIdx.x; i < kLutBytes / 16; i += blockDim.x) s4[i] = __ldg(g + i);
+  }
+  __syncthreads();
+  const uint4* src = reinterpret_cast<const uint4*>(scratch.out[frame]);
+  uint4* dst = reinterpret_cast<uint4*>(fp.out[frame]);
+  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n16; i += (long long)gridDim.x * blockDim.x) {
+    const uint4 w0 = __ldcs(src + 2 * i), w1 = __ldcs(src + 2 * i + 1);
+    const uint32_t w[8] = {w0.x, w0.y, w0.z, w0.w, w1.x, w1.y, w1.z, w1.w};
+    uint32_t o[4];
+#pragma unroll
+    for (int j = 0; j < 4; ++j) {
+      const uint32_t a = s_lut[w[2 * j] & 0xFFFFu], b = s_lut[w[2 * j] >> 16], c = s_lut[w[2 * j + 1] & 0xFFFFu], d = s_lut[w[2 * j + 1] >> 16];
+      o[j] = a | (b << 8) | (c << 16) | (d << 24);
+    }
+    __stcs(dst + i, make_uint4(o[0], o[1], o[2], o[3]));
+  }
+}
+
+int run_lut_pass(const FramePtrs& sc, const FramePtrs& fp, int n_frames, long long n_elems, uint8_t* lut, float gamma, const Workspace* ws,
+                 cudaStream_t s) {
+  reinhard_lut_build_kernel<<<dim3(kLutBytes / 256, (unsigned)n_frames), 256, 0, s>>>(lut, gamma, ws);
+  int st = cuda_status(cudaPeekAtLastError(), "reinhard_lut_build_kernel");
+  if (st) return st;
+  static bool attr_set = false;          // per process; the attribute belongs to the function, not to a device context
+  if (!attr_set) {
+    st = cuda_status(cudaFuncSetAttribute(reinhard_lut_out_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kLutBytes), "lut smem attribute");
+    if (st) return st;
+    attr_set = true;
+  }
+  const dim3 grid((unsigned)std::min<long long>((n_elems / 16 + 511) / 512, (3 * kNumSMs + n_frames - 1) / n_frames), (unsigned)n_frames);
+  reinhard_lut_out_kernel<<<grid, 512, kLutBytes, s>>>(sc, fp, n_elems / 16, lut);
+  return cuda_status(cudaPeekAtLastError(), "reinhard_lut_out_kernel");
+}
 }  // namespace isp
 
 extern "C" size_t b200isp_reinhard_scratch_bytes(const b200isp_fused_params* params, int n_frames) {
   IspConsts k;
-  if (!params || fused_consts("reinhard_scratch_bytes", n_frames, *params, k) || process_checks(*params)) return 0;
+  if (!params || fused_consts("reinhard_scratch_bytes", n_frames, *params, k) || process_checks(*params, k)) return 0;
   return reinhard_plan(*params, k, n_frames).bytes;
 }
 
@@ -215,7 +271,7 @@ extern "C" int b200isp_process_packed12(const uint8_t* const* packed_host, void*
   ISP_REQUIRE(out_host, B200ISP_E_ARG, "process_packed12: null output list");
   {
     int st = fused_setup("process_packed12", packed_host, out_host, n_frames, params, metrics, workspace, fp, k);
-    if (!st) st = process_checks(*params);
+    if (!st) st = process_checks(*params, k);
     if (st) return st;
   }
   const b200isp_fused_params& p = *params;

@@ -71,7 +71,6 @@ template <bool CAM16, bool EXT = false>
 struct Packed12Loader2 {
   FramePtrs fp;
   int pitch_words;       // W * 3 / 8
-  int frame0;
   int ids;               // 0: standard layout (packed.py:23-31), 1: IDS layout (packed.py:36-44), kernel-uniform
   static constexpr uint32_t kRowMask = 0x007FF800u;
   struct Raw { uint32_t w[5]; };
@@ -81,7 +80,7 @@ struct Packed12Loader2 {
 
   template <int KIND>
   __device__ __forceinline__ void open(Cursor& c, int frame, int tcol, const StreamGeom& g) const {
-    c.p = reinterpret_cast<const uint32_t*>(fp.in[frame0 + frame]) + 3 * tcol;
+    c.p = reinterpret_cast<const uint32_t*>(fp.in[frame]) + 3 * tcol;
     c.left = KIND == K_CORE || tcol > 0;
     c.right = KIND == K_CORE || tcol < g.ntcols - 1;
     c.mL = c.left ? 0xFFFFFFFFu : 0u;
@@ -186,10 +185,10 @@ struct IspConsts {
   float gamma, intensity, la, ca;
   const float* metrics;      // device, 9 floats
   Workspace* ws;
-  int frame0;
   int kbase;                 // 0: Malvar-He-Cutler, kBilinearBase: bilinear demosaic (offset into c_taps / c_border)
   int ids;                   // packed layout of the input frames: 0 standard, 1 IDS
-  int flip;                  // transform applied by the store: bit 0 horizontal, bit 1 vertical (rotate_180 = 3), bit 2 transposed
+  int flip;                  // transform applied inside the call: bit 0 horizontal, bit 1 vertical (rotate_180 = 3) by the store;
+                             //    bit 2 transposed, by reinhard_out_transposed_kernel only (the sweep never sees it)
   int orow;                  // elements per OUTPUT row: 3 W for dense frames, more when the frames are tiles of a grid image
   int gate;                  // 1: the sweep runs only on the frames the one-sweep u16 Reinhard map declined (reinhard_map16_declined),
                              //    their max goes to / comes from ws->frame_max2; 0 everywhere else
@@ -295,59 +294,11 @@ __device__ __forceinline__ void store_row8(const WarpCtx& wc, OutT* warp_out /* 
 // (lane order reversed in the stage, the lane's eight pixels reversed before packing) -- no extra pass over the image.
 // k.flip: bit 0 = horizontal, bit 1 = vertical; kernel-uniform, 0 on the hot path.
 // EXT: only the extended instantiations carry the flip code (see Packed12Loader2).
-// The TRANSPOSING transforms (k.flip bit 2; interpolate.py:36-56: rotate_90 / rotate_270 / transpose / transverse) turn an
-// image row into an output column: output (i, j) = source (r, c) with i = c or W-1-c (bit 0) and j = r or H-1-r (bit 1),
-// output shape (W, H).  A lane owns its eight source columns for the whole task, so the pixels that are contiguous in an
-// output row -- the same column of consecutive source rows -- all come from the same lane: it collects 24 bytes per column
-// (kTileRows rows) in a private piece of the warp's stage (layout [pixel][lane], pitch 7 words: conflict-free) and then
-// writes each as three 8-byte stores.  The 24-byte pieces of one task are adjacent in the output row, so L2 merges them
-// into whole sectors before they reach DRAM (default write policy, not evict-first).  Tasks start on tile boundaries
-// (Stream2Geom::border = 8, rows_per_task % 8 == 0, H % 8 == 0: checked on the host).
-constexpr int kTransposeStageWords = 8 * 32 * 7;
-template <typename OutT>
-__device__ __forceinline__ void store_transposed(const WarpCtx& wc, OutT* frame_out, const IspConsts& k, int row, const uint32_t (&v)[24]) {
-  constexpr int ES = (int)sizeof(OutT);
-  constexpr int TR = 8 / ES;                      // rows per tile: 8 (u8), 4 (u16 / f16), 2 (f32)
-  const int s = row & (TR - 1);
-  const int slot = (k.flip & 2) ? TR - 1 - s : s;
-  OutT* mine = reinterpret_cast<OutT*>(wc.stage + 7 * wc.lane) + 3 * slot;
-#pragma unroll
-  for (int q = 0; q < 8; ++q) {
-    OutT* p = mine + q * (32 * 28 / ES);
-#pragma unroll
-    for (int ch = 0; ch < 3; ++ch) {
-      if constexpr (std::is_same<OutT, __half>::value) p[ch] = __float2half_rn(__uint_as_float(v[3 * q + ch]));
-      else if constexpr (std::is_same<OutT, float>::value) p[ch] = __uint_as_float(v[3 * q + ch]);
-      else p[ch] = (OutT)v[3 * q + ch];
-    }
-  }
-  if (s != TR - 1) return;
-  const int rt = row - (TR - 1);
-  const int j0 = (k.flip & 2) ? k.H - TR - rt : rt;                 // first output column of the pieces
-  const size_t opitch = (size_t)k.orow * ES;                        // bytes per output row (dense: 3 * H elements)
-  const int c0 = 8 * (wc.tcol0 + wc.lane);
-  if (wc.lane >= wc.nvalid) return;
-  char* obase = reinterpret_cast<char*>(frame_out) + (size_t)j0 * 3 * ES;
-#pragma unroll
-  for (int q = 0; q < 8; ++q) {
-    const uint32_t* sp = wc.stage + 7 * (q * 32 + wc.lane);
-    const int c = c0 + q;                                           // < W: the width is a multiple of 8
-    uint2* d = reinterpret_cast<uint2*>(obase + (size_t)((k.flip & 1) ? k.W - 1 - c : c) * opitch);
-    d[0] = make_uint2(sp[0], sp[1]);
-    d[1] = make_uint2(sp[2], sp[3]);
-    d[2] = make_uint2(sp[4], sp[5]);
-  }
-}
-
 template <typename OutT, bool FULL = false, bool EXT = false>
 __device__ __forceinline__ void store_out(const WarpCtx& wc, OutT* warp_out /* frame + 24 * tcol0 */, const IspConsts& k, int row,
                                           const uint32_t (&v)[24]) {
   if (!EXT || k.flip == 0) {
     store_row8<OutT, FULL>(wc, warp_out, k.orow, row, v);
-    return;
-  }
-  if (k.flip & 4) {
-    store_transposed<OutT>(wc, warp_out - 24 * wc.tcol0, k, row, v);
     return;
   }
   const int orow_idx = (k.flip & 2) ? k.H - 1 - row : row;
@@ -452,7 +403,7 @@ __device__ __forceinline__ ReinhardConsts reinhard_consts(const IspConsts& k, in
   c.out_scale_inv_max = 0.f;
   c.max_out = 1.0f;
   if (with_max) {
-    c.max_out = fmaxf(1e-6f, __ldcg(k.gate ? &k.ws->frame_max2[k.frame0 + frame] : &k.ws->frame_max[k.frame0 + frame]));      // camera_isp.py:190, :213
+    c.max_out = fmaxf(1e-6f, __ldcg(k.gate ? &k.ws->frame_max2[frame] : &k.ws->frame_max[frame]));      // camera_isp.py:190, :213
     c.out_scale_inv_max = __fdiv_rn(1.0f, c.max_out);
   }
   return c;
@@ -740,10 +691,10 @@ template <bool CAM16, typename OutT, bool EXT = false>
 struct EpiRgb2 {      // load_packed12: ISP-dtype float RGB out
   FramePtrs fp;
   IspConsts k;
-  static constexpr int kStageWords = EXT ? kTransposeStageWords : 32 * Quant<OutT>::kWords;
+  static constexpr int kStageWords = 32 * Quant<OutT>::kWords;
   struct State { OutT* out; WarpCtx wc; int edge; };
   __device__ __forceinline__ void init(State& st, int frame, int tcol, const WarpCtx& wc) const {
-    st.out = reinterpret_cast<OutT*>(fp.out[k.frame0 + frame]) + 24 * wc.tcol0;
+    st.out = reinterpret_cast<OutT*>(fp.out[frame]) + 24 * wc.tcol0;
     st.wc = wc;
     st.edge = edge_bits(tcol, k.W);
   }
@@ -772,11 +723,11 @@ struct EpiLinear2 {
   static_assert(!(FAST && CAM16), "the packed fast path is Camera32 only");
   FramePtrs fp;
   IspConsts k;
-  static constexpr int kStageWords = EXT ? kTransposeStageWords : 32 * Quant<OutT>::kWords;
+  static constexpr int kStageWords = 32 * Quant<OutT>::kWords;
   struct State { LinearConsts c; OutT* out; WarpCtx wc; int edge; bool inside; };
   __device__ __forceinline__ void init(State& st, int frame, int tcol, const WarpCtx& wc) const {
     st.c = linear_consts(k.metrics, k.gamma);
-    st.out = reinterpret_cast<OutT*>(fp.out[k.frame0 + frame]) + 24 * wc.tcol0;
+    st.out = reinterpret_cast<OutT*>(fp.out[frame]) + 24 * wc.tcol0;
     st.wc = wc;
     st.edge = edge_bits(tcol, k.W);
     // With bounds inside [0,1] (always true for metered bounds: the metered images are clamped to [0,1],
@@ -887,13 +838,13 @@ struct EpiReinhardMax2 {      // pass 1: frame-global max of the mapped values (
   static constexpr bool kGated = GATED;
   static constexpr int kStageWords = STORE ? 32 * Quant<ScratchT>::kWords : 0;
   struct State { ReinhardConsts c; float mx; int edge; ScratchT* out; WarpCtx wc; };
-  __device__ __forceinline__ bool enabled(int frame) const { return reinhard_map16_declined(__ldcg(&k.ws->frame_max[k.frame0 + frame])); }
+  __device__ __forceinline__ bool enabled(int frame) const { return reinhard_map16_declined(__ldcg(&k.ws->frame_max[frame])); }
   __device__ __forceinline__ void init(State& st, int frame, int tcol, const WarpCtx& wc) const {
     st.c = reinhard_consts(k, frame, false);
     st.mx = 0.f;
     st.edge = edge_bits(tcol, k.W);
     st.wc = wc;
-    st.out = STORE ? reinterpret_cast<ScratchT*>(fp.out[k.frame0 + frame]) + 24 * wc.tcol0 : nullptr;
+    st.out = STORE ? reinterpret_cast<ScratchT*>(fp.out[frame]) + 24 * wc.tcol0 : nullptr;
   }
   static constexpr bool kSplitEdge = false;     // measured: a separate K_CORE copy costs more (instruction cache) than its leaner code saves
   static constexpr bool kCompactLoop = true;
@@ -994,7 +945,7 @@ struct EpiReinhardMax2 {      // pass 1: frame-global max of the mapped values (
   __device__ __forceinline__ void finish(State& st, int frame, int lane, bool task_ok) const {
     const float m = warp_max(st.mx);
     if (lane == 0 && task_ok && m > 0.f)
-      atomicMax(reinterpret_cast<unsigned int*>(GATED ? &k.ws->frame_max2[k.frame0 + frame] : &k.ws->frame_max[k.frame0 + frame]),
+      atomicMax(reinterpret_cast<unsigned int*>(GATED ? &k.ws->frame_max2[frame] : &k.ws->frame_max[frame]),
                 __float_as_uint(m));
   }
 };
@@ -1004,12 +955,12 @@ struct EpiReinhard2 {         // pass 2 recomputed from the packed frame: map, n
   FramePtrs fp;
   IspConsts k;                // GATED (k.gate == 1): only the frames the one-sweep u16 map declined, max from ws->frame_max2
   static constexpr bool kGated = GATED;
-  __device__ __forceinline__ bool enabled(int frame) const { return reinhard_map16_declined(__ldcg(&k.ws->frame_max[k.frame0 + frame])); }
-  static constexpr int kStageWords = EXT ? kTransposeStageWords : 32 * Quant<OutT>::kWords;
+  __device__ __forceinline__ bool enabled(int frame) const { return reinhard_map16_declined(__ldcg(&k.ws->frame_max[frame])); }
+  static constexpr int kStageWords = 32 * Quant<OutT>::kWords;
   struct State { ReinhardConsts c; OutT* out; WarpCtx wc; int edge; };
   __device__ __forceinline__ void init(State& st, int frame, int tcol, const WarpCtx& wc) const {
     st.c = reinhard_consts(k, frame, true);
-    st.out = reinterpret_cast<OutT*>(fp.out[k.frame0 + frame]) + 24 * wc.tcol0;
+    st.out = reinterpret_cast<OutT*>(fp.out[frame]) + 24 * wc.tcol0;
     st.wc = wc;
     st.edge = edge_bits(tcol, k.W);
   }
@@ -1304,12 +1255,11 @@ static int launch_reinhard(const Packed12Loader2<CAM16, EXT>& ld, const FramePtr
 // bilinear + IDS / flip through the re-pack pass / the transform kernel.
 template <bool CAM16, int MODE, typename OutT, bool EXT>
 static int run_pass_ext(const FramePtrs& fp, IspConsts k, int nframes, int rows_per_task, cudaStream_t s, void* ev_start, void* ev_stop) {
-  k.frame0 = 0;
-  const Stream2Geom g = make_geom2(k.H, k.W, nframes, rows_per_task, (EXT && MODE != MODE_RMAX && (k.flip & 4)) ? 8 : 2);
+  const Stream2Geom g = make_geom2(k.H, k.W, nframes, rows_per_task);
   const bool bl = !EXT && k.kbase != 0;
   if (EXT && k.kbase != 0) { set_error("process_packed12: the IDS layout / flips are fused for the Malvar demosaic only"); return B200ISP_E_ARG; }
   Packed12Loader2<CAM16, EXT> ld;
-  ld.fp = fp; ld.pitch_words = k.W * 3 / 8; ld.frame0 = 0; ld.ids = k.ids;
+  ld.fp = fp; ld.pitch_words = k.W * 3 / 8; ld.ids = k.ids;
   int st = B200ISP_OK;
   auto record = [&](void* ev) { record_profile_event(ev, s); };
   if (ev_start) record(ev_start);
@@ -1411,8 +1361,8 @@ __device__ __forceinline__ uint32_t pack4_u8(uint32_t a, uint32_t b, uint32_t c,
 
 template <bool GAMMA, bool PITCHED>
 __global__ void __launch_bounds__(256) reinhard_map16_out_kernel(const FramePtrs scratch /* .out = u16 maps */, const FramePtrs fp,
-                                                                 int H, int W, int orow, float gamma, const Workspace* ws, int frame0) {
-  const int frame = frame0 + gridDim.y - 1 - blockIdx.y;       // last frame first: the sweep wrote it last, part of its map is still in L2
+                                                                 int H, int W, int orow, float gamma, const Workspace* ws) {
+  const int frame = gridDim.y - 1 - blockIdx.y;       // last frame first: the sweep wrote it last, part of its map is still in L2
   const float mx = __ldcg(&ws->frame_max[frame]);
   if (reinhard_map16_declined(mx)) return;
   const uint4* src = reinterpret_cast<const uint4*>(scratch.out[frame]);
@@ -1463,79 +1413,17 @@ __global__ void __launch_bounds__(256) reinhard_map16_out_kernel(const FramePtrs
   }
 }
 
-// pass B through a table (gamma != 1, dense u8 outputs): both 16-bit scratch formats -- the f16 map of Camera16 and the u16
-// fixed-point map of Camera32 -- have only 65 536 patterns, and the output is a pure function of the pattern and the frame
-// maximum.  reinhard_lut_build_kernel evaluates that function once per pattern and frame with exactly the arithmetic of
-// reinhard_scratch_out_kernel / map16_pair (so the result is bit-identical to them); reinhard_lut_out_kernel keeps the frame's
-// 64 KB table in shared memory and turns every value into one LDS.U8: no MUFU (the arithmetic pass needs 6 per pixel and sits
-// at 74 % of the MUFU pipe), 10 instead of 21 instructions per pixel -- the pass becomes a plain HBM stream.  run_fused
-// uses it for Camera16 only: the Camera32 pass (reinhard_map16_out_kernel) is bound by its 2 : 1 read / write DRAM stream
-// (4.75 TB/s), not by the MUFU pipe, and the table form measured 134.9 vs 131.5 us on cfg3.
+// pass B through a table (Camera16, gamma != 1, dense u8 outputs): the f16 map has only 65 536 patterns, and the output is a
+// pure function of the pattern and the frame maximum.  reinhard_lut_build_kernel evaluates that function once per pattern and
+// frame with exactly the arithmetic of reinhard_scratch_out_kernel (so the result is bit-identical to it); reinhard_lut_out_kernel
+// keeps the frame's 64 KB table in shared memory and turns every value into one LDS.U8: no MUFU (the arithmetic pass needs 6 per
+// pixel and sits at 74 % of the MUFU pipe), 10 instead of 21 instructions per pixel -- the pass becomes a plain HBM stream.
+// Camera32 has no table form: its pass (reinhard_map16_out_kernel) is bound by its 2 : 1 read / write DRAM stream (4.75 TB/s),
+// not by the MUFU pipe, and the table form measured 134.9 vs 131.5 us on cfg3.
 constexpr int kLutBytes = 65536;
-template <bool CAM16>
-__global__ void __launch_bounds__(256) reinhard_lut_build_kernel(uint8_t* lut /* n_frames x 65536 */, float gamma, const Workspace* ws) {
-  const int frame = blockIdx.y;
-  const uint32_t v = blockIdx.x * 256 + threadIdx.x;
-  const float mx = __ldcg(&ws->frame_max[frame]);
-  uint32_t out;
-  if constexpr (CAM16) {
-    const float inv_max = __fdiv_rn(1.0f, fmaxf(1e-6f, mx));
-    float q = __saturatef(__half2float(__ushort_as_half((unsigned short)v)) * inv_max);
-    if (gamma != 1.0f) q = fast_pow(q, (float)(1.0 / (double)gamma));
-    out = Quant<uint8_t>::q(q);
-  } else {
-    if (reinhard_map16_declined(mx)) return;
-    const float a = __fdiv_rn(__fdiv_rn(1.0f, mx), kMap16Scale);
-    uint32_t v1;
-    map16_pair(v | (v << 16), bc(a), bc(0.5f * a), bc((float)(1.0 / (double)gamma)), gamma != 1.0f, out, v1);
-  }
-  lut[(size_t)frame * kLutBytes + v] = (uint8_t)out;
-}
-
-template <bool CAM16>
-__global__ void __launch_bounds__(512) reinhard_lut_out_kernel(const FramePtrs scratch, const FramePtrs fp, long long n16 /* 16-value chunks per frame */,
-                                                               const uint8_t* __restrict__ lut, const Workspace* ws) {
-  extern __shared__ __align__(16) uint8_t s_lut[];
-  const int frame = gridDim.y - 1 - blockIdx.y;       // last frame first: the sweep wrote it last, part of its map is still in L2
-  if (!CAM16 && reinhard_map16_declined(__ldcg(&ws->frame_max[frame]))) return;
-  {
-    const uint4* g = reinterpret_cast<const uint4*>(lut + (size_t)frame * kLutBytes);
-    uint4* s4 = reinterpret_cast<uint4*>(s_lut);
-    for (int i = threadIdx.x; i < kLutBytes / 16; i += blockDim.x) s4[i] = __ldg(g + i);
-  }
-  __syncthreads();
-  const uint4* src = reinterpret_cast<const uint4*>(scratch.out[frame]);
-  uint4* dst = reinterpret_cast<uint4*>(fp.out[frame]);
-  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n16; i += (long long)gridDim.x * blockDim.x) {
-    const uint4 w0 = __ldcs(src + 2 * i), w1 = __ldcs(src + 2 * i + 1);
-    const uint32_t w[8] = {w0.x, w0.y, w0.z, w0.w, w1.x, w1.y, w1.z, w1.w};
-    uint32_t o[4];
-#pragma unroll
-    for (int j = 0; j < 4; ++j) {
-      const uint32_t a = s_lut[w[2 * j] & 0xFFFFu], b = s_lut[w[2 * j] >> 16], c = s_lut[w[2 * j + 1] & 0xFFFFu], d = s_lut[w[2 * j + 1] >> 16];
-      o[j] = a | (b << 8) | (c << 16) | (d << 24);
-    }
-    __stcs(dst + i, make_uint4(o[0], o[1], o[2], o[3]));
-  }
-}
-
-// launches the table form of pass B; lut = n_frames x 64 KB behind the maps in the caller's scratch
-template <bool CAM16>
-static int run_lut_pass(const FramePtrs& sc, const FramePtrs& fp, int n_frames, long long n_elems, uint8_t* lut, float gamma, const Workspace* ws,
-                        cudaStream_t s) {
-  reinhard_lut_build_kernel<CAM16><<<dim3(kLutBytes / 256, (unsigned)n_frames), 256, 0, s>>>(lut, gamma, ws);
-  int st = cuda_status(cudaPeekAtLastError(), "reinhard_lut_build_kernel");
-  if (st) return st;
-  static bool attr_set = false;          // per process and instantiation; the attribute belongs to the function, not to a device context
-  if (!attr_set) {
-    st = cuda_status(cudaFuncSetAttribute(reinhard_lut_out_kernel<CAM16>, cudaFuncAttributeMaxDynamicSharedMemorySize, kLutBytes), "lut smem attribute");
-    if (st) return st;
-    attr_set = true;
-  }
-  const dim3 grid((unsigned)std::min<long long>((n_elems / 16 + 511) / 512, (3 * kNumSMs + n_frames - 1) / n_frames), (unsigned)n_frames);
-  reinhard_lut_out_kernel<CAM16><<<grid, 512, kLutBytes, s>>>(sc, fp, n_elems / 16, lut, ws);
-  return cuda_status(cudaPeekAtLastError(), "reinhard_lut_out_kernel");
-}
+// the table form of pass B (defined in fused_api.cu); lut = n_frames x 64 KB behind the maps in the caller's scratch
+int run_lut_pass(const FramePtrs& sc, const FramePtrs& fp, int n_frames, long long n_elems, uint8_t* lut, float gamma, const Workspace* ws,
+                 cudaStream_t s);
 
 // pass B with planar YUV 4:2:0 output (SURVEY 8f-2, for video encoders): the u8 RGB of reinhard_scratch_out_kernel
 // is formed in registers and converted with the arithmetic of color/yuv_420.py:47-64 (csrc/yuv420.cu: x / 255, the
@@ -1692,12 +1580,11 @@ static int run_out_transposed(const FramePtrs& sc, const FramePtrs& fp, int n_fr
 // map (any color_adapt), Camera32 the u16 fixed-point map (color_adapt == 0 only: the caller checks)
 template <bool CAM16>
 int run_rstore(const FramePtrs& fp_scratch, IspConsts k, int nframes, int rows_per_task, cudaStream_t s, void* ev_start, void* ev_stop) {
-  k.frame0 = 0;
   const Stream2Geom g = make_geom2(k.H, k.W, nframes, rows_per_task);
   int st = B200ISP_OK;
   if (ev_start) record_profile_event(ev_start, s);
   auto launch = [&](auto ld, bool bl) -> int {
-    ld.fp = fp_scratch; ld.pitch_words = k.W * 3 / 8; ld.frame0 = 0; ld.ids = k.ids;
+    ld.fp = fp_scratch; ld.pitch_words = k.W * 3 / 8; ld.ids = k.ids;
     ISP_DISPATCH_PATTERN(k.pattern, P, {
       if (k.ca == 0.f) { EpiReinhardMax2<CAM16, true, true> e{fp_scratch, k}; st = launch_stream2<P>(ld, e, g, s, "isp_stream<reinhard_store>", bl); }
       else if constexpr (CAM16) { EpiReinhardMax2<true, false, true> e{fp_scratch, k}; st = launch_stream2<P>(ld, e, g, s, "isp_stream<reinhard_store>", bl); }
@@ -1760,6 +1647,10 @@ int run_fused(const FramePtrs& fp, int n_frames, const b200isp_fused_params& p, 
     set_error("process_packed12: YUV 4:2:0 output needs Camera16 (f16), Reinhard, u8 and the reinhard_scratch buffer");
     return B200ISP_E_ARG;
   }
+  if ((k.flip & 4) && plan.form == ReinhardForm::kExact) {
+    set_error("process_packed12: the transposing transforms need the reinhard_scratch buffer (b200isp_reinhard_scratch_bytes)");
+    return B200ISP_E_ARG;
+  }
   constexpr bool kIspOut = (CAM16 && std::is_same<OutT, __half>::value) || (!CAM16 && std::is_same<OutT, float>::value);
   if (p.tonemap == B200ISP_TM_NONE) {
     if constexpr (kIspOut) return run_pass<CAM16, MODE_RGB, OutT>(fp, k, n_frames, rpt, s, p.profile_start, p.profile_stop);
@@ -1794,7 +1685,7 @@ int run_fused(const FramePtrs& fp, int n_frames, const b200isp_fused_params& p, 
         const long long n_elems = (long long)k.H * k.W * 3;
         if constexpr (std::is_same<OutT, uint8_t>::value) {
           if (plan.form == ReinhardForm::kF16Table)
-            return run_lut_pass<true>(sc, fp, n_frames, n_elems, (uint8_t*)p.reinhard_scratch + plan.map_bytes, k.gamma, k.ws, s);
+            return run_lut_pass(sc, fp, n_frames, n_elems, (uint8_t*)p.reinhard_scratch + plan.map_bytes, k.gamma, k.ws, s);
         }
         const dim3 grid((unsigned)std::min<long long>((n_elems / 8 + 255) / 256, 4 * kNumSMs), (unsigned)n_frames);
         reinhard_scratch_out_kernel<OutT><<<grid, 256, 0, s>>>(sc, fp, n_elems, k.gamma, k.ws);
@@ -1832,10 +1723,10 @@ int run_fused(const FramePtrs& fp, int n_frames, const b200isp_fused_params& p, 
         const long long n_elems = (long long)k.H * k.W * 3;
         const bool gam = k.gamma != 1.0f, pitched = k.orow != 3 * k.W;
         const dim3 grid((unsigned)std::min<long long>((n_elems / 16 + 255) / 256, (8 * kNumSMs + n_frames - 1) / n_frames), (unsigned)n_frames);
-        if (gam && pitched) reinhard_map16_out_kernel<true, true><<<grid, 256, 0, s>>>(sc, fp, k.H, k.W, k.orow, k.gamma, k.ws, 0);
-        else if (gam) reinhard_map16_out_kernel<true, false><<<grid, 256, 0, s>>>(sc, fp, k.H, k.W, k.orow, k.gamma, k.ws, 0);
-        else if (pitched) reinhard_map16_out_kernel<false, true><<<grid, 256, 0, s>>>(sc, fp, k.H, k.W, k.orow, k.gamma, k.ws, 0);
-        else reinhard_map16_out_kernel<false, false><<<grid, 256, 0, s>>>(sc, fp, k.H, k.W, k.orow, k.gamma, k.ws, 0);
+        if (gam && pitched) reinhard_map16_out_kernel<true, true><<<grid, 256, 0, s>>>(sc, fp, k.H, k.W, k.orow, k.gamma, k.ws);
+        else if (gam) reinhard_map16_out_kernel<true, false><<<grid, 256, 0, s>>>(sc, fp, k.H, k.W, k.orow, k.gamma, k.ws);
+        else if (pitched) reinhard_map16_out_kernel<false, true><<<grid, 256, 0, s>>>(sc, fp, k.H, k.W, k.orow, k.gamma, k.ws);
+        else reinhard_map16_out_kernel<false, false><<<grid, 256, 0, s>>>(sc, fp, k.H, k.W, k.orow, k.gamma, k.ws);
         if ((st = cuda_status(cudaPeekAtLastError(), "reinhard_map16_out_kernel"))) return st;
         IspConsts kg = k;
         kg.gate = 1;

@@ -48,7 +48,6 @@ int run_resize_pass(const FramePtrs& io, const IspConsts& k, const b200isp_fused
 template <bool CAM16, int MODE, typename OutT>
 int run_resize_pass_impl(const FramePtrs& io, const IspConsts& k0, const b200isp_fused_params& p, int n_frames, cudaStream_t s) {
   IspConsts k = k0;
-  k.frame0 = 0;
   const ResizeSrc<CAM16> src = make_resize_src<CAM16>(io, k, p);
   const bool sweep = p.scale_r <= 1.0f && p.scale_c <= 1.0f && p.out_width >= 64 && p.out_height >= 8 && !p.resize_gather;
   if (!sweep) {
@@ -58,7 +57,7 @@ int run_resize_pass_impl(const FramePtrs& io, const IspConsts& k0, const b200isp
   }
   const ResizeTasks rt = make_resize_tasks(k.H, k.W, n_frames, p.out_height, p.scale_r, p.rows_per_task);
   Packed12Loader2<CAM16> ld;
-  ld.fp = io; ld.pitch_words = k.W * 3 / 8; ld.frame0 = 0; ld.ids = 0;
+  ld.fp = io; ld.pitch_words = k.W * 3 / 8; ld.ids = 0;
   const EpiResize2<CAM16, MODE, OutT> epi{io, k, p.out_height, p.out_width, p.scale_r, p.scale_c};
   const long long blocks = (rt.total_tasks + kS2Warps - 1) / kS2Warps;
   ISP_DISPATCH_PATTERN(k.pattern, P, {

@@ -1,7 +1,6 @@
 // Per-pixel (gather) form of the Malvar demosaic, literal to bayer.py:137-155: 13 bounds-checked taps
 // accumulated in table order, products and sums rounded separately, normaliser t = in-bounds weights.
-// Used (a) by the border kernels that rewrite the 2-pixel image frame after a streaming kernel,
-// (b) by the sparse metering samplers, (c) for ragged / mixed-dtype stand-alone demosaic.
+// Used by the sparse metering samplers, the resizing ISP's gather and the ragged / mixed-dtype stand-alone demosaic.
 #pragma once
 #include "common.cuh"
 
@@ -58,26 +57,6 @@ __device__ __forceinline__ void ccm_apply(const float* m, float& r, float& g, fl
   const float y = __fadd_rn(__fadd_rn(__fmul_rn(r, m[3]), __fmul_rn(g, m[4])), __fmul_rn(b, m[5]));
   const float z = __fadd_rn(__fadd_rn(__fmul_rn(r, m[6]), __fmul_rn(g, m[7])), __fmul_rn(b, m[8]));
   r = x; g = y; b = z;
-}
-
-// ---------------------------------------------------------------- border frame enumeration
-// The 2-pixel frame of an H x W image: rows {0,1,H-2,H-1} in full, columns {0,1,W-2,W-1} of the rest.
-__host__ __device__ inline long long border_count(int H, int W) {
-  if (H < 4 || W < 4) return (long long)H * W;
-  return 4LL * W + 4LL * (H - 4);
-}
-__device__ __forceinline__ void border_coord(long long idx, int H, int W, int& row, int& col) {
-  if (H < 4 || W < 4) { row = (int)(idx / W); col = (int)(idx % W); return; }
-  if (idx < 4LL * W) {
-    const int k = (int)(idx / W);
-    row = k < 2 ? k : H - 4 + k;
-    col = (int)(idx % W);
-  } else {
-    const long long k = idx - 4LL * W;
-    row = 2 + (int)(k >> 2);
-    const int q = (int)(k & 3);
-    col = q < 2 ? q : W - 4 + q;
-  }
 }
 
 }  // namespace isp

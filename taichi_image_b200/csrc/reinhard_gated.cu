@@ -7,10 +7,9 @@
 namespace isp {
 
 int run_rmax_gated(const FramePtrs& fp, IspConsts k, int nframes, int rows_per_task, cudaStream_t s) {
-  k.frame0 = 0;
   const Stream2Geom g = make_geom2(k.H, k.W, nframes, rows_per_task);
   Packed12Loader2<false, false> ld;
-  ld.fp = fp; ld.pitch_words = k.W * 3 / 8; ld.frame0 = 0; ld.ids = 0;
+  ld.fp = fp; ld.pitch_words = k.W * 3 / 8; ld.ids = 0;
   int st = B200ISP_OK;
   ISP_DISPATCH_PATTERN(k.pattern, P, {
     EpiReinhardMax2<false, true, false, true> e{fp, k};
@@ -20,10 +19,9 @@ int run_rmax_gated(const FramePtrs& fp, IspConsts k, int nframes, int rows_per_t
 }
 
 int run_write_gated(const FramePtrs& fp, IspConsts k, int nframes, int rows_per_task, cudaStream_t s) {
-  k.frame0 = 0;
   const Stream2Geom g = make_geom2(k.H, k.W, nframes, rows_per_task);
   Packed12Loader2<false, false> ld;
-  ld.fp = fp; ld.pitch_words = k.W * 3 / 8; ld.frame0 = 0; ld.ids = 0;
+  ld.fp = fp; ld.pitch_words = k.W * 3 / 8; ld.ids = 0;
   int st = B200ISP_OK;
   ISP_DISPATCH_PATTERN(k.pattern, P, {
     if (k.gamma != 1.0f) { EpiReinhard2<false, uint8_t, true, true, false, true> e{fp, k}; st = launch_stream2<P>(ld, e, g, s, "isp_stream<reinhard,gated>", k.kbase != 0); }

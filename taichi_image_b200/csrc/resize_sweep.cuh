@@ -125,7 +125,7 @@ struct EpiResize2 {
 
   __device__ __forceinline__ void init(State& st, int frame, int tcol, const WarpCtx& wc, int ro0, int ro1, bool last_strip) const {
     st.tone.init(k, frame);
-    st.out = reinterpret_cast<OutT*>(fp.out[k.frame0 + frame]);
+    st.out = reinterpret_cast<OutT*>(fp.out[frame]);
     st.ring = reinterpret_cast<float*>(wc.stage);
     st.lane = wc.lane;
     st.edge = edge_bits(tcol, k.W);
@@ -232,7 +232,7 @@ struct EpiResize2 {
     if constexpr (MODE == RZ_RSTORE) {
       const float m = warp_max(st.mx);
       if (lane == 0 && task_ok && m > 0.f)
-        atomicMax(reinterpret_cast<unsigned int*>(&k.ws->frame_max[k.frame0 + frame]), __float_as_uint(m));
+        atomicMax(reinterpret_cast<unsigned int*>(&k.ws->frame_max[frame]), __float_as_uint(m));
     }
   }
 };

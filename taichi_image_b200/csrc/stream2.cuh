@@ -148,12 +148,12 @@ enum { K_CORE = 0, K_EDGE = 1, K_GENERAL = 2 };
 //       scaled filter sums (SiteScale2); out-of-image taps contributed the zero sample; the epilogue renormalises
 //       the frame pixels its KIND can contain (border_fix.cuh).
 
+constexpr int kBorderRows = 2;   // rows of the top / bottom border tasks (K_GENERAL)
+
 struct Stream2Geom {
-  StreamGeom g;             // rows_per_task / nchunks describe the INTERIOR rows border .. H-border-1
+  StreamGeom g;             // rows_per_task / nchunks describe the INTERIOR rows 2 .. H-3
   long long interior_tasks; // nframes * nchunks * warps_per_row
   long long total_tasks;    // + nframes * 2 * warps_per_row
-  int border;               // rows of the top / bottom border tasks (K_GENERAL): 2, or 8 for the transposing stores whose
-                            // 8-row tiles must not straddle a task
 };
 
 // rows_per_task <= 0: 24 rows per task (4 halo rows = 17 % extra loads, all L2 hits), shrunk for small jobs until
@@ -170,12 +170,10 @@ inline int auto_rows_per_task2(int H, int W, int nframes) {
   return rpt;
 }
 
-inline Stream2Geom make_geom2(int H, int W, int nframes, int rows_per_task, int border = 2) {
+inline Stream2Geom make_geom2(int H, int W, int nframes, int rows_per_task) {
   Stream2Geom s;
-  s.border = border;
   if (rows_per_task <= 0) rows_per_task = auto_rows_per_task2(H, W, nframes);
-  if (border > 2) rows_per_task = (rows_per_task + border - 1) / border * border;      // tasks start on tile boundaries
-  const int interior = H - 2 * border;
+  const int interior = H - 2 * kBorderRows;
   s.g = make_geom(interior > 0 ? interior : 0, W, nframes, rows_per_task);      // chunking of the interior rows
   s.g.H = H;
   s.interior_tasks = (interior > 0) ? s.g.total_tasks : 0;
@@ -313,15 +311,15 @@ __device__ __forceinline__ void stream2_task(const Loader& ld, const Epi& epi, c
     const long long t2 = task / g.warps_per_row;
     const int chunk = (int)(t2 % g.nchunks);
     frame = (int)(t2 / g.nchunks);
-    r0 = sg.border + chunk * g.rows_per_task;
-    rend = min(r0 + g.rows_per_task, g.H - sg.border);
+    r0 = kBorderRows + chunk * g.rows_per_task;
+    rend = min(r0 + g.rows_per_task, g.H - kBorderRows);
   } else {
     const long long t = task - sg.interior_tasks;
     strip = (int)(t % g.warps_per_row);
     const long long t2 = t / g.warps_per_row;
     frame = (int)(t2 >> 1);
-    r0 = (t2 & 1) ? g.H - sg.border : 0;
-    rend = r0 + sg.border;
+    r0 = (t2 & 1) ? g.H - kBorderRows : 0;
+    rend = r0 + kBorderRows;
   }
   const int tcol = min(strip * 32 + lane, g.ntcols - 1);   // lanes past the last column recompute it (never stored)
   if constexpr (has_gate<Epi>::value) {

@@ -33,9 +33,9 @@ class RigPipeline:
                  depth: int = 2, yuv420: bool = False, ids_format: bool = False, **tonemap_args):
         """``isp`` may resize (outputs are then the resized images) and ``yuv420=True`` selects the planar YUV 4:2:0
         output of ``process_packed12`` (1.5 instead of 3 bytes per pixel over PCIe).  The ISP's flips are applied by the sweep's
-        store, so the result still lands in the slot; the transposing transforms (rotate_90, the rig script's default) run the
-        transform kernel behind the sweep and copy into the slot, or -- opt-in, B200ISP_FUSED_TRANSPOSE=1 -- the transposing
-        store.  No transform with resize / YUV."""
+        store, so the result still lands in the slot; the transposing transforms (rotate_90, the rig script's default) are
+        applied by the normalise pass of the one-sweep Reinhard -> u8 forms, which also writes the slot, and elsewhere by the
+        transform kernel behind the sweep, whose result is copied into the slot.  No transform with resize / YUV."""
         assert width % 8 == 0 and height % 2 == 0, "fused path needs width % 8 == 0 and even height"
         base = getattr(isp, "isp", isp)
         tname = base.transform.value

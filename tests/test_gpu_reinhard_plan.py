@@ -5,8 +5,8 @@ scratch of exactly that size inside guard bands.
 * exact size: nothing outside the scratch changes, every frame's map is written, and the outputs equal those of the same
   call with a generous scratch;
 * one byte less: the map forms leave the scratch alone and run the exact form (Camera32: the outputs of the
-  ``reinhard_exact=True`` ISP); YUV 4:2:0 and resizing ISPs refuse the call (E_ARG); the Camera16 table pass falls back to the
-  arithmetic pass, which is bit-identical, and leaves the tables alone.
+  ``reinhard_exact=True`` ISP); YUV 4:2:0, resizing ISPs and the transposing transforms refuse the call (E_ARG); the Camera16
+  table pass falls back to the arithmetic pass, which is bit-identical, and leaves the tables alone.
 """
 import pytest
 import torch
@@ -24,12 +24,12 @@ E_ARG = -1
 CASES = {
     "resize_cam16": ("Camera16", "u8", 0.6, dict(scale=0.5), False, True),
     "resize_cam32": ("Camera32", "u16", 0.9, dict(scale=0.5), False, True),
-    "cam16_turned": ("Camera16", "u8", 0.6, dict(transform="rotate_90"), False, False),
+    "cam16_turned_no_fallback": ("Camera16", "u8", 0.6, dict(transform="rotate_90"), False, True),
     "cam16_yuv": ("Camera16", "u8", 0.6, {}, True, True),
     "cam16_table": ("Camera16", "u8", 0.6, {}, False, False),
     "cam16_arith": ("Camera16", "u16", 0.6, {}, False, False),
     "cam32_map16": ("Camera32", "u8", 0.9, {}, False, False),
-    "cam32_turned": ("Camera32", "u8", 0.9, dict(transform="rotate_90"), False, False),
+    "cam32_turned_no_fallback": ("Camera32", "u8", 0.9, dict(transform="rotate_90"), False, True),
 }
 
 
@@ -96,6 +96,7 @@ def test_reported_scratch_size_is_exactly_what_the_call_uses(cuda, case):
     rc = _call(isp, p, frames, less, metrics, buf[PAD:PAD + need - 1])
     if refused:
         assert rc == E_ARG, rc
+        assert bool((buf == CANARY).all()), "a refused call wrote to the scratch"
         return
     _lib.check(rc, case)
     if "table" in case:                                   # the maps are written, the tables are not; same outputs

@@ -11,7 +11,7 @@ from oracle import isp_oracle as O
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
-def test_library_loads_exports_every_declared_symbol_and_reports_abi_102():
+def test_library_loads_exports_every_declared_symbol_and_reports_abi_103():
     from taichi_image_b200 import _lib
     header = open(os.path.join(ROOT, "include", "b200isp.h")).read()
     declared = set(re.findall(r"\b(b200isp_[a-z0-9_]+)\s*\(", header))
@@ -21,7 +21,7 @@ def test_library_loads_exports_every_declared_symbol_and_reports_abi_102():
     for name in sorted(declared):
         assert hasattr(lib, name), f"{name} declared in include/b200isp.h but not exported"
     assert declared == set(_lib.EXPORTS), declared ^ set(_lib.EXPORTS)
-    assert _lib.lib.b200isp_version() == 102
+    assert _lib.lib.b200isp_version() == 103
     assert _lib.WORKSPACE_BYTES >= 4096
 
 
@@ -175,6 +175,26 @@ def test_c_abi_rejects_bad_arguments_without_touching_the_gpu():
     p.isp_dtype, p.gamma = 4, 0.0
     ptrs16 = (C.c_void_p * 1)(0x1000)
     assert lib.b200isp_process_packed12(ptrs16, ptrs16, 1, p, dummy, dummy, None) == E_ARG          # gamma must be positive
+    # transposing transforms (flip 4..7) only where the normalise pass of a one-sweep Reinhard -> u8 form turns the image
+    from taichi_image_b200 import dtypes
+    h, w = 32, 64
+    f16, f32, u8, u16 = (d.code for d in (dtypes.f16, dtypes.f32, dtypes.u8, dtypes.u16))
+    pitched = 3 * h + 48                                 # elements per row of the (W, H) output, a multiple of 16 bytes
+    for isp, what, fields in ((f16, "linear", dict(tonemap=0, gamma=1.0)), (f32, "linear", dict(tonemap=0, gamma=1.0)),
+                              (f16, "RGB16 Reinhard", dict(out_dtype=u16)), (f32, "RGB16 Reinhard", dict(out_dtype=u16)),
+                              (f16, "IDS Reinhard", dict(ids_layout=1)), (f32, "IDS Reinhard", dict(ids_layout=1)),
+                              (f32, "pitched Reinhard, gamma > 1", dict(out_pitch=pitched, gamma=1.2)),
+                              (f32, "pitched Reinhard, color_adapt", dict(out_pitch=pitched, color_adapt=0.5))):
+        for flip in range(4, 8):
+            q = _lib.FusedParams()
+            q.height, q.width, q.isp_dtype, q.out_dtype, q.tonemap, q.gamma, q.flip = h, w, isp, u8, 1, 0.9, flip
+            for name, value in fields.items():
+                setattr(q, name, value)
+            assert lib.b200isp_process_packed12(ptrs, ptrs, 1, q, dummy, dummy, None) == E_ARG, (isp, what, flip)
+            assert b"transposing" in lib.b200isp_last_error()
+            assert lib.b200isp_reinhard_scratch_bytes(q, 1) == 0
+            q.out_dtype, q.tonemap, q.gamma, q.color_adapt, q.ids_layout = u8, 1, 0.9, 0.0, 0
+            assert lib.b200isp_reinhard_scratch_bytes(q, 1) > 0, (isp, what, flip)     # Reinhard -> u8: a turned form
     assert lib.b200isp_mailbox_bytes(0) == 0 and lib.b200isp_mailbox_bytes(8) > 0
     assert lib.b200isp_mailbox_exchange(dummy, 3, ptrs, 1, 0, dummy, None) == E_ARG                  # kind must be 1 | 2
     assert lib.b200isp_sample_histogram(dummy, 10, 0, dummy, None) == E_ARG
@@ -183,7 +203,7 @@ def test_c_abi_rejects_bad_arguments_without_touching_the_gpu():
 
 
 
-def test_fused_call_routes_transforms_without_routing_switches(monkeypatch):
+def test_fused_call_turns_images_only_in_the_one_sweep_reinhard_forms(monkeypatch):
     """host logic of ISP._fused_flip (no GPU): which ISP transforms the fused call applies itself -- flips in the sweep's
     store on every path, transposing transforms (interpolate.py:36-56) in the normalise pass of the one-sweep Reinhard -> u8
     forms only; everything else returns 0 = the transform kernel runs behind the call"""
@@ -191,8 +211,7 @@ def test_fused_call_routes_transforms_without_routing_switches(monkeypatch):
     from taichi_image_b200 import camera_isp, bayer
     from taichi_image_b200.dtypes import u8, u16, f16
     from taichi_image_b200.interpolate import ImageTransform as T
-    for var in ("B200ISP_FUSED_TRANSPOSE", "B200ISP_REINHARD_EXACT"):
-        monkeypatch.delenv(var, raising=False)
+    monkeypatch.delenv("B200ISP_REINHARD_EXACT", raising=False)
     cpu = torch.device("cpu")
     codes = {T.flip_horiz: 1, T.flip_vert: 2, T.rotate_180: 3, T.transpose: 4, T.rotate_270: 5, T.rotate_90: 6, T.transverse: 7}
     for cam in (camera_isp.Camera16, camera_isp.Camera32):
@@ -212,8 +231,6 @@ def test_fused_call_routes_transforms_without_routing_switches(monkeypatch):
     assert isp._fused_flip(3000, "reinhard", u8, 1.2, 0.0) == 0 and isp._fused_flip(3000, "reinhard", u8, 0.9, 0.5) == 0
     assert camera_isp.Camera32(bayer.BayerPattern.RGGB, transform=T.rotate_90, reinhard_exact=True, device=cpu)._fused_flip(3000, "reinhard", u8, 0.9, 0.0) == 0
     assert camera_isp.Camera16(bayer.BayerPattern.RGGB, transform=T.rotate_90, device=cpu)._fused_flip(3000, "reinhard", u8, 1.2, 0.5) == 6
-    monkeypatch.setenv("B200ISP_FUSED_TRANSPOSE", "1")                                               # the sweep's own transposing store (opt-in)
-    assert isp._fused_flip(3000, "linear", u16, 1.0, 0.0) == 6
 
 
 def _expected_reinhard_scratch(isp, out, tonemap, gamma, ca, mode, flip, yuv, ids, pitched, resize, n, h, w, ho, wo):
