@@ -35,7 +35,7 @@ FUSED_OUT = {"u8": "uint8_t", "u16": "uint16_t", "f16": "__half", "f32": "float"
 
 def translation_units():
     """(object name, source, extra defines)"""
-    tus = [(n, CSRC / f"{n}.cu", []) for n in ("api", "pack", "demosaic", "tonemap", "resize", "fused_api", "fused_resize", "reinhard_gated", "exchange", "yuv420")]
+    tus = [(n, CSRC / f"{n}.cu", []) for n in ("api", "pack", "demosaic", "tonemap", "resize", "fused_api", "fused_resize", "normalise", "exchange", "yuv420")]
     for name, ctype in (("u8", "uint8_t"), ("u16", "uint16_t"), ("i16", "int16_t"), ("f16", "__half"), ("f32", "float")):
         tus.append((f"demosaic_{name}", CSRC / "demosaic_inst.cu", [f"-DISP_PLANE_T={ctype}"]))
     for cam in (0, 1):
@@ -48,6 +48,7 @@ def translation_units():
                 continue
             tus.append((f"fused_cam{16 if cam else 32}_{name}", CSRC / "fused_inst.cu",
                         [f"-DISP_INST_CAM16={cam}", f"-DISP_INST_OUT={ctype}"]))
+    tus.append(("fused_gated_cam32", CSRC / "fused_inst.cu", ["-DISP_INST_CAM16=0", "-DISP_INST_GATED"]))
     return tus
 
 

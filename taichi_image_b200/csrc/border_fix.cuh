@@ -59,12 +59,6 @@ static __constant__ BorderTable c_border = border_detail::make_table();
 
 __device__ __forceinline__ int edge_class(int x, int n) { return x < 2 ? x : (x >= n - 2 ? x - n + 5 : 2); }
 
-// site kernel of bayer.py:92-97 at (row, col): slot = (row & 1) + 2 * (col & 1)
-__device__ __forceinline__ int border_site_kernel(int pattern, int row, int col) {
-  const unsigned table = pattern == 0 ? 0xE4u : (pattern == 1 ? 0x4Eu : (pattern == 2 ? 0xB1u : 0x1Bu));
-  return (table >> (2 * ((row & 1) + 2 * (col & 1)))) & 3;
-}
-
 // x = the demosaiced value of one channel normalised by 16 (what the sweep computes everywhere); returns the
 // value normalised by the in-bounds weight sum t instead.  x * 16 is exact, the IEEE division keeps the
 // Camera16 result correctly rounded (quotients of f16-valued sums by small integers hit f16 rounding ties

@@ -1,17 +1,7 @@
-// C entry point of the fused packed12 sweep + the sparse metering launch (see fused_isp.cuh), and the table form of the
-// Camera16 Reinhard normalise pass.
+// C entry points of the fused packed12 sweep and its sparse metering (see fused_isp.cuh), and run_fused: the launch sequence of
+// every ReinhardForm.
 #include "fused_isp.cuh"
 #include "resize_isp.cuh"
-
-namespace isp {
-extern template int run_fused<true, uint8_t>(const FramePtrs&, int, const b200isp_fused_params&, IspConsts, cudaStream_t);
-extern template int run_fused<true, uint16_t>(const FramePtrs&, int, const b200isp_fused_params&, IspConsts, cudaStream_t);
-extern template int run_fused<true, __half>(const FramePtrs&, int, const b200isp_fused_params&, IspConsts, cudaStream_t);
-extern template int run_fused<false, uint8_t>(const FramePtrs&, int, const b200isp_fused_params&, IspConsts, cudaStream_t);
-extern template int run_fused<false, uint16_t>(const FramePtrs&, int, const b200isp_fused_params&, IspConsts, cudaStream_t);
-extern template int run_fused<false, __half>(const FramePtrs&, int, const b200isp_fused_params&, IspConsts, cudaStream_t);
-extern template int run_fused<false, float>(const FramePtrs&, int, const b200isp_fused_params&, IspConsts, cudaStream_t);
-}  // namespace isp
 
 using namespace isp;
 
@@ -111,56 +101,6 @@ ReinhardPlan reinhard_plan(const b200isp_fused_params& p, const IspConsts& k, in
   return {ReinhardForm::kExact, 0, 0};
 }
 
-// ReinhardForm::kF16Table: the table form of the Camera16 normalise pass (see kLutBytes in fused_isp.cuh)
-__global__ void __launch_bounds__(256) reinhard_lut_build_kernel(uint8_t* lut /* n_frames x 65536 */, float gamma, const Workspace* ws) {
-  const int frame = blockIdx.y;
-  const uint32_t v = blockIdx.x * 256 + threadIdx.x;
-  const float inv_max = __fdiv_rn(1.0f, fmaxf(1e-6f, __ldcg(&ws->frame_max[frame])));
-  float q = __saturatef(__half2float(__ushort_as_half((unsigned short)v)) * inv_max);
-  if (gamma != 1.0f) q = fast_pow(q, (float)(1.0 / (double)gamma));
-  lut[(size_t)frame * kLutBytes + v] = (uint8_t)Quant<uint8_t>::q(q);
-}
-
-__global__ void __launch_bounds__(512) reinhard_lut_out_kernel(const FramePtrs scratch, const FramePtrs fp, long long n16 /* 16-value chunks per frame */,
-                                                               const uint8_t* __restrict__ lut) {
-  extern __shared__ __align__(16) uint8_t s_lut[];
-  const int frame = gridDim.y - 1 - blockIdx.y;       // last frame first: the sweep wrote it last, part of its map is still in L2
-  {
-    const uint4* g = reinterpret_cast<const uint4*>(lut + (size_t)frame * kLutBytes);
-    uint4* s4 = reinterpret_cast<uint4*>(s_lut);
-    for (int i = threadIdx.x; i < kLutBytes / 16; i += blockDim.x) s4[i] = __ldg(g + i);
-  }
-  __syncthreads();
-  const uint4* src = reinterpret_cast<const uint4*>(scratch.out[frame]);
-  uint4* dst = reinterpret_cast<uint4*>(fp.out[frame]);
-  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n16; i += (long long)gridDim.x * blockDim.x) {
-    const uint4 w0 = __ldcs(src + 2 * i), w1 = __ldcs(src + 2 * i + 1);
-    const uint32_t w[8] = {w0.x, w0.y, w0.z, w0.w, w1.x, w1.y, w1.z, w1.w};
-    uint32_t o[4];
-#pragma unroll
-    for (int j = 0; j < 4; ++j) {
-      const uint32_t a = s_lut[w[2 * j] & 0xFFFFu], b = s_lut[w[2 * j] >> 16], c = s_lut[w[2 * j + 1] & 0xFFFFu], d = s_lut[w[2 * j + 1] >> 16];
-      o[j] = a | (b << 8) | (c << 16) | (d << 24);
-    }
-    __stcs(dst + i, make_uint4(o[0], o[1], o[2], o[3]));
-  }
-}
-
-int run_lut_pass(const FramePtrs& sc, const FramePtrs& fp, int n_frames, long long n_elems, uint8_t* lut, float gamma, const Workspace* ws,
-                 cudaStream_t s) {
-  reinhard_lut_build_kernel<<<dim3(kLutBytes / 256, (unsigned)n_frames), 256, 0, s>>>(lut, gamma, ws);
-  int st = cuda_status(cudaPeekAtLastError(), "reinhard_lut_build_kernel");
-  if (st) return st;
-  static bool attr_set = false;          // per process; the attribute belongs to the function, not to a device context
-  if (!attr_set) {
-    st = cuda_status(cudaFuncSetAttribute(reinhard_lut_out_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kLutBytes), "lut smem attribute");
-    if (st) return st;
-    attr_set = true;
-  }
-  const dim3 grid((unsigned)std::min<long long>((n_elems / 16 + 511) / 512, (3 * kNumSMs + n_frames - 1) / n_frames), (unsigned)n_frames);
-  reinhard_lut_out_kernel<<<grid, 512, kLutBytes, s>>>(sc, fp, n_elems / 16, lut);
-  return cuda_status(cudaPeekAtLastError(), "reinhard_lut_out_kernel");
-}
 }  // namespace isp
 
 extern "C" size_t b200isp_reinhard_scratch_bytes(const b200isp_fused_params* params, int n_frames) {
@@ -168,6 +108,51 @@ extern "C" size_t b200isp_reinhard_scratch_bytes(const b200isp_fused_params* par
   if (!params || fused_consts("reinhard_scratch_bytes", n_frames, *params, k) || process_checks(*params, k)) return 0;
   return reinhard_plan(*params, k, n_frames).bytes;
 }
+
+namespace isp {
+// The metering kernels that do not depend on the sampler (metering.cuh), compiled here only.
+__global__ void meter_fold_bounds_kernel(const float* __restrict__ g1, int world, float alpha, const float* __restrict__ prev,
+                                         Workspace* ws) {
+  if (threadIdx.x == 0 && blockIdx.x == 0) fold_bounds(g1, world, alpha, prev, ws->bounds[0], ws->bounds[1]);
+}
+
+__global__ void meter_finalize_kernel(const float* __restrict__ g1, const float* __restrict__ g2, int world, float alpha,
+                                      const float* prev, float* metrics /* out; may alias prev */) {
+  if (threadIdx.x != 0 || blockIdx.x != 0) return;
+  float bmin, bmax;
+  fold_bounds(g1, world, alpha, prev, bmin, bmax);
+  float f[8] = {INFINITY, -INFINITY, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
+  for (int r = 0; r < world; ++r) {
+    f[0] = fminf(f[0], g2[8 * r]);
+    f[1] = fmaxf(f[1], g2[8 * r + 1]);
+    for (int k = 2; k < 8; ++k) f[k] += g2[8 * r + k];
+  }
+  const float fn = f[7];                                                  // camera_isp.py:131-134 with n = all ranks' samples
+  const float stats[9] = {bmin, bmax, f[0], f[1], __fdiv_rn(f[2], fn), __fdiv_rn(f[3], fn),
+                          __fdiv_rn(f[4], fn), __fdiv_rn(f[5], fn), __fdiv_rn(f[6], fn)};
+  for (int k = 0; k < 9; ++k) {                                           // camera_isp.py:165-166
+    const float p = prev[k];
+    metrics[k] = __fadd_rn(stats[k], __fmul_rn(alpha, __fsub_rn(p, stats[k])));
+  }
+}
+
+int launch_meter_fold_bounds(const float* g1, int world, float alpha, const float* prev, Workspace* ws, cudaStream_t s) {
+  meter_fold_bounds_kernel<<<1, 32, 0, s>>>(g1, world, alpha, prev, ws);
+  return cuda_status(cudaPeekAtLastError(), "meter_fold_bounds_kernel");
+}
+
+int launch_meter_finalize(const float* g1, const float* g2, int world, float alpha, const float* prev, float* metrics, cudaStream_t s) {
+  meter_finalize_kernel<<<1, 32, 0, s>>>(g1, g2, world, alpha, prev, metrics);
+  return cuda_status(cudaPeekAtLastError(), "meter_finalize_kernel");
+}
+
+int launch_meter_phase2_cached(int grid, const CachedSampler& smp, long long n, float alpha, const float* prev, float* metrics, Workspace* ws,
+                               cudaStream_t s, float* rec_out) {
+  meter_phase2_kernel<CachedSampler><<<grid, 256, 0, s>>>(smp, n, alpha, prev, metrics, ws, rec_out);
+  return cuda_status(cudaPeekAtLastError(), "meter_phase2_kernel");
+}
+
+}  // namespace isp
 
 // Builds the metering sampler for the packed frames (stride % 8 == 0: word-aligned fast sampler) and
 // hands it to f(sampler, n_samples, cache).
@@ -222,9 +207,7 @@ extern "C" int b200isp_meter_packed12_phase2(const uint8_t* const* packed_host, 
 extern "C" int b200isp_metering_finalize(const float* gathered1, const float* gathered2, int world, float alpha,
                                          const float* metrics_prev, float* metrics_out, b200isp_stream stream) {
   ISP_REQUIRE(gathered1 && gathered2 && metrics_prev && metrics_out && world >= 1, B200ISP_E_ARG, "metering_finalize: bad argument");
-  meter_finalize_kernel<<<1, 32, 0, (cudaStream_t)stream>>>(gathered1, gathered2, world, alpha, metrics_prev, metrics_out);
-  ISP_LAUNCH_CHECK("meter_finalize_kernel");
-  return B200ISP_OK;
+  return launch_meter_finalize(gathered1, gathered2, world, alpha, metrics_prev, metrics_out, (cudaStream_t)stream);
 }
 
 extern "C" int b200isp_meter_packed12(const uint8_t* const* packed_host, int n_frames, const b200isp_fused_params* params,
@@ -264,30 +247,24 @@ extern "C" int b200isp_meter_packed12_shared(const uint8_t* const* packed_host, 
   });
 }
 
-extern "C" int b200isp_process_packed12(const uint8_t* const* packed_host, void* const* out_host, int n_frames,
-                                        const b200isp_fused_params* params, float* metrics, void* workspace,
-                                        b200isp_stream stream) {
-  FramePtrs fp; IspConsts k;
-  ISP_REQUIRE(out_host, B200ISP_E_ARG, "process_packed12: null output list");
-  {
-    int st = fused_setup("process_packed12", packed_host, out_host, n_frames, params, metrics, workspace, fp, k);
-    if (!st) st = process_checks(*params, k);
-    if (st) return st;
-  }
-  const b200isp_fused_params& p = *params;
-  ISP_REQUIRE(p.tonemap == B200ISP_TM_NONE || metrics, B200ISP_E_ARG, "process_packed12: metrics required for tone mapping");
-  cudaStream_t s = (cudaStream_t)stream;
+// profile hooks: inside a stream capture the record must be an "external" event node to stay queryable
+static void record_profile_event(void* ev, cudaStream_t s) {
+  if (!ev) return;
+  cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
+  if (cudaStreamIsCapturing(s, &cs) == cudaSuccess && cs == cudaStreamCaptureStatusActive)
+    cudaEventRecordWithFlags((cudaEvent_t)ev, s, cudaEventRecordExternal);
+  else
+    cudaEventRecord((cudaEvent_t)ev, s);
+}
+
+// Sweep sw over fp with k: the instantiation of the call's ISP dtype (and output dtype, for the sweeps that write the output)
+static int run_sweep(Sweep sw, const FramePtrs& fp, const IspConsts& k, const b200isp_fused_params& p, int n_frames, cudaStream_t s) {
+  const int rpt = p.rows_per_task;
   const bool cam16 = p.isp_dtype == B200ISP_F16;
-
-  if (p.update_metering && p.tonemap != B200ISP_TM_NONE) {
-    const int st = with_packed12_sampler(fp, p, k, n_frames, [&](const auto& smp, long long n, float* cache) {
-      return launch_metering(smp, n, p.alpha, metrics, metrics, k.ws, s, cache);
-    });
-    if (st) return st;
-  }
-
-  if (resizes(p)) return run_resize(fp, n_frames, p, k, s);
-#define RUN(CAM, T) return run_fused<CAM, T>(fp, n_frames, p, k, s)
+  if (sw == Sweep::kMax || sw == Sweep::kStore)
+    return cam16 ? run_max_sweep<true>(sw, fp, k, n_frames, rpt, s) : run_max_sweep<false>(sw, fp, k, n_frames, rpt, s);
+  if (sw == Sweep::kMaxGated || sw == Sweep::kReinhardGated) return run_gated_sweep(sw, fp, k, n_frames, rpt, s);
+#define RUN(CAM, T) return run_out_sweep<CAM, T>(sw, fp, k, n_frames, rpt, s)
   if (cam16) {
     switch (p.out_dtype) {
       case B200ISP_U8: RUN(true, uint8_t);
@@ -307,4 +284,124 @@ extern "C" int b200isp_process_packed12(const uint8_t* const* packed_host, void*
 #undef RUN
   isp::set_error("process_packed12: unsupported isp/out dtype combination %d/%d", p.isp_dtype, p.out_dtype);
   return B200ISP_E_DTYPE;
+}
+
+// The launches of a b200isp_process_packed12 call after its metering: the Reinhard form's sequence (fused_isp.cuh) or the one
+// sweep without Reinhard.  p.profile_start / p.profile_stop bracket the pass that writes the output or the maps (the max sweep
+// of kExact and the normalise passes stay outside).
+static int run_fused(const FramePtrs& fp, int n_frames, const b200isp_fused_params& p, const IspConsts& k, cudaStream_t s) {
+  ReinhardPlan plan = reinhard_plan(p, k, n_frames);
+  if (plan.form == ReinhardForm::kResizeMap)
+    ISP_REQUIRE(p.reinhard_scratch && p.reinhard_scratch_bytes >= plan.bytes, B200ISP_E_ARG,
+                "process_packed12: Reinhard with resize needs reinhard_scratch of n_frames * out_height * out_width * 3 ISP-dtype values");
+  else if (plan.map_bytes && (!p.reinhard_scratch || p.reinhard_scratch_bytes < plan.map_bytes)) plan = {ReinhardForm::kExact, 0, 0};
+  else if (plan.form == ReinhardForm::kF16Table && p.reinhard_scratch_bytes < plan.bytes) plan.form = ReinhardForm::kF16Arith;
+  ISP_REQUIRE(!(p.out_yuv420 && plan.form == ReinhardForm::kExact), B200ISP_E_ARG,
+              "process_packed12: YUV 4:2:0 output needs Camera16 (f16), Reinhard, u8 and the reinhard_scratch buffer");
+  ISP_REQUIRE(!((k.flip & 4) && plan.form == ReinhardForm::kExact), B200ISP_E_ARG,
+              "process_packed12: the transposing transforms need the reinhard_scratch buffer (b200isp_reinhard_scratch_bytes)");
+  // The extended sweeps (IDS layout, flips in the store) are Malvar only.  The map sweeps write plain images: only the layout counts.
+  const bool one_sweep = plan.form != ReinhardForm::kNone && plan.form != ReinhardForm::kExact;
+  ISP_REQUIRE(k.kbase == 0 || !(k.ids || (k.flip && !one_sweep)), B200ISP_E_ARG, "process_packed12: the IDS layout %s fused for the Malvar demosaic only",
+              one_sweep ? "is" : "/ flips are");
+  if (plan.form != ReinhardForm::kNone) {
+    // frame_max and frame_max2 are adjacent in the workspace: one memset node
+    static_assert(offsetof(Workspace, frame_max2) == offsetof(Workspace, frame_max) + sizeof(float) * B200ISP_MAX_FRAMES, "adjacent");
+    const int st = cuda_status(cudaMemsetAsync(k.ws->frame_max, 0, sizeof(float) * 2 * B200ISP_MAX_FRAMES, s), "memset frame_max");
+    if (st) return st;
+  }
+
+  const bool cam16 = p.isp_dtype == B200ISP_F16;
+  FramePtrs sc = fp;                     // the one-sweep forms: each frame's map in the caller's scratch
+  for (int f = 0; f < n_frames; ++f) sc.out[f] = (char*)p.reinhard_scratch + (size_t)f * (plan.map_bytes / n_frames);
+  IspConsts km = k;                      // the map is a plain dense (H, W, 3) image whatever the output looks like
+  km.flip = 0;
+  km.orow = 3 * k.W;
+  IspConsts kg = k;                      // the gated exact sweeps of the u16 map forms
+  kg.gate = 1;
+  const long long n_elems = (long long)k.H * k.W * 3;
+  auto timed = [&](auto&& pass) {
+    record_profile_event(p.profile_start, s);
+    const int st = pass();
+    record_profile_event(p.profile_stop, s);
+    return st;
+  };
+  auto store = [&] { return timed([&] { return run_sweep(Sweep::kStore, sc, km, p, n_frames, s); }); };
+  int st;
+  switch (plan.form) {
+    case ReinhardForm::kNone:
+      if (resizes(p)) return timed([&] { return run_resize(fp, n_frames, p, k, s); });
+      return timed([&] { return run_sweep(p.tonemap == B200ISP_TM_NONE ? Sweep::kRgb : Sweep::kLinear, fp, k, p, n_frames, s); });
+    case ReinhardForm::kExact:
+      // max sweep, then the write sweep recomputes the map.  Both sweeps are bound by instruction issue, not by DRAM, so the
+      // second read of the packed frames (1.5 B/px) is cheaper than cutting the call into L2-sized groups whose short launches
+      // end in idle tails (measured, profiles/r02_reinhard_diet.txt).
+      if ((st = run_sweep(Sweep::kMax, fp, k, p, n_frames, s))) return st;
+      return timed([&] { return run_sweep(Sweep::kReinhard, fp, k, p, n_frames, s); });
+    case ReinhardForm::kResizeMap: {
+      if ((st = timed([&] { return run_resize(sc, n_frames, p, k, s); }))) return st;
+      const long long n_out = (long long)p.out_height * p.out_width * 3;
+      if (cam16 && n_out % 8 == 0) return run_scratch_out(sc, fp, n_frames, n_out, p.out_dtype, k.gamma, k.ws, 8 * kNumSMs, s);
+      return run_resize_normalise(sc, fp, n_frames, n_out, cam16, p.out_dtype, k.gamma, k.ws, s);
+    }
+    // Camera16: the reference stores the map as f16 anyway -> one sweep writes it to the caller's scratch, a light element-wise
+    // pass normalises it (no second sweep)
+    case ReinhardForm::kF16Turned:       // the normalise pass turns the image
+      if ((st = store())) return st;
+      return run_out_transposed(true, sc, fp, n_frames, k, s);
+    case ReinhardForm::kF16Yuv:
+      if ((st = store())) return st;
+      return run_scratch_yuv(sc, fp, n_frames, k, s);
+    case ReinhardForm::kF16Table:
+      if ((st = store())) return st;
+      return run_lut_pass(sc, fp, n_frames, n_elems, (uint8_t*)p.reinhard_scratch + plan.map_bytes, k.gamma, k.ws, s);
+    case ReinhardForm::kF16Arith:
+      if ((st = store())) return st;
+      return run_scratch_out(sc, fp, n_frames, n_elems, p.out_dtype, k.gamma, k.ws, 4 * kNumSMs, s);
+    // Camera32 -> u8, color_adapt == 0, gamma in [0.3, 1]: ONE sweep that also stores the map as u16 fixed point (6 B/px
+    // scratch) + an element-wise normalise / gamma / quantise pass.  The second demosaic of the two-sweep form (66 of its 106
+    // instructions per pixel) disappears; the u8 result is within 1 LSB of the two-sweep result (measured:
+    // profiles/r02_reinhard_map16.txt).  Frames whose map does not fit [0, 1) (reinhard_map16_declined) are redone exactly by
+    // the gated sweeps.
+    case ReinhardForm::kU16Map:
+      // the normalise pass runs after the sweep with 8 CTAs per SM; running it under the sweep on a side stream measured
+      // 212-186 vs 215 Gpixel/s on cfg3 (profiles/r02_reinhard_map16.txt)
+      if ((st = store())) return st;
+      if ((st = run_map16_out(sc, fp, n_frames, k, s))) return st;
+      if ((st = run_sweep(Sweep::kMaxGated, fp, kg, p, n_frames, s))) return st;
+      return run_sweep(Sweep::kReinhardGated, fp, kg, p, n_frames, s);
+    case ReinhardForm::kU16Turned:
+      // the gated sweeps leave the frames the map declined as plain (H, W, 3) u8 images in their scratch, then ONE pass
+      // normalises / turns every frame into the output
+      if ((st = store())) return st;
+      km.gate = 1;
+      if ((st = run_sweep(Sweep::kMaxGated, sc, km, p, n_frames, s))) return st;
+      if ((st = run_sweep(Sweep::kReinhardGated, sc, km, p, n_frames, s))) return st;
+      return run_out_transposed(false, sc, fp, n_frames, k, s);
+  }
+  return B200ISP_E_ARG;
+}
+
+extern "C" int b200isp_process_packed12(const uint8_t* const* packed_host, void* const* out_host, int n_frames,
+                                        const b200isp_fused_params* params, float* metrics, void* workspace,
+                                        b200isp_stream stream) {
+  FramePtrs fp; IspConsts k;
+  ISP_REQUIRE(out_host, B200ISP_E_ARG, "process_packed12: null output list");
+  {
+    int st = fused_setup("process_packed12", packed_host, out_host, n_frames, params, metrics, workspace, fp, k);
+    if (!st) st = process_checks(*params, k);
+    if (st) return st;
+  }
+  const b200isp_fused_params& p = *params;
+  ISP_REQUIRE(p.tonemap == B200ISP_TM_NONE || metrics, B200ISP_E_ARG, "process_packed12: metrics required for tone mapping");
+  cudaStream_t s = (cudaStream_t)stream;
+
+  if (p.update_metering && p.tonemap != B200ISP_TM_NONE) {
+    const int st = with_packed12_sampler(fp, p, k, n_frames, [&](const auto& smp, long long n, float* cache) {
+      return launch_metering(smp, n, p.alpha, metrics, metrics, k.ws, s, cache);
+    });
+    if (st) return st;
+  }
+
+  return run_fused(fp, n_frames, p, k, s);
 }

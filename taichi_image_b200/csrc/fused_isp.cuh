@@ -8,20 +8,24 @@
 // the demosaiced RGB and the Reinhard intermediate through f16; Camera32 keeps f32.
 //
 // Launch plan per call (all on one stream, no host sync; the 2-pixel image frame is renormalised INSIDE the sweep,
-// border_fix.cuh -- there is no border kernel):
+// border_fix.cuh -- there is no border kernel).  run_fused (fused_api.cu) issues it, one case per ReinhardForm (below); the
+// sweeps are launched by fused_inst.cu, the normalise passes live in normalise.cu:
 //   [metering]  meter_fused_kernel (one cooperative launch) or meter_phase1 -> meter_phase2; sampler straight from the packed bytes
 //   linear      stream2<EpiLinear2>                          one sweep
-//   reinhard    Camera32: stream2<EpiReinhardMax2> (frame-global max of the mapped values) -> stream2<EpiReinhard2>
+//   reinhard    kExact: stream2<EpiReinhardMax2> (frame-global max of the mapped values) -> stream2<EpiReinhard2>
 //                         (the write sweep recomputes the map), one pair of launches for all frames of the call
-//               Camera32 -> u8 (color_adapt 0, gamma 0.3 .. 1): stream2<EpiReinhardMax2, STORE> (u16 fixed-point map)
-//                         -> reinhard_map16_out_kernel (normalise / gamma / quantise) -> the two gated exact sweeps
+//               kU16Map (Camera32 -> u8, color_adapt 0, gamma 0.3 .. 1): stream2<EpiReinhardMax2, STORE> (u16 fixed-point
+//                         map) -> reinhard_map16_out_kernel (normalise / gamma / quantise) -> the two gated exact sweeps
 //                         (they leave at once unless the map declined a frame)
-//               Camera16: stream2<EpiReinhardMax2, STORE> (writes the f16 map the reference stores back anyway)
-//                         -> reinhard_scratch_out_kernel (element-wise normalise / gamma / quantise)
-//               either one-sweep form -> u8 with a transposing ISP transform: the pass is reinhard_out_transposed_kernel
-//                         (same arithmetic, the image turned through a shared-memory tile; Camera32: after the gated sweeps)
+//               kF16*: stream2<EpiReinhardMax2, STORE> (writes the f16 map the reference stores back anyway)
+//                         -> reinhard_scratch_out_kernel (element-wise normalise / gamma / quantise), the table pass (u8,
+//                         gamma != 1) or reinhard_scratch_yuv_kernel (YUV 4:2:0)
+//               kF16Turned / kU16Turned (either one-sweep form -> u8 with a transposing ISP transform): the pass is
+//                         reinhard_out_transposed_kernel (same arithmetic, the image turned through a shared-memory tile;
+//                         Camera32: after the gated sweeps)
 //   none        stream2<EpiRgb2>                             load_packed12 only: float RGB out
-//   resizing ISP: csrc/resize_sweep.cuh (stream2_resize_kernel + orphan columns [+ normalise pass])
+//   resizing ISP: fused_resize.cu (stream2_resize_kernel + orphan columns [-> resize_normalise_kernel or
+//                         reinhard_scratch_out_kernel: kResizeMap])
 #pragma once
 #include <algorithm>
 #include "stream2.cuh"
@@ -39,21 +43,17 @@ struct FramePtrs {
   void* out[B200ISP_MAX_FRAMES];
 };
 
-// ---------------------------------------------------------------- packed12 row loader (standard layout)
-// Thread column tcol owns pixels 8*tcol..8*tcol+7 = bytes 12*tcol..12*tcol+11 = words 3*tcol..3*tcol+2;
-// the halo pixels live in the top 3 bytes of word 3*tcol-1 and the low 3 bytes of word 3*tcol+3.
-// Camera32: samples are decoded as b = 1 + v/4096 (12 bits dropped into the mantissa of 1.0f: one
-// shift + one LOP3 per pixel, no int->float conversion).  All filter weights sum to 16, so the sums
-// come out as 16 + S/4096 exactly and the bias folds into the epilogue's FMA.
-// Camera16: the reference stores cfa = f16(v * f32(1/4095)); the same value is produced with one FMA
-// (exact product, single rounding) and a packed f32->f16->f32 round trip.
-// (biased_from_shifted: common.cuh)
-
 // ---------------------------------------------------------------- packed12 row loader of the pair engine (stream2.cuh)
-// Same words and the same one-LOP3 decode as Packed12Loader, but: the decode mask is a register (0 for rows
-// outside the image and for the halo columns of the first / last thread column -> "zero sample"), the halo
-// loads are predicated on per-thread constants instead of being zero-filled, and the row is delivered as the
-// eight pairs (v[k], v[k+4]).
+// Thread column tcol owns pixels 8*tcol..8*tcol+7 = bytes 12*tcol..12*tcol+11 = words 3*tcol..3*tcol+2; the halo pixels
+// live in the top 3 bytes of word 3*tcol-1 and the low 3 bytes of word 3*tcol+3.  The decode mask is a register (0 for rows
+// outside the image and for the halo columns of the first / last thread column -> "zero sample"), the halo loads are
+// predicated on per-thread constants, and the row is delivered as the eight pairs (v[k], v[k+4]).
+// Camera32: samples are decoded as b = 1 + v/4096 (12 bits dropped into the mantissa of 1.0f: one shift + one LOP3 per
+// pixel, no int->float conversion).  All filter weights sum to 16, so the sums come out as 16 + S/4096 exactly and the bias
+// folds into the epilogue's FMA.
+// Camera16: the reference stores cfa = f16(v * f32(1/4095)); the same value is produced with one FMA (exact product,
+// single rounding) and a packed f32->f16->f32 round trip.
+// (biased_from_shifted: common.cuh)
 // IDS layout (packed.py:36-44): a pixel pair is the bytes (b0, b1, b2) with p0 = b0 << 4 | (b2 & 0xF), p1 = b1 << 4 | b2 >> 4,
 // so a sample's twelve bits are a byte plus a nibble from another byte.  Given the two shifted copies of the word(s) that
 // bring the byte to mantissa bits 15..22 (a) and the nibble to bits 11..14 (b), the biased sample 1 + v/4096 is two LOP3:
@@ -316,15 +316,6 @@ __device__ __forceinline__ void store_out(const WarpCtx& wc, OutT* warp_out /* f
   warp_store_row<NW, false>(wc, base + (size_t)((unsigned)orow_idx * (unsigned)k.orow), w, wc.lane < wc.nvalid ? wc.nvalid - 1 - wc.lane : wc.lane);
 }
 
-template <typename OutT> __device__ __forceinline__ void store_px(void* frame_out, int W, int row, int col, const float (&y)[3]) {
-  OutT* dst = reinterpret_cast<OutT*>(frame_out) + ((size_t)row * W + col) * 3;
-#pragma unroll
-  for (int k = 0; k < 3; ++k) {
-    if constexpr (DT<OutT>::is_int) dst[k] = (OutT)(Quant<OutT>::q(y[k]) & (uint32_t)DT<OutT>::scale);
-    else dst[k] = cast_from_f32<OutT>(y[k]);
-  }
-}
-
 // ---------------------------------------------------------------- tone-map stages (per pixel, shared by hot + border)
 struct LinearConsts { float a, bmin, inv_gamma; int has_gamma; };
 
@@ -360,13 +351,6 @@ __device__ __forceinline__ void reinhard_p(const ReinhardConsts& c, const float 
 #pragma unroll
   for (int k = 0; k < 3; ++k) s[k] = fmaf(rgb[k], c.p.inv_range, c.b);
   reinhard_map_fast<CA0>(c.p, s, p);
-}
-
-// run-time colour-adapt switch (kernel-uniform) for the pair-engine epilogues
-template <bool CAM16>
-__device__ __forceinline__ void reinhard_p_rt(const ReinhardConsts& c, const float (&rgb)[3], float (&p)[3]) {
-  if (c.ca0) reinhard_p<CAM16, true>(c, rgb, p);
-  else reinhard_p<CAM16, false>(c, rgb, p);
 }
 
 // camera_isp.py:211-218: stored = cast_T(p); out = trunc(scale * (stored / max_out)^(1/gamma))
@@ -1032,8 +1016,6 @@ struct EpiReinhard2 {         // pass 2 recomputed from the packed frame: map, n
   }
 };
 
-enum { MODE_RGB = 0, MODE_LINEAR = 1, MODE_RMAX = 2, MODE_REINHARD = 3 };
-
 // ---------------------------------------------------------------- metering samplers straight from packed12
 // generic: any stride, literal per-pixel demosaic
 template <bool CAM16>
@@ -1230,406 +1212,22 @@ struct Packed12FastSampler {
   }
 };
 
-// ---------------------------------------------------------------- host orchestration
-// profile hooks: inside a stream capture the record must be an "external" event node to stay queryable
-static inline void record_profile_event(void* ev, cudaStream_t s) {
-  cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
-  if (cudaStreamIsCapturing(s, &cs) == cudaSuccess && cs == cudaStreamCaptureStatusActive)
-    cudaEventRecordWithFlags((cudaEvent_t)ev, s, cudaEventRecordExternal);
-  else
-    cudaEventRecord((cudaEvent_t)ev, s);
-}
-
-// host dispatch of the Reinhard write sweep on (color_adapt == 0, gamma != 1)
-template <int P, bool CAM16, typename OutT, bool EXT>
-static int launch_reinhard(const Packed12Loader2<CAM16, EXT>& ld, const FramePtrs& fp, const IspConsts& k, const Stream2Geom& g, cudaStream_t s) {
-  const bool ca0 = k.ca == 0.f, gam = k.gamma != 1.0f, bl = !EXT && k.kbase != 0;
-  if (ca0 && gam) { EpiReinhard2<CAM16, OutT, true, true, EXT> e{fp, k}; return launch_stream2<P>(ld, e, g, s, "isp_stream<reinhard>", bl); }
-  if (ca0) { EpiReinhard2<CAM16, OutT, true, false, EXT> e{fp, k}; return launch_stream2<P>(ld, e, g, s, "isp_stream<reinhard>", bl); }
-  if (gam) { EpiReinhard2<CAM16, OutT, false, true, EXT> e{fp, k}; return launch_stream2<P>(ld, e, g, s, "isp_stream<reinhard>", bl); }
-  EpiReinhard2<CAM16, OutT, false, false, EXT> e{fp, k};
-  return launch_stream2<P>(ld, e, g, s, "isp_stream<reinhard>", bl);
-}
-
-// EXT: the extended kernels (IDS layout in the row loader, flips in the store); Malvar only -- the host mirror routes
-// bilinear + IDS / flip through the re-pack pass / the transform kernel.
-template <bool CAM16, int MODE, typename OutT, bool EXT>
-static int run_pass_ext(const FramePtrs& fp, IspConsts k, int nframes, int rows_per_task, cudaStream_t s, void* ev_start, void* ev_stop) {
-  const Stream2Geom g = make_geom2(k.H, k.W, nframes, rows_per_task);
-  const bool bl = !EXT && k.kbase != 0;
-  if (EXT && k.kbase != 0) { set_error("process_packed12: the IDS layout / flips are fused for the Malvar demosaic only"); return B200ISP_E_ARG; }
-  Packed12Loader2<CAM16, EXT> ld;
-  ld.fp = fp; ld.pitch_words = k.W * 3 / 8; ld.ids = k.ids;
-  int st = B200ISP_OK;
-  auto record = [&](void* ev) { record_profile_event(ev, s); };
-  if (ev_start) record(ev_start);
-  ISP_DISPATCH_PATTERN(k.pattern, P, {
-    if constexpr (MODE == MODE_RGB) { EpiRgb2<CAM16, OutT, EXT> e{fp, k}; st = launch_stream2<P>(ld, e, g, s, "isp_stream<rgb>", bl); }
-    else if constexpr (MODE == MODE_LINEAR) {
-      bool fast = false;
-      if constexpr (!CAM16) fast = !k.ccm && k.gamma == 1.0f;
-      if constexpr (!CAM16) { if (fast) { EpiLinear2<false, OutT, true, EXT> e{fp, k}; st = launch_stream2<P>(ld, e, g, s, "isp_stream<linear,fast>", bl); } }
-      if (!fast) { EpiLinear2<CAM16, OutT, false, EXT> e{fp, k}; st = launch_stream2<P>(ld, e, g, s, "isp_stream<linear>", bl); }
-    }
-    else if constexpr (MODE == MODE_RMAX) {
-      if (k.ca == 0.f) { EpiReinhardMax2<CAM16, true> e{fp, k}; st = launch_stream2<P>(ld, e, g, s, "isp_stream<reinhard_max>", bl); }
-      else { EpiReinhardMax2<CAM16, false> e{fp, k}; st = launch_stream2<P>(ld, e, g, s, "isp_stream<reinhard_max>", bl); }
-    } else {
-      st = launch_reinhard<P, CAM16, OutT, EXT>(ld, fp, k, g, s);
-    }
-  });
-  if (ev_stop) record(ev_stop);
-  return st;     // the 2-pixel image frame is renormalised inside the sweep (border_fix.cuh): no border kernel
-}
-
-template <bool CAM16, int MODE, typename OutT>
-static int run_pass(const FramePtrs& fp, IspConsts k, int nframes, int rows_per_task, cudaStream_t s,
-                    void* ev_start = nullptr, void* ev_stop = nullptr) {
-  // the max sweep stores nothing: it only needs the extended loader for IDS frames
-  const bool ext = k.ids != 0 || (MODE != MODE_RMAX && k.flip != 0);
-  if (ext) return run_pass_ext<CAM16, MODE, OutT, true>(fp, k, nframes, rows_per_task, s, ev_start, ev_stop);
-  return run_pass_ext<CAM16, MODE, OutT, false>(fp, k, nframes, rows_per_task, s, ev_start, ev_stop);
-}
-
-// ---------------------------------------------------------------- Camera16 Reinhard in ONE sweep + a light second pass
-// pass A: the max sweep with STORE over all frames (scratch = f16 map); pass B: out = quantise((p / max)^(1/gamma))
-// element-wise on the scratch, all frames in one launch (blockIdx.y = frame).
-template <typename OutT>
-__global__ void __launch_bounds__(256) reinhard_scratch_out_kernel(const FramePtrs scratch /* .out = f16 maps */, const FramePtrs fp,
-                                                                   long long n_elems /* per frame, % 8 == 0 */, float gamma, const Workspace* ws) {
-  const int frame = gridDim.y - 1 - blockIdx.y;       // last frame first: the sweep wrote it last, part of its map is still in L2
-  const __half* src = reinterpret_cast<const __half*>(scratch.out[frame]);
-  OutT* dst = reinterpret_cast<OutT*>(fp.out[frame]);
-  const float inv_max = __fdiv_rn(1.0f, fmaxf(1e-6f, __ldcg(&ws->frame_max[frame])));
-  const float inv_gamma = (float)(1.0 / (double)gamma);
-  const bool has_gamma = gamma != 1.0f;
-  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n_elems / 8; i += (long long)gridDim.x * blockDim.x) {
-    const uint4 w = __ldcs(reinterpret_cast<const uint4*>(src) + i);
-    const __half* t = reinterpret_cast<const __half*>(&w);
-    uint32_t v[8];
-#pragma unroll
-    for (int j = 0; j < 8; ++j) {
-      float q = __saturatef(__half2float(t[j]) * inv_max);
-      if (has_gamma) q = fast_pow(q, inv_gamma);
-      v[j] = Quant<OutT>::q(q);
-    }
-    if constexpr (std::is_same<OutT, uint8_t>::value) {
-      uint2 o;
-      o.x = __byte_perm(__byte_perm(v[0], v[1], 0x0040), __byte_perm(v[2], v[3], 0x0040), 0x5410);
-      o.y = __byte_perm(__byte_perm(v[4], v[5], 0x0040), __byte_perm(v[6], v[7], 0x0040), 0x5410);
-      __stcs(reinterpret_cast<uint2*>(dst) + i, o);
-    } else if constexpr (std::is_same<OutT, uint16_t>::value) {
-      uint4 o = make_uint4(__byte_perm(v[0], v[1], 0x5410), __byte_perm(v[2], v[3], 0x5410), __byte_perm(v[4], v[5], 0x5410),
-                           __byte_perm(v[6], v[7], 0x5410));
-      __stcs(reinterpret_cast<uint4*>(dst) + i, o);
-    } else {
-      alignas(16) __half o[8];
-#pragma unroll
-      for (int j = 0; j < 8; ++j) o[j] = __float2half_rn(__uint_as_float(v[j]));
-      __stcs(reinterpret_cast<uint4*>(dst) + i, *reinterpret_cast<const uint4*>(o));
-    }
-  }
-}
-
-// pass B of the one-sweep Camera32 Reinhard -> u8 path: out = trunc(255 * ((v + 0.5) / 65535 / max)^(1/gamma)) for the u16
-// map v of EpiReinhardMax2<false, CA0, STORE>; frames the map declined are skipped (the gated sweeps write them).
-// u16 -> f32 by dropping the halves into the mantissa of 2^23 (PRMT) and one exact packed subtraction -- no conversion
-// instruction, packed arithmetic throughout.  Dense outputs: 16 values per thread and iteration (two 16-byte loads, one
-// 16-byte store); PITCHED (the outputs are tiles of a grid image, orow > 3 W): 8 values, row / column from the chunk index.
-__device__ __forceinline__ void map16_pair(uint32_t w, f2 a2, f2 h2, f2 ig2, bool gamma, uint32_t& v0, uint32_t& v1) {
-  const f2 t = add2(pk(__uint_as_float(__byte_perm(w, 0x4B000000u, 0x7610)), __uint_as_float(__byte_perm(w, 0x4B000000u, 0x7632))),
-                    bc(-8388608.f));
-  f2 q = fma2(t, a2, h2);
-  if (gamma) {
-    float lo, hi, l0, l1;
-    upk(q, lo, hi);
-    asm("lg2.approx.ftz.f32 %0, %1;" : "=f"(l0) : "f"(lo));
-    asm("lg2.approx.ftz.f32 %0, %1;" : "=f"(l1) : "f"(hi));
-    upk(mul2(pk(l0, l1), ig2), lo, hi);
-    asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(l0) : "f"(lo));
-    asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(l1) : "f"(hi));
-    q = pk(l0, l1);
-  }
-  float ql, qh;
-  upk(fma2_rz(q, bc(255.f), bc(8388608.f)), ql, qh);
-  v0 = __float_as_uint(ql);
-  v1 = __float_as_uint(qh);
-}
-__device__ __forceinline__ uint32_t pack4_u8(uint32_t a, uint32_t b, uint32_t c, uint32_t d) {
-  return __byte_perm(__byte_perm(a, b, 0x0040), __byte_perm(c, d, 0x0040), 0x5410);
-}
-
-template <bool GAMMA, bool PITCHED>
-__global__ void __launch_bounds__(256) reinhard_map16_out_kernel(const FramePtrs scratch /* .out = u16 maps */, const FramePtrs fp,
-                                                                 int H, int W, int orow, float gamma, const Workspace* ws) {
-  const int frame = gridDim.y - 1 - blockIdx.y;       // last frame first: the sweep wrote it last, part of its map is still in L2
-  const float mx = __ldcg(&ws->frame_max[frame]);
-  if (reinhard_map16_declined(mx)) return;
-  const uint4* src = reinterpret_cast<const uint4*>(scratch.out[frame]);
-  const float a = __fdiv_rn(__fdiv_rn(1.0f, mx), kMap16Scale);
-  const f2 a2 = bc(a), h2 = bc(0.5f * a), ig2 = bc((float)(1.0 / (double)gamma));
-  const long long stride = (long long)gridDim.x * blockDim.x;
-  if constexpr (!PITCHED) {
-    // two 16-value chunks per iteration, the four 16-byte loads issued before the first use.  Measured on cfg3 (gamma 0.9):
-    // 8 CTAs per SM 131 us, 4: 155 us, 2: slower still -- unlike a plain copy this pass wants every thread slot
-    // (profiles/r02_reinhard_map16.txt)
-    uint4* dst = reinterpret_cast<uint4*>(fp.out[frame]);
-    const long long n16 = (long long)H * W * 3 / 16;                   // H even, W % 8 == 0
-    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n16; i += 2 * stride) {
-      const long long i2 = i + stride;
-      const bool two = i2 < n16;
-      const uint4 w0 = __ldcs(src + 2 * i), w1 = __ldcs(src + 2 * i + 1);
-      uint4 w2 = w0, w3 = w1;
-      if (two) { w2 = __ldcs(src + 2 * i2); w3 = __ldcs(src + 2 * i2 + 1); }
-      {
-        const uint32_t w[8] = {w0.x, w0.y, w0.z, w0.w, w1.x, w1.y, w1.z, w1.w};
-        uint32_t v[16];
-#pragma unroll
-        for (int j = 0; j < 8; ++j) map16_pair(w[j], a2, h2, ig2, GAMMA, v[2 * j], v[2 * j + 1]);
-        __stcs(dst + i, make_uint4(pack4_u8(v[0], v[1], v[2], v[3]), pack4_u8(v[4], v[5], v[6], v[7]), pack4_u8(v[8], v[9], v[10], v[11]),
-                                   pack4_u8(v[12], v[13], v[14], v[15])));
-      }
-      if (two) {
-        const uint32_t w[8] = {w2.x, w2.y, w2.z, w2.w, w3.x, w3.y, w3.z, w3.w};
-        uint32_t v[16];
-#pragma unroll
-        for (int j = 0; j < 8; ++j) map16_pair(w[j], a2, h2, ig2, GAMMA, v[2 * j], v[2 * j + 1]);
-        __stcs(dst + i2, make_uint4(pack4_u8(v[0], v[1], v[2], v[3]), pack4_u8(v[4], v[5], v[6], v[7]), pack4_u8(v[8], v[9], v[10], v[11]),
-                                    pack4_u8(v[12], v[13], v[14], v[15])));
-      }
-    }
-  } else {
-    uint8_t* dst = reinterpret_cast<uint8_t*>(fp.out[frame]);
-    const int cpr = W * 3 / 8;                                         // 8-value chunks per row
-    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < (long long)H * cpr; i += stride) {
-      const int row = (int)(i / cpr), c = (int)(i - (long long)row * cpr);
-      const uint4 w0 = __ldcs(src + i);
-      const uint32_t w[4] = {w0.x, w0.y, w0.z, w0.w};
-      uint32_t v[8];
-#pragma unroll
-      for (int j = 0; j < 4; ++j) map16_pair(w[j], a2, h2, ig2, GAMMA, v[2 * j], v[2 * j + 1]);
-      __stcs(reinterpret_cast<uint2*>(dst + (size_t)row * orow + 8 * c), make_uint2(pack4_u8(v[0], v[1], v[2], v[3]), pack4_u8(v[4], v[5], v[6], v[7])));
-    }
-  }
-}
-
-// pass B through a table (Camera16, gamma != 1, dense u8 outputs): the f16 map has only 65 536 patterns, and the output is a
-// pure function of the pattern and the frame maximum.  reinhard_lut_build_kernel evaluates that function once per pattern and
-// frame with exactly the arithmetic of reinhard_scratch_out_kernel (so the result is bit-identical to it); reinhard_lut_out_kernel
-// keeps the frame's 64 KB table in shared memory and turns every value into one LDS.U8: no MUFU (the arithmetic pass needs 6 per
-// pixel and sits at 74 % of the MUFU pipe), 10 instead of 21 instructions per pixel -- the pass becomes a plain HBM stream.
-// Camera32 has no table form: its pass (reinhard_map16_out_kernel) is bound by its 2 : 1 read / write DRAM stream (4.75 TB/s),
-// not by the MUFU pipe, and the table form measured 134.9 vs 131.5 us on cfg3.
-constexpr int kLutBytes = 65536;
-// the table form of pass B (defined in fused_api.cu); lut = n_frames x 64 KB behind the maps in the caller's scratch
-int run_lut_pass(const FramePtrs& sc, const FramePtrs& fp, int n_frames, long long n_elems, uint8_t* lut, float gamma, const Workspace* ws,
-                 cudaStream_t s);
-
-// pass B with planar YUV 4:2:0 output (SURVEY 8f-2, for video encoders): the u8 RGB of reinhard_scratch_out_kernel
-// is formed in registers and converted with the arithmetic of color/yuv_420.py:47-64 (csrc/yuv420.cu: x / 255, the
-// BT.601 matrix applied to the BGR-swizzled pixel, chroma = mean of the 2x2 quad, one-sided clamp) -- bit-identical
-// to rgb_yuv420_image(process_packed12(...)) without writing or re-reading the RGB image: 1.5 B/px out instead of 3.
-// Thread = 8 pixel columns x 2 rows (four quads); out = (3H/2, W) u8: H rows of Y, then chroma plane 0 (third
-// matrix row) and plane 1 (second matrix row).
-static __global__ void __launch_bounds__(128) reinhard_scratch_yuv_kernel(const FramePtrs scratch, const FramePtrs fp, int H, int W, float gamma,
-                                                                   const Workspace* ws) {
-  // x / 255 (correctly rounded, yuv_420.py:50) for the 256 possible inputs: a table instead of three IEEE divisions per pixel
-  __shared__ float unit[256];
-  for (int i = threadIdx.x; i < 256; i += blockDim.x) unit[i] = __fdiv_rn((float)i, 255.0f);
-  __syncthreads();
-  const int gx = blockIdx.x * blockDim.x + threadIdx.x, qy = blockIdx.y, frame = blockIdx.z;
-  if (gx >= W / 8) return;
-  const __half* src = reinterpret_cast<const __half*>(scratch.out[frame]);
-  uint8_t* yuv = reinterpret_cast<uint8_t*>(fp.out[frame]);
-  const float inv_max = __fdiv_rn(1.0f, fmaxf(1e-6f, __ldcg(&ws->frame_max[frame])));
-  const float inv_gamma = (float)(1.0 / (double)gamma);
-  const bool has_gamma = gamma != 1.0f;
-  constexpr float M[9] = {0.299f, 0.587f, 0.114f, -0.168736f, -0.331264f, 0.5f, 0.5f, -0.418688f, -0.081312f};   // yuv_420.py:12-16
-  float rgb[2][24];
-#pragma unroll
-  for (int dy = 0; dy < 2; ++dy) {
-    alignas(16) __half h[24];
-    ld_bytes<48>(src + ((size_t)(2 * qy + dy) * W + 8 * gx) * 3, h);
-#pragma unroll
-    for (int e = 0; e < 24; ++e) {
-      float q = __saturatef(__half2float(h[e]) * inv_max);
-      if (has_gamma) q = fast_pow(q, inv_gamma);
-      rgb[dy][e] = unit[Quant<uint8_t>::q(q) & 0xFFu];                          // the u8 value the RGB path stores, / in_scale
-    }
-  }
-  alignas(8) uint8_t yrow[2][8];
-  alignas(4) uint8_t cu4[4], cv4[4];
-#pragma unroll
-  for (int q = 0; q < 4; ++q) {
-    float u = 0.f, v = 0.f;
-#pragma unroll
-    for (int dy = 0; dy < 2; ++dy)
-#pragma unroll
-      for (int dx = 0; dx < 2; ++dx) {
-        const float* p = &rgb[dy][3 * (2 * q + dx)];
-        float o[3];
-#pragma unroll
-        for (int r = 0; r < 3; ++r)      // M @ (B, G, R), products and sums rounded separately, left to right
-          o[r] = __fadd_rn(__fadd_rn(__fmul_rn(M[3 * r], p[2]), __fmul_rn(M[3 * r + 1], p[1])), __fmul_rn(M[3 * r + 2], p[0]));
-        const float cu = __fadd_rn(o[1], 0.5f), cv = __fadd_rn(o[2], 0.5f);
-        yrow[dy][2 * q + dx] = cast_from_f32<uint8_t>(__fmul_rn(fminf(1.0f, o[0]), 255.0f));
-        if (dy == 0 && dx == 0) { u = cu; v = cv; } else { u = __fadd_rn(u, cu); v = __fadd_rn(v, cv); }
-      }
-    // u / 4.0 (yuv_420.py:62-63): a power-of-two divisor, the product with 0.25 is the same correctly rounded value
-    cu4[q] = cast_from_f32<uint8_t>(__fmul_rn(fminf(1.0f, __fmul_rn(u, 0.25f)), 255.0f));
-    cv4[q] = cast_from_f32<uint8_t>(__fmul_rn(fminf(1.0f, __fmul_rn(v, 0.25f)), 255.0f));
-  }
-#pragma unroll
-  for (int dy = 0; dy < 2; ++dy) st_bytes<8>(yuv + (size_t)(2 * qy + dy) * W + 8 * gx, yrow[dy]);
-  uint8_t* planes = yuv + (size_t)H * W;
-  const size_t plane = (size_t)(H / 2) * (W / 2), idx = (size_t)qy * (W / 2) + 4 * gx;
-  st_bytes<4>(planes + plane + idx, cu4);
-  st_bytes<4>(planes + idx, cv4);
-}
-
-// pass B with a TRANSPOSING transform (k.flip bit 2: transpose / rotate_90 / rotate_270 / transverse, interpolate.py:36-56 --
-// rotate_90 is the rig script's default, scripts/tonemap_scan.py) for both one-sweep Reinhard -> u8 forms: the element-wise
-// pass is the cheap place to turn the image, the sweep keeps its plain row stores and the separate transform kernel
-// (3 + 3 B/px) disappears.  Output (i, j) = source (r, c), i = c or W-1-c (bit 0), j = r or H-1-r (bit 1), shape (W, H).
-// CTA = a tile of 128 output columns (source rows) x 16 source columns.  Load phase: thread = 8 pixels of one source row
-// (3 x 16 bytes of the map; the tile's 96-byte row segments are whole sectors), normalise / gamma / quantise exactly like
-// the dense pass, one RGBx word per pixel into shared memory at [column][j + (j >> 3)] (row pitch 144 words).  Store phase:
-// thread = 8 consecutive pixels of one OUTPUT row (24 bytes, three 8-byte stores): a half warp writes 384 contiguous
-// bytes, and with that layout the 32 lanes of every LDS hit 32 different banks.  Default write policy: the two partial
-// sectors at the ends of a 384-byte piece meet their neighbours' (blockIdx.x runs along the output row) in L2.
-// Camera32: frames the u16 map declined were written as plain (H, W, 3) u8 into the frame's scratch by the gated write sweep
-// BEFORE this pass, which then only turns them.
-#ifndef ISP_TURNED_MINBLOCKS
-#define ISP_TURNED_MINBLOCKS 6     // measured: 8 CTAs per SM (32 registers, no spills) gain 2 % on eager Camera32 calls but lose 1 % on
-                                   // Camera16 and 2 % on the graphed look-ahead step (cfg3_rot90 214 -> 207 Gpixel/s)
-#endif
-constexpr int kTpRows = 128, kTpCols = 16, kTpPitch = 144;
-template <bool CAM16, bool GAMMA>
-__global__ void __launch_bounds__(256, ISP_TURNED_MINBLOCKS) reinhard_out_transposed_kernel(const FramePtrs scratch, const FramePtrs fp, int H, int W, int orow, int flip,
-                                                                      float gamma, const Workspace* ws) {
-  __shared__ uint32_t tile[kTpCols * kTpPitch];
-  const int frame = gridDim.z - 1 - blockIdx.z;        // last frame first, like the dense pass
-  const int j0 = blockIdx.x * kTpRows, c0 = blockIdx.y * kTpCols;
-  const float mx = __ldcg(&ws->frame_max[frame]);
-  {
-    const int cg = threadIdx.x & 1, lr = threadIdx.x >> 1;
-    const int j = j0 + lr, c = c0 + 8 * cg;
-    if (j < H && c < W) {
-      const int r = (flip & 2) ? H - 1 - j : j;
-      const size_t px = (size_t)r * W + c;
-      uint32_t v[24];
-      if constexpr (CAM16) {
-        const uint4* src = reinterpret_cast<const uint4*>(reinterpret_cast<const __half*>(scratch.out[frame]) + px * 3);
-        const uint4 w3[3] = {__ldcs(src), __ldcs(src + 1), __ldcs(src + 2)};
-        const __half* t = reinterpret_cast<const __half*>(w3);
-        const float inv_max = __fdiv_rn(1.0f, fmaxf(1e-6f, mx));
-        const float inv_gamma = (float)(1.0 / (double)gamma);
-#pragma unroll
-        for (int e = 0; e < 24; ++e) {
-          float q = __saturatef(__half2float(t[e]) * inv_max);
-          if (GAMMA) q = fast_pow(q, inv_gamma);
-          v[e] = Quant<uint8_t>::q(q);
-        }
-      } else if (reinhard_map16_declined(mx)) {
-        const uint2* src = reinterpret_cast<const uint2*>(reinterpret_cast<const uint8_t*>(scratch.out[frame]) + px * 3);
-        const uint2 b3[3] = {__ldcs(src), __ldcs(src + 1), __ldcs(src + 2)};
-        const uint8_t* t = reinterpret_cast<const uint8_t*>(b3);
-#pragma unroll
-        for (int e = 0; e < 24; ++e) v[e] = t[e];
-      } else {
-        const uint4* src = reinterpret_cast<const uint4*>(reinterpret_cast<const uint16_t*>(scratch.out[frame]) + px * 3);
-        const uint4 w3[3] = {__ldcs(src), __ldcs(src + 1), __ldcs(src + 2)};
-        const uint32_t* w = reinterpret_cast<const uint32_t*>(w3);
-        const float a = __fdiv_rn(__fdiv_rn(1.0f, mx), kMap16Scale);
-        const f2 a2 = bc(a), h2 = bc(0.5f * a), ig2 = bc((float)(1.0 / (double)gamma));
-#pragma unroll
-        for (int e = 0; e < 12; ++e) map16_pair(w[e], a2, h2, ig2, GAMMA, v[2 * e], v[2 * e + 1]);
-      }
-      uint32_t* col = tile + (8 * cg) * kTpPitch + lr + (lr >> 3);
-#pragma unroll
-      for (int q = 0; q < 8; ++q)      // the values' low bytes -> R | G << 8 | B << 16 (the top byte is never read)
-        col[q * kTpPitch] = __byte_perm(__byte_perm(v[3 * q], v[3 * q + 1], 0x0040), v[3 * q + 2], 0x0410);
-    }
-  }
-  __syncthreads();
-  {
-    const int rg = threadIdx.x & 15, lc = threadIdx.x >> 4;
-    const int j = j0 + 8 * rg, c = c0 + lc;
-    if (j < H && c < W) {                               // H % 8 == 0: the group is inside the row or entirely outside
-      const uint32_t* sp = tile + lc * kTpPitch + 9 * rg;
-      uint32_t p[8];
-#pragma unroll
-      for (int q = 0; q < 8; ++q) p[q] = sp[q];
-      const int i = (flip & 1) ? W - 1 - c : c;
-      uint2* d = reinterpret_cast<uint2*>(reinterpret_cast<uint8_t*>(fp.out[frame]) + (size_t)i * orow + 3 * j);
-      d[0] = make_uint2(__byte_perm(p[0], p[1], 0x4210), __byte_perm(p[1], p[2], 0x5421));
-      d[1] = make_uint2(__byte_perm(p[2], p[3], 0x6542), __byte_perm(p[4], p[5], 0x4210));
-      d[2] = make_uint2(__byte_perm(p[5], p[6], 0x5421), __byte_perm(p[6], p[7], 0x6542));
-    }
-  }
-}
-template <bool CAM16>
-static int run_out_transposed(const FramePtrs& sc, const FramePtrs& fp, int n_frames, const IspConsts& k, cudaStream_t s) {
-  const dim3 grid((unsigned)((k.H + kTpRows - 1) / kTpRows), (unsigned)((k.W + kTpCols - 1) / kTpCols), (unsigned)n_frames);
-  if (k.gamma != 1.0f) reinhard_out_transposed_kernel<CAM16, true><<<grid, 256, 0, s>>>(sc, fp, k.H, k.W, k.orow, k.flip, k.gamma, k.ws);
-  else reinhard_out_transposed_kernel<CAM16, false><<<grid, 256, 0, s>>>(sc, fp, k.H, k.W, k.orow, k.flip, k.gamma, k.ws);
-  return cuda_status(cudaPeekAtLastError(), "reinhard_out_transposed_kernel");
-}
-
-// pass A for frames [0, nframes): instantiated once per ISP dtype (fused_inst.cu with ISP_INST_RMAX); Camera16 stores the f16
-// map (any color_adapt), Camera32 the u16 fixed-point map (color_adapt == 0 only: the caller checks)
-template <bool CAM16>
-int run_rstore(const FramePtrs& fp_scratch, IspConsts k, int nframes, int rows_per_task, cudaStream_t s, void* ev_start, void* ev_stop) {
-  const Stream2Geom g = make_geom2(k.H, k.W, nframes, rows_per_task);
-  int st = B200ISP_OK;
-  if (ev_start) record_profile_event(ev_start, s);
-  auto launch = [&](auto ld, bool bl) -> int {
-    ld.fp = fp_scratch; ld.pitch_words = k.W * 3 / 8; ld.ids = k.ids;
-    ISP_DISPATCH_PATTERN(k.pattern, P, {
-      if (k.ca == 0.f) { EpiReinhardMax2<CAM16, true, true> e{fp_scratch, k}; st = launch_stream2<P>(ld, e, g, s, "isp_stream<reinhard_store>", bl); }
-      else if constexpr (CAM16) { EpiReinhardMax2<true, false, true> e{fp_scratch, k}; st = launch_stream2<P>(ld, e, g, s, "isp_stream<reinhard_store>", bl); }
-      else { set_error("process_packed12: the one-sweep Camera32 Reinhard map needs color_adapt == 0"); return B200ISP_E_ARG; }
-    });
-    return st;
-  };
-  if (k.ids) {
-    if (k.kbase != 0) { set_error("process_packed12: the IDS layout is fused for the Malvar demosaic only"); return B200ISP_E_ARG; }
-    st = launch(Packed12Loader2<CAM16, true>{}, false);
-  } else {
-    st = launch(Packed12Loader2<CAM16, false>{}, k.kbase != 0);
-  }
-  if (ev_stop) record_profile_event(ev_stop, s);
-  return st;
-}
-
-// The gated exact fallback of the one-sweep Camera32 path (color_adapt == 0, standard layout): max sweep into ws->frame_max2
-// + write sweep, both over all frames, every warp leaving at once unless its frame was declined -- in the usual case two
-// launches of CTAs that exit immediately.
-int run_rmax_gated(const FramePtrs& fp, IspConsts k, int nframes, int rows_per_task, cudaStream_t s);
-
-// frame-global Reinhard max: independent of the output dtype, instantiated once per ISP dtype (fused_inst.cu with ISP_INST_RMAX)
-template <bool CAM16>
-int run_rmax(const FramePtrs& fp, IspConsts k, int nframes, int rows_per_task, cudaStream_t s) {
-  return run_pass<CAM16, MODE_RMAX, uint8_t>(fp, k, nframes, rows_per_task, s);
-}
-
-int run_write_gated(const FramePtrs& fp, IspConsts k, int nframes, int rows_per_task, cudaStream_t s);
-
-// How b200isp_process_packed12 runs the Reinhard tone map of a parameter block that passed its checks, and the bytes of
-// reinhard_scratch that form uses: the maps of all frames, plus the per-frame tables of kF16Table.  reinhard_plan
-// (fused_api.cu) is the only place that decides this; run_fused, run_resize_t and b200isp_reinhard_scratch_bytes ask it.
-// A scratch smaller than map_bytes means the exact form (YUV 4:2:0 and resizing ISPs: refused); one that holds the maps
-// but not the tables means kF16Arith, whose result is bit-identical to kF16Table's.
+// ---------------------------------------------------------------- what b200isp_process_packed12 launches (run_fused, fused_api.cu)
+// How a call runs the Reinhard tone map of a parameter block that passed its checks, and the bytes of reinhard_scratch that
+// form uses: the maps of all frames, plus the per-frame tables of kF16Table.  reinhard_plan (fused_api.cu) is the only place
+// that decides this; run_fused and b200isp_reinhard_scratch_bytes ask it.  A scratch smaller than map_bytes means the exact
+// form (YUV 4:2:0, transposing transforms and resizing ISPs: refused); one that holds the maps but not the tables means
+// kF16Arith, whose result is bit-identical to kF16Table's.
 enum class ReinhardForm {
   kNone,          // no Reinhard tone map (linear, TM_NONE): one sweep
-  kExact,         // max sweep + write sweep (run_rmax, MODE_REINHARD)
-  kResizeMap,     // resizing ISP: the map at output resolution in the ISP dtype + a normalise pass (fused_resize.cu)
-  kF16Turned,     // Camera16 f16 map + reinhard_out_transposed_kernel (transposing transforms)
-  kF16Yuv,        // Camera16 f16 map + reinhard_scratch_yuv_kernel
+  kExact,         // Sweep::kMax + Sweep::kReinhard
+  kResizeMap,     // resizing ISP: the map at output resolution in the ISP dtype (run_resize) + a normalise pass
+  kF16Turned,     // Camera16 f16 map (Sweep::kStore) + run_out_transposed (transposing transforms)
+  kF16Yuv,        // Camera16 f16 map + run_scratch_yuv
   kF16Table,      // Camera16 f16 map + run_lut_pass (u8, gamma != 1: a 64 KB table per frame behind the maps)
-  kF16Arith,      // Camera16 f16 map + reinhard_scratch_out_kernel
-  kU16Map,        // Camera32 u16 fixed-point map + reinhard_map16_out_kernel + the gated exact sweeps
-  kU16Turned,     // Camera32 u16 fixed-point map + the gated exact sweeps + reinhard_out_transposed_kernel
+  kF16Arith,      // Camera16 f16 map + run_scratch_out
+  kU16Map,        // Camera32 u16 fixed-point map (Sweep::kStore) + run_map16_out + the gated exact sweeps
+  kU16Turned,     // Camera32 u16 fixed-point map + the gated exact sweeps + run_out_transposed
 };
 struct ReinhardPlan {
   ReinhardForm form;
@@ -1637,116 +1235,34 @@ struct ReinhardPlan {
 };
 ReinhardPlan reinhard_plan(const b200isp_fused_params& p, const IspConsts& k, int n_frames);
 
-template <bool CAM16, typename OutT>
-int run_fused(const FramePtrs& fp, int n_frames, const b200isp_fused_params& p, IspConsts k, cudaStream_t s) {
-  const int rpt = p.rows_per_task;
-  ReinhardPlan plan = reinhard_plan(p, k, n_frames);
-  if (plan.map_bytes && (!p.reinhard_scratch || p.reinhard_scratch_bytes < plan.map_bytes)) plan.form = ReinhardForm::kExact;
-  else if (plan.form == ReinhardForm::kF16Table && p.reinhard_scratch_bytes < plan.bytes) plan.form = ReinhardForm::kF16Arith;
-  if (p.out_yuv420 && plan.form == ReinhardForm::kExact) {
-    set_error("process_packed12: YUV 4:2:0 output needs Camera16 (f16), Reinhard, u8 and the reinhard_scratch buffer");
-    return B200ISP_E_ARG;
-  }
-  if ((k.flip & 4) && plan.form == ReinhardForm::kExact) {
-    set_error("process_packed12: the transposing transforms need the reinhard_scratch buffer (b200isp_reinhard_scratch_bytes)");
-    return B200ISP_E_ARG;
-  }
-  constexpr bool kIspOut = (CAM16 && std::is_same<OutT, __half>::value) || (!CAM16 && std::is_same<OutT, float>::value);
-  if (p.tonemap == B200ISP_TM_NONE) {
-    if constexpr (kIspOut) return run_pass<CAM16, MODE_RGB, OutT>(fp, k, n_frames, rpt, s, p.profile_start, p.profile_stop);
-    else { set_error("process_packed12: TM_NONE writes the ISP dtype"); return B200ISP_E_DTYPE; }
-  }
-  if constexpr (std::is_same<OutT, float>::value) {
-    set_error("process_packed12: tone-mapped output must be u8, u16 or f16");
-    return B200ISP_E_DTYPE;
-  } else {
-    if (p.tonemap == B200ISP_TM_LINEAR) return run_pass<CAM16, MODE_LINEAR, OutT>(fp, k, n_frames, rpt, s, p.profile_start, p.profile_stop);
-    // frame_max and frame_max2 are adjacent in the workspace: one memset node
-    static_assert(offsetof(Workspace, frame_max2) == offsetof(Workspace, frame_max) + sizeof(float) * B200ISP_MAX_FRAMES, "adjacent");
-    int st = cuda_status(cudaMemsetAsync(k.ws->frame_max, 0, sizeof(float) * 2 * B200ISP_MAX_FRAMES, s), "memset frame_max");
-    if (st) return st;
-    if constexpr (CAM16) {
-      // Camera16: the reference stores the map as f16 anyway -> one sweep writes it to the caller's scratch, a light
-      // element-wise pass normalises it (no second sweep, no L2 grouping)
-      if (plan.form != ReinhardForm::kExact) {
-        FramePtrs sc = fp;
-        for (int f = 0; f < n_frames; ++f) sc.out[f] = (char*)p.reinhard_scratch + (size_t)f * k.H * k.W * 3 * sizeof(__half);
-        IspConsts kp = k;            // the map is a plain dense (H, W, 3) image whatever the output looks like
-        kp.flip = 0;
-        kp.orow = 3 * k.W;
-        st = run_rstore<true>(sc, kp, n_frames, rpt, s, p.profile_start, p.profile_stop);
-        if (st) return st;
-        if (plan.form == ReinhardForm::kF16Turned) return run_out_transposed<true>(sc, fp, n_frames, k, s);     // the normalise pass turns the image
-        if (plan.form == ReinhardForm::kF16Yuv) {
-          const dim3 grid((unsigned)((k.W / 8 + 127) / 128), (unsigned)(k.H / 2), (unsigned)n_frames);
-          reinhard_scratch_yuv_kernel<<<grid, 128, 0, s>>>(sc, fp, k.H, k.W, k.gamma, k.ws);
-          return cuda_status(cudaPeekAtLastError(), "reinhard_scratch_yuv_kernel");
-        }
-        const long long n_elems = (long long)k.H * k.W * 3;
-        if constexpr (std::is_same<OutT, uint8_t>::value) {
-          if (plan.form == ReinhardForm::kF16Table)
-            return run_lut_pass(sc, fp, n_frames, n_elems, (uint8_t*)p.reinhard_scratch + plan.map_bytes, k.gamma, k.ws, s);
-        }
-        const dim3 grid((unsigned)std::min<long long>((n_elems / 8 + 255) / 256, 4 * kNumSMs), (unsigned)n_frames);
-        reinhard_scratch_out_kernel<OutT><<<grid, 256, 0, s>>>(sc, fp, n_elems, k.gamma, k.ws);
-        return cuda_status(cudaPeekAtLastError(), "reinhard_scratch_out_kernel");
-      }
-    }
-    if constexpr (!CAM16 && std::is_same<OutT, uint8_t>::value) {
-      // Camera32 -> u8, color_adapt == 0, gamma in [0.3, 1]: ONE sweep that also stores the map as u16 fixed point
-      // (6 B/px scratch) + an element-wise normalise / gamma / quantise pass.  The second demosaic of the two-sweep form
-      // (66 of its 106 instructions per pixel) disappears; the u8 result is within 1 LSB of the two-sweep result
-      // (measured: profiles/r02_reinhard_map16.txt).  Frames whose map does not fit [0, 1) (reinhard_map16_declined) are
-      // redone exactly by the gated sweeps.
-      if (plan.form != ReinhardForm::kExact) {
-        FramePtrs sc = fp;
-        for (int f = 0; f < n_frames; ++f) sc.out[f] = (char*)p.reinhard_scratch + (size_t)f * k.H * k.W * 3 * sizeof(uint16_t);
-        if (plan.form == ReinhardForm::kU16Turned) {
-          // transposing transform: map sweep (plain row stores), then the gated exact sweeps leave the frames the map declined
-          // as plain (H, W, 3) u8 images in their scratch, then ONE pass normalises / turns every frame into the output
-          IspConsts kp = k;
-          kp.flip = 0;
-          kp.orow = 3 * k.W;
-          st = run_rstore<false>(sc, kp, n_frames, rpt, s, p.profile_start, p.profile_stop);
-          if (st) return st;
-          kp.gate = 1;
-          st = run_rmax_gated(sc, kp, n_frames, rpt, s);
-          if (st) return st;
-          st = run_write_gated(sc, kp, n_frames, rpt, s);
-          if (st) return st;
-          return run_out_transposed<false>(sc, fp, n_frames, k, s);
-        }
-        // the normalise pass runs after the sweep with 8 CTAs per SM; running it under the sweep on a side stream measured
-        // 212-186 vs 215 Gpixel/s on cfg3 (profiles/r02_reinhard_map16.txt)
-        st = run_rstore<false>(sc, k, n_frames, rpt, s, p.profile_start, p.profile_stop);
-        if (st) return st;
-        const long long n_elems = (long long)k.H * k.W * 3;
-        const bool gam = k.gamma != 1.0f, pitched = k.orow != 3 * k.W;
-        const dim3 grid((unsigned)std::min<long long>((n_elems / 16 + 255) / 256, (8 * kNumSMs + n_frames - 1) / n_frames), (unsigned)n_frames);
-        if (gam && pitched) reinhard_map16_out_kernel<true, true><<<grid, 256, 0, s>>>(sc, fp, k.H, k.W, k.orow, k.gamma, k.ws);
-        else if (gam) reinhard_map16_out_kernel<true, false><<<grid, 256, 0, s>>>(sc, fp, k.H, k.W, k.orow, k.gamma, k.ws);
-        else if (pitched) reinhard_map16_out_kernel<false, true><<<grid, 256, 0, s>>>(sc, fp, k.H, k.W, k.orow, k.gamma, k.ws);
-        else reinhard_map16_out_kernel<false, false><<<grid, 256, 0, s>>>(sc, fp, k.H, k.W, k.orow, k.gamma, k.ws);
-        if ((st = cuda_status(cudaPeekAtLastError(), "reinhard_map16_out_kernel"))) return st;
-        IspConsts kg = k;
-        kg.gate = 1;
-        st = run_rmax_gated(fp, kg, n_frames, rpt, s);
-        if (st) return st;
-        return run_write_gated(fp, kg, n_frames, rpt, s);
-      }
-    }
-    // Camera32 (or no scratch): max sweep, then the write sweep recomputes the map.  Both sweeps are bound by
-    // instruction issue, not by DRAM, so the second read of the packed frames (1.5 B/px) is cheaper than cutting the
-    // call into L2-sized groups whose short launches end in idle tails (measured, profiles/r02_reinhard_diet.txt).
-    st = run_rmax<CAM16>(fp, k, n_frames, rpt, s);
-    if (st) return st;
-    return run_pass<CAM16, MODE_REINHARD, OutT>(fp, k, n_frames, rpt, s, p.profile_start, p.profile_stop);
-  }
-}
+// The sweeps over the packed frames fp.in (fused_inst.cu, one translation unit per group so that the kernel variants compile
+// in parallel).  rows_per_task <= 0: auto_rows_per_task2.
+enum class Sweep {
+  kRgb,           // EpiRgb2: the ISP dtype's float RGB (TM_NONE)
+  kLinear,        // EpiLinear2
+  kReinhard,      // EpiReinhard2: the write sweep of the exact form, max from ws->frame_max
+  kMax,           // EpiReinhardMax2: the max sweep of the exact form
+  kStore,         // EpiReinhardMax2<STORE>: the max sweep that also writes the map to fp.out (Camera32: color_adapt == 0)
+  kMaxGated,      // the exact max sweep (into ws->frame_max2) and write sweep of the frames the u16 map declined
+  kReinhardGated, //   (Camera32 -> u8, color_adapt == 0, standard layout; k.gate == 1): CTAs that exit at once otherwise
+};
+template <bool CAM16, typename OutT>     // kRgb, kLinear, kReinhard writing OutT
+int run_out_sweep(Sweep sw, const FramePtrs& fp, const IspConsts& k, int nframes, int rows_per_task, cudaStream_t s);
+template <bool CAM16>                    // kMax, kStore
+int run_max_sweep(Sweep sw, const FramePtrs& fp, const IspConsts& k, int nframes, int rows_per_task, cudaStream_t s);
+int run_gated_sweep(Sweep sw, const FramePtrs& fp, const IspConsts& k, int nframes, int rows_per_task, cudaStream_t s);
 
-extern template int run_rstore<true>(const FramePtrs&, IspConsts, int, int, cudaStream_t, void*, void*);
-extern template int run_rstore<false>(const FramePtrs&, IspConsts, int, int, cudaStream_t, void*, void*);
-extern template int run_rmax<true>(const FramePtrs&, IspConsts, int, int, cudaStream_t);
-extern template int run_rmax<false>(const FramePtrs&, IspConsts, int, int, cudaStream_t);
+// The normalise passes of the one-sweep forms (normalise.cu): the maps sc.out -> the outputs fp.out, frame maxima from k.ws.
+constexpr int kLutBytes = 65536;         // kF16Table: one u8 per f16 pattern and frame
+// kF16Arith, and kResizeMap on Camera16: n_elems values per frame, % 8 == 0; at most max_ctas CTAs per frame
+int run_scratch_out(const FramePtrs& sc, const FramePtrs& fp, int n_frames, long long n_elems, int out_dtype, float gamma,
+                    const Workspace* ws, int max_ctas, cudaStream_t s);
+int run_lut_pass(const FramePtrs& sc, const FramePtrs& fp, int n_frames, long long n_elems, uint8_t* lut, float gamma, const Workspace* ws,
+                 cudaStream_t s);                                       // kF16Table; lut = n_frames x kLutBytes behind the maps
+int run_scratch_yuv(const FramePtrs& sc, const FramePtrs& fp, int n_frames, const IspConsts& k, cudaStream_t s);        // kF16Yuv
+int run_map16_out(const FramePtrs& sc, const FramePtrs& fp, int n_frames, const IspConsts& k, cudaStream_t s);          // kU16Map
+int run_out_transposed(bool cam16, const FramePtrs& sc, const FramePtrs& fp, int n_frames, const IspConsts& k, cudaStream_t s);
+int run_resize_normalise(const FramePtrs& sc, const FramePtrs& fp, int n_frames, long long n_elems, bool cam16, int out_dtype,
+                         float gamma, const Workspace* ws, cudaStream_t s);     // kResizeMap: any n_elems, the ISP dtype's map
 
 }  // namespace isp

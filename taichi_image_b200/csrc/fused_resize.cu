@@ -22,24 +22,6 @@ __global__ void __launch_bounds__(256) resize_gather_kernel(const ResizeSrc<CAM1
   }
 }
 
-// pass B of Reinhard on the output-resolution scratch (ISP dtype): out = quantise((p / max_out)^(1/gamma)), camera_isp.py:217-218
-template <typename ScratchT, typename OutT>
-__global__ void __launch_bounds__(256) resize_normalise_kernel(const FramePtrs scratch, const FramePtrs outs, long long n_elems,
-                                                               float gamma, const Workspace* ws) {
-  const int frame = blockIdx.y;
-  const ScratchT* src = reinterpret_cast<const ScratchT*>(scratch.out[frame]);
-  OutT* dst = reinterpret_cast<OutT*>(outs.out[frame]);
-  const float inv_max = __fdiv_rn(1.0f, fmaxf(1e-6f, __ldcg(&ws->frame_max[frame])));
-  const float inv_gamma = (float)(1.0 / (double)gamma);
-  const bool has_gamma = gamma != 1.0f;
-  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n_elems; i += (long long)gridDim.x * blockDim.x) {
-    float q = __saturatef(to_f32(src[i]) * inv_max);
-    if (has_gamma) q = fast_pow(q, inv_gamma);
-    if constexpr (DT<OutT>::is_int) dst[i] = (OutT)(Quant<OutT>::q(q) & (uint32_t)DT<OutT>::scale);
-    else dst[i] = cast_from_f32<OutT>(q);
-  }
-}
-
 // One pass over the packed frames -> output-resolution images (io.out): the sweep form for down-scaling, the gather
 // otherwise.  Instantiated per (ISP dtype, mode) in resize_inst.cu.
 template <bool CAM16, int MODE, typename OutT>
@@ -86,56 +68,19 @@ ISP_RZ_EXT(false, uint8_t) ISP_RZ_EXT(false, uint16_t) ISP_RZ_EXT(false, __half)
 #undef ISP_RZ_EXT
 
 template <bool CAM16>
-static int run_resize_t(const FramePtrs& fp, int n_frames, const b200isp_fused_params& p, const IspConsts& k, cudaStream_t s) {
+static int run_resize_t(const FramePtrs& io, int n_frames, const b200isp_fused_params& p, const IspConsts& k, cudaStream_t s) {
   using IspT = std::conditional_t<CAM16, __half, float>;
-  if (p.profile_start) record_profile_event(p.profile_start, s);
-  int st = B200ISP_OK;
-  if (p.tonemap == B200ISP_TM_NONE) {
-    st = run_resize_pass<CAM16, RZ_RGB, IspT>(fp, k, p, n_frames, s);
-  } else if (p.tonemap == B200ISP_TM_LINEAR) {
-    switch (p.out_dtype) {
-      case B200ISP_U8: st = run_resize_pass<CAM16, RZ_LINEAR, uint8_t>(fp, k, p, n_frames, s); break;
-      case B200ISP_U16: st = run_resize_pass<CAM16, RZ_LINEAR, uint16_t>(fp, k, p, n_frames, s); break;
-      default: st = run_resize_pass<CAM16, RZ_LINEAR, __half>(fp, k, p, n_frames, s); break;
-    }
-  } else {
-    const size_t frame_bytes = (size_t)p.out_height * p.out_width * 3 * sizeof(IspT);
-    ISP_REQUIRE(p.reinhard_scratch && p.reinhard_scratch_bytes >= reinhard_plan(p, k, n_frames).bytes, B200ISP_E_ARG,
-                "process_packed12: Reinhard with resize needs reinhard_scratch of n_frames * out_height * out_width * 3 ISP-dtype values");
-    st = cuda_status(cudaMemsetAsync(k.ws->frame_max, 0, sizeof(float) * B200ISP_MAX_FRAMES, s), "memset frame_max");
-    if (st) return st;
-    FramePtrs sc = fp;
-    for (int f = 0; f < n_frames; ++f) sc.out[f] = (char*)p.reinhard_scratch + (size_t)f * frame_bytes;
-    st = run_resize_pass<CAM16, RZ_RSTORE, IspT>(sc, k, p, n_frames, s);
-    if (st) return st;
-    if (p.profile_stop) record_profile_event(p.profile_stop, s);
-    const long long n_elems = (long long)p.out_height * p.out_width * 3;
-    if constexpr (CAM16) {
-      if (n_elems % 8 == 0) {        // 16-byte vector form (fused_isp.cuh), shared with the full-resolution Camera16 path
-        const dim3 g8((unsigned)std::min<long long>((n_elems / 8 + 255) / 256, 8 * kNumSMs), (unsigned)n_frames);
-        switch (p.out_dtype) {
-          case B200ISP_U8: reinhard_scratch_out_kernel<uint8_t><<<g8, 256, 0, s>>>(sc, fp, n_elems, k.gamma, k.ws); break;
-          case B200ISP_U16: reinhard_scratch_out_kernel<uint16_t><<<g8, 256, 0, s>>>(sc, fp, n_elems, k.gamma, k.ws); break;
-          default: reinhard_scratch_out_kernel<__half><<<g8, 256, 0, s>>>(sc, fp, n_elems, k.gamma, k.ws); break;
-        }
-        return cuda_status(cudaPeekAtLastError(), "reinhard_scratch_out_kernel");
-      }
-    }
-    const dim3 g2((unsigned)std::min<long long>((n_elems + 255) / 256, 8 * kNumSMs), (unsigned)n_frames);
-    switch (p.out_dtype) {
-      case B200ISP_U8: resize_normalise_kernel<IspT, uint8_t><<<g2, 256, 0, s>>>(sc, fp, n_elems, k.gamma, k.ws); break;
-      case B200ISP_U16: resize_normalise_kernel<IspT, uint16_t><<<g2, 256, 0, s>>>(sc, fp, n_elems, k.gamma, k.ws); break;
-      default: resize_normalise_kernel<IspT, __half><<<g2, 256, 0, s>>>(sc, fp, n_elems, k.gamma, k.ws); break;
-    }
-    return cuda_status(cudaPeekAtLastError(), "resize_normalise_kernel");
+  if (p.tonemap == B200ISP_TM_NONE) return run_resize_pass<CAM16, RZ_RGB, IspT>(io, k, p, n_frames, s);
+  if (p.tonemap == B200ISP_TM_REINHARD) return run_resize_pass<CAM16, RZ_RSTORE, IspT>(io, k, p, n_frames, s);
+  switch (p.out_dtype) {
+    case B200ISP_U8: return run_resize_pass<CAM16, RZ_LINEAR, uint8_t>(io, k, p, n_frames, s);
+    case B200ISP_U16: return run_resize_pass<CAM16, RZ_LINEAR, uint16_t>(io, k, p, n_frames, s);
+    default: return run_resize_pass<CAM16, RZ_LINEAR, __half>(io, k, p, n_frames, s);
   }
-  if (p.profile_stop) record_profile_event(p.profile_stop, s);
-  return st;
 }
 
-// entry point used by fused_api.cu
-int run_resize(const FramePtrs& fp, int n_frames, const b200isp_fused_params& p, const IspConsts& k, cudaStream_t s) {
-  return p.isp_dtype == B200ISP_F16 ? run_resize_t<true>(fp, n_frames, p, k, s) : run_resize_t<false>(fp, n_frames, p, k, s);
+int run_resize(const FramePtrs& io, int n_frames, const b200isp_fused_params& p, const IspConsts& k, cudaStream_t s) {
+  return p.isp_dtype == B200ISP_F16 ? run_resize_t<true>(io, n_frames, p, k, s) : run_resize_t<false>(io, n_frames, p, k, s);
 }
 #endif
 

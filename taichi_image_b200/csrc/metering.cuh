@@ -186,30 +186,13 @@ __device__ __forceinline__ void fold_bounds(const float* __restrict__ g1, int wo
   bmax = __fadd_rn(mx, __fmul_rn(alpha, __fsub_rn(prev[1], mx)));
 }
 
-static __global__ void meter_fold_bounds_kernel(const float* __restrict__ g1, int world, float alpha, const float* __restrict__ prev,
-                                         Workspace* ws) {
-  if (threadIdx.x == 0 && blockIdx.x == 0) fold_bounds(g1, world, alpha, prev, ws->bounds[0], ws->bounds[1]);
-}
-
-static __global__ void meter_finalize_kernel(const float* __restrict__ g1, const float* __restrict__ g2, int world, float alpha,
-                                      const float* prev, float* metrics /* out; may alias prev */) {
-  if (threadIdx.x != 0 || blockIdx.x != 0) return;
-  float bmin, bmax;
-  fold_bounds(g1, world, alpha, prev, bmin, bmax);
-  float f[8] = {INFINITY, -INFINITY, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
-  for (int r = 0; r < world; ++r) {
-    f[0] = fminf(f[0], g2[8 * r]);
-    f[1] = fmaxf(f[1], g2[8 * r + 1]);
-    for (int k = 2; k < 8; ++k) f[k] += g2[8 * r + k];
-  }
-  const float fn = f[7];                                                  // camera_isp.py:131-134 with n = all ranks' samples
-  const float stats[9] = {bmin, bmax, f[0], f[1], __fdiv_rn(f[2], fn), __fdiv_rn(f[3], fn),
-                          __fdiv_rn(f[4], fn), __fdiv_rn(f[5], fn), __fdiv_rn(f[6], fn)};
-  for (int k = 0; k < 9; ++k) {                                           // camera_isp.py:165-166
-    const float p = prev[k];
-    metrics[k] = __fadd_rn(stats[k], __fmul_rn(alpha, __fsub_rn(p, stats[k])));
-  }
-}
+// The fold kernels of the shared exposure and phase 2 over the cached samples, defined in fused_api.cu so that each is compiled
+// once.
+int launch_meter_fold_bounds(const float* g1, int world, float alpha, const float* prev, Workspace* ws, cudaStream_t s);
+int launch_meter_finalize(const float* g1, const float* g2, int world, float alpha, const float* prev, float* metrics, cudaStream_t s);
+struct CachedSampler;
+int launch_meter_phase2_cached(int grid, const CachedSampler& smp, long long n, float alpha, const float* prev, float* metrics, Workspace* ws,
+                               cudaStream_t s, float* rec_out);
 
 // ---------------------------------------------------------------- shared exposure with the exchange INSIDE the kernels
 // Same two reductions, but the last block to finish a phase also runs that phase's cross-rank exchange (one warp:
@@ -457,8 +440,8 @@ inline int launch_metering(const Sampler& smp, long long n, float alpha, const f
   meter_phase1_kernel<Sampler><<<grid, 256, 0, s>>>(smp, n, alpha, prev, ws, cache);
   int st = cuda_status(cudaPeekAtLastError(), "meter_phase1_kernel");
   if (st) return st;
-  if (cache) meter_phase2_kernel<CachedSampler><<<grid, 256, 0, s>>>(CachedSampler{cache}, n, alpha, prev, metrics, ws);
-  else meter_phase2_kernel<Sampler><<<grid, 256, 0, s>>>(smp, n, alpha, prev, metrics, ws);
+  if (cache) return launch_meter_phase2_cached(grid, CachedSampler{cache}, n, alpha, prev, metrics, ws, s, nullptr);
+  meter_phase2_kernel<Sampler><<<grid, 256, 0, s>>>(smp, n, alpha, prev, metrics, ws);
   return cuda_status(cudaPeekAtLastError(), "meter_phase2_kernel");
 }
 
@@ -471,10 +454,11 @@ inline int launch_metering_phase1(const Sampler& smp, long long n, Workspace* ws
 template <class Sampler>
 inline int launch_metering_phase2(const Sampler& smp, long long n, const float* g1, int world, float alpha, const float* prev,
                                   Workspace* ws, cudaStream_t s, const float* cache, float* rec2) {
-  meter_fold_bounds_kernel<<<1, 32, 0, s>>>(g1, world, alpha, prev, ws);
+  const int st = launch_meter_fold_bounds(g1, world, alpha, prev, ws, s);
+  if (st) return st;
   const int grid = meter_grid(n);
-  if (cache) meter_phase2_kernel<CachedSampler><<<grid, 256, 0, s>>>(CachedSampler{cache}, n, alpha, nullptr, nullptr, ws, rec2);
-  else meter_phase2_kernel<Sampler><<<grid, 256, 0, s>>>(smp, n, alpha, nullptr, nullptr, ws, rec2);
+  if (cache) return launch_meter_phase2_cached(grid, CachedSampler{cache}, n, alpha, nullptr, nullptr, ws, s, rec2);
+  meter_phase2_kernel<Sampler><<<grid, 256, 0, s>>>(smp, n, alpha, nullptr, nullptr, ws, rec2);
   return cuda_status(cudaPeekAtLastError(), "meter_phase2_kernel");
 }
 

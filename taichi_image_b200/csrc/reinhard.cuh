@@ -1,8 +1,6 @@
 // Reinhard photoreceptor tone map of the ISP (reference: camera_isp.py:177-218; the same per-pixel
-// map as tonemap.py:107-131).  Two flavours share the parameter block:
-//   map_exact : literal operation order with IEEE division / powf, used by the eager per-stage API;
-//   map_fast  : MUFU-based (lg2/ex2/rcp) evaluation for the fused kernel; relative error ~1e-6,
-//               far inside the <= 1 LSB contract of the quantised outputs.
+// map as tonemap.py:107-131): the parameter block and the MUFU-based (lg2/ex2/rcp) evaluation every Reinhard kernel uses;
+// relative error ~1e-6, far inside the <= 1 LSB contract of the quantised outputs.
 #pragma once
 #include "common.cuh"
 
@@ -31,21 +29,6 @@ __device__ __forceinline__ ReinhardParams reinhard_params(const float* __restric
 #pragma unroll
   for (int k = 0; k < 3; ++k) p.mean[k] = __fadd_rn(mean, __fmul_rn(color_adapt, __fsub_rn(m[6 + k], mean)));
   return p;
-}
-
-// literal camera_isp.py:200-210; x = stored ISP-dtype RGB as f32
-__device__ __forceinline__ void reinhard_map_exact(const ReinhardParams& p, const float (&x)[3], float (&out)[3]) {
-  float s[3];
-#pragma unroll
-  for (int k = 0; k < 3; ++k) s[k] = __fdiv_rn(__fsub_rn(x[k], p.bmin), p.range);
-  const float gray = rgb_gray(s[0], s[1], s[2]);
-#pragma unroll
-  for (int k = 0; k < 3; ++k) {
-    const float ac = __fadd_rn(gray, __fmul_rn(p.ca, __fsub_rn(s[k], gray)));
-    const float am = __fadd_rn(p.mean[k], __fmul_rn(p.la, __fsub_rn(ac, p.mean[k])));
-    const float adapt = powf(__fmul_rn(p.ki, am), p.map_key);
-    out[k] = __fmul_rn(s[k], __fdiv_rn(1.0f, __fadd_rn(adapt, s[k])));
-  }
 }
 
 // x^y through the two MUFU ops only (lg2.approx / ex2.approx, no range fix-ups: arguments are O(1) here; x <= 0

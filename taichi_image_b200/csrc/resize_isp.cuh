@@ -179,6 +179,8 @@ inline ResizeSrc<CAM16> make_resize_src(const FramePtrs& fp, const IspConsts& k,
   return ResizeSrc<CAM16>{fp, k, p.width * 3 / 8, p.out_height, p.out_width, p.scale_r, p.scale_c};
 }
 
-int run_resize(const FramePtrs& fp, int n_frames, const b200isp_fused_params& p, const IspConsts& k, cudaStream_t s);
+// The resizing pass of p.tonemap into io.out (fused_resize.cu): the output images, or with Reinhard the output-resolution
+// maps in the ISP dtype (ReinhardForm::kResizeMap) and the frame maxima in ws->frame_max.
+int run_resize(const FramePtrs& io, int n_frames, const b200isp_fused_params& p, const IspConsts& k, cudaStream_t s);
 
 }  // namespace isp

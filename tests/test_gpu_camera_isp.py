@@ -425,7 +425,7 @@ def test_flips_in_the_store(cuda, dt, tname, shape):
 @pytest.mark.parametrize("shape", [(40, 64), (48, 1032), (16, 776), (64, 264), (44, 72)])
 def test_transposing_transforms_after_the_sweep_or_in_the_turned_pass(cuda, dt, tname, shape):
     """rotate_90 (the rig script's default) / rotate_270 / transpose / transverse: the normalise pass of the one-sweep
-    Reinhard -> u8 forms turns the image (csrc/fused_isp.cuh reinhard_out_transposed_kernel; here Camera16, whose turned form
+    Reinhard -> u8 forms turns the image (csrc/normalise.cu reinhard_out_transposed_kernel; here Camera16, whose turned form
     does not depend on reinhard_exact), every other call runs the transform kernel on its results -- bit for bit
     interpolate.transform of the untransformed result for every output dtype, default tasks and tasks of 8 rows"""
     from taichi_image_b200.interpolate import ImageTransform, transform

@@ -220,7 +220,7 @@ def test_sweep_geometry_and_epilogue(cuda, fam, i, shape):
 
     if fam == "turn":
         # rotate_90 / transpose of the Reinhard -> u8 forms: the element-wise normalise pass turns the image
-        # (csrc/fused_isp.cuh reinhard_out_transposed_kernel) -- Camera32 from its u16 map, Camera16 from its f16 map
+        # (csrc/normalise.cu reinhard_out_transposed_kernel) -- Camera32 from its u16 map, Camera16 from its f16 map
         from taichi_image_b200.dtypes import u8
         from taichi_image_b200.interpolate import ImageTransform
         tname = ("rotate_90", "transpose")[i % 2]

@@ -1,5 +1,5 @@
 """Transposing ISP transforms (interpolate.py:36-56; rotate_90 is the default of scripts/tonemap_scan.py) applied by the
-element-wise normalise pass of the one-sweep Reinhard -> u8 forms (csrc/fused_isp.cuh reinhard_out_transposed_kernel):
+element-wise normalise pass of the one-sweep Reinhard -> u8 forms (csrc/normalise.cu reinhard_out_transposed_kernel):
 
 * the turned result equals ``interpolate.transform`` of the untransformed result of the SAME path bit for bit (the pass runs
   the same arithmetic; only the store differs) -- Camera16 (f16 map, arithmetic and table pass) and Camera32 (u16 map), all
